@@ -6,7 +6,8 @@ gradient all-reduce; optimizer and metrics excluded) on N B200s of one node.
   python bench.py --impl reference ...                   # the reference path on the host CPU cores
   torchrun --nproc-per-node N bench.py --gpus N ...      # N > 1: one rank per GPU, NCCL
 
-Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for every field.
+Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for every field.  Inputs and weights are seeded, so two builds
+run with the same arguments and `--dump-outputs DIR` can be compared output for output.
 """
 from __future__ import annotations
 
@@ -201,6 +202,22 @@ def cpu_reference_run(cfg, kw, cond_in, steps, warmup, budget_s, threads=None):
           'ms_per_step': dt * 1e3, 'steps': len(times)}
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, loss, grads):
+  """What one training step hands its caller, as float32 .npy files: loss.npy = [loss, reg_loss] and grads.npy = the
+  gradients of every variable, flattened and concatenated in variable order.  When the gradients exceed the size limit,
+  grads.npy holds a fixed, seeded sample of their entries (in index order), the same for every run of the same workload."""
+  os.makedirs(out_dir, exist_ok=True)
+  g = np.concatenate([v.ravel() for v in grads.values()]).astype(np.float32)
+  budget = (DUMP_LIMIT_BYTES - (1 << 12)) // g.itemsize - loss.size   # (1 << 12): the two .npy headers
+  if g.size > budget:
+    g = g[np.sort(np.random.default_rng(0).choice(g.size, budget, replace=False))]
+  np.save(os.path.join(out_dir, 'loss.npy'), loss.astype(np.float32))
+  np.save(os.path.join(out_dir, 'grads.npy'), g)
+
+
 def model_allreduce_kind(model):
   if model.n_replicas <= 1:
     return 'none (1 replica)'
@@ -275,7 +292,13 @@ def main():
   ap.add_argument('--sustain-seconds', type=float, default=3.0, help='length of the additional seconds-long timed region (0 = off)')
   ap.add_argument('--dropout', type=float, default=None, help="override the config's dropout (defaults.yaml:17 trains with 0.1)")
   ap.add_argument('--check-grads', action='store_true', help='compare the all-reduced N-GPU gradients with a 1-GPU step on the concatenated batch')
+  ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                  help='write the loss and gradients of the last timed step to DIR/loss.npy and DIR/grads.npy (float32, at most 64 MB)')
   args = ap.parse_args()
+  if args.steps < 1:
+    ap.error('--steps must be at least 1')
+  if args.dump_outputs and args.impl != 'b200':
+    ap.error('--dump-outputs writes the outputs of the CUDA path (--impl b200)')
   if args.warmup < 3 and args.impl == 'b200':
     args.warmup = 3   # timing rule: W >= 3
 
@@ -396,6 +419,8 @@ def main():
   ar_early = int(h.lib.wn_allreduce_buckets(h.h))
   clocks = sampler.stop() if sampler else None
   loss_last = float(loss_t[0].item())
+  # the steps below overwrite the gradient buffer: keep what the last timed step returned
+  last_outputs = (loss_t.cpu().numpy(), model.get_grads()) if args.dump_outputs and rank == 0 else None
 
   # ---- timed region 2: end to end through the public API with HOST buffers
   sync_all()
@@ -617,6 +642,8 @@ def main():
     if world == 1 and not args.no_cpu_baseline:
       r = cpu_reference_run(cfg, kw, cond_in, steps=5, warmup=1, budget_s=25.0)
       line['cpu_baseline'] = {k: r[k] for k in ('value', 'unit', 'cores', 'kind', 'sample')}
+    if last_outputs is not None:
+      dump_outputs(args.dump_outputs, *last_outputs)
     print(json.dumps(line))
   if world > 1:
     dist.barrier()

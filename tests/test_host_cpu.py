@@ -96,9 +96,11 @@ def test_layer_attributes_and_errors():
 
 
 def test_reference_yaml_loads():
+  """tests/golden/defaults.yaml restates the reference's configfiles/defaults.yaml in its 27-line layout: train.py's key
+  names (the `use_resiudal` typo included) and the file's dataset path, which differs from train.py's default."""
   from wavenets_b200 import load_config, model_kwargs, CONFIGS
-  ref = '/root/reference/configfiles/defaults.yaml'
-  cfg = load_config(ref if os.path.exists(ref) else None)
+  cfg = load_config(os.path.join(ROOT, 'tests', 'golden', 'defaults.yaml'))
+  assert cfg['dataset'] == './datasets/svd8000'
   kw = model_kwargs(cfg)
   assert kw['use_residual'] is True and kw['channels'] == 32 and kw['final_layers_channels'] == [128, 256]
   assert set(CONFIGS) == {'c1', 'c2', 'c3', 'c4', 'c5'}
