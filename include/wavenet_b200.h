@@ -217,6 +217,15 @@ int wn_layer_forward(wn_handle* h, int block, const float* x_dev, const float* c
  * Philox draw for this block, and wn_layer_backward of the block uses the same mask. */
 int wn_layer_forward_ex(wn_handle* h, int block, const float* x_dev, const float* cond_dev, int B, int T, int training,
                         float* x_out_dev, float* skip_dev, void* stream);
+/* WaveNetLayer.call with a conditioning SEQUENCE (layers.py:115-120,203-204): cond (B,T,cond_in) fp32, one vector per
+ * time step (local conditioning), added to the gated conv's pre-activation as conv_cond(cond) at every t; the dropout
+ * mask (training != 0) applies to x only.  The block must have conditioning and the handle no head (has_head = 0).  Any
+ * cond_in and every kernel_size work on both tiers.  The sequence buffer must stay valid until the block's wn_layer_backward.
+ * WN_ERR_VALUE: NULL sequence or a block without conditioning; WN_ERR_UNSUPPORTED: a model handle. */
+int wn_layer_forward_seq(wn_handle* h, int block, const float* x_dev, const float* cond_dev /* (B,T,cond_in) fp32 */, int B, int T,
+                         int training, float* x_out_dev, float* skip_dev, void* stream);
+/* Adjoint of the block's last forward (WN_ERR_STATE before any): dcond_dev receives (B,T,cond_in) when that forward was
+ * wn_layer_forward_seq, (B,cond_in) otherwise. */
 int wn_layer_backward(wn_handle* h, int block, const float* dx_out_dev, const float* dskip_dev,
                       float* dx_dev, float* dcond_dev, void* stream);
 

@@ -24,7 +24,7 @@ EXPORTS = [
   'wn_fused_forward_blocks', 'wn_grouped_wgrad_tiles', 'wn_stack_forward_layers', 'wn_profile_begin', 'wn_profile_end', 'wn_profile_get', 'wn_build_info', 'wn_set_dropout_masks', 'wn_set_dropout_seed', 'wn_layer_forward_ex', 'wn_num_frames', 'wn_preprocess_frames', 'wn_inverse_mu_law', 'wn_one_hot', 'wn_sample_waveform', 'wn_sample_last_step', 'wn_generate', 'wn_adam_init', 'wn_clip_grads', 'wn_adam_step', 'wn_adam_state', 'wn_debug_conv_gemm', 'wn_debug_wgrad', 'wn_debug_bench',
   'wn_forward_ex', 'wn_loss_fn', 'wn_adam_restore', 'wn_nccl_unique_id', 'wn_comm_init', 'wn_comm_attach', 'wn_comm_fuse_allreduce',
   'wn_allreduce_grads', 'wn_nccl_info', 'wn_grouped_wgrad_info', 'wn_debug_tensor', 'wn_stack_backward_layers',
-  'wn_allreduce_buckets',
+  'wn_allreduce_buckets', 'wn_layer_forward_seq',
 ]
 
 
@@ -98,6 +98,7 @@ def load():
   lib.wn_train_step_host.argtypes = [vp, vp, vp, i32, i32, i32, vp]
   lib.wn_layer_forward.argtypes = [vp, i32, vp, vp, i32, i32, vp, vp, vp]
   lib.wn_layer_forward_ex.argtypes = [vp, i32, vp, vp, i32, i32, i32, vp, vp, vp]
+  lib.wn_layer_forward_seq.argtypes = [vp, i32, vp, vp, i32, i32, i32, vp, vp, vp]
   lib.wn_layer_backward.argtypes = [vp, i32, vp, vp, vp, vp, vp]
   lib.wn_last_launch_count.argtypes = [vp]
   lib.wn_last_launch_count.restype = i64

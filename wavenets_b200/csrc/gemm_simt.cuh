@@ -13,7 +13,9 @@
 #pragma once
 #include "common.cuh"
 
-#define WN_MAX_SEG 4
+#define WN_MAX_TAPS 4
+// + 1: the gated conv of a layer called with a conditioning sequence contracts it as one more segment (shift 0)
+#define WN_MAX_SEG (WN_MAX_TAPS + 1)
 
 struct SegF {
   const float* A;   // [(b*T + t) * lda + c]

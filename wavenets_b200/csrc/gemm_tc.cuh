@@ -27,7 +27,9 @@
 #include "tc_epilogues.cuh"
 
 #define WN_MAX_WGRAD_SPLITS 64
-#define TC_MAX_SEG 4
+#define TC_MAX_TAPS 4
+// + 1: the gated conv of a layer called with a conditioning sequence contracts it as one more segment (shift 0)
+#define TC_MAX_SEG (TC_MAX_TAPS + 1)
 
 struct TcSeg { const bf16* A; int lda; int shift; int K; };
 // L2 policy per tensor of a launch: 0 = normal, 1 = evict_first (streaming), 2 = evict_last (the next kernel reads it)
@@ -45,7 +47,7 @@ struct TcGemmDesc {
   int B, T, nseg; TcSeg seg[TC_MAX_SEG]; int n_outer; long long outer_stride;
   const bf16* W; int ktot; int N16; int tileN;
   int l2_a = 0, l2_in[2] = {0, 0}, l2_out[3] = {0, 0, 0};   // TC_L2_* codes: activation operand, epilogue inputs, outputs
-  int l2_seg[TC_MAX_SEG] = {-1, -1, -1, -1};                // per-segment override of l2_a (-1: none)
+  int l2_seg[TC_MAX_SEG] = {-1, -1, -1, -1, -1};            // per-segment override of l2_a (-1: none)
 };
 struct TcWgradDesc {
   int l2_a = 0, l2_g = 0;
@@ -60,7 +62,7 @@ struct TcWgradPlan { int nsplit, chunks_per_split, chunks_t, slots, mtiles; };
 // the next tap's rows, which meet those zeros.  Output panels are 32 columns wide.
 static inline int tc_check_config(int R, int D, int S, int K) {
   if (R % 32 || D % 32 || S % 32) return -1;
-  if (K > TC_MAX_SEG) return -2;
+  if (K > TC_MAX_TAPS) return -2;
   return 0;
 }
 // column tiling of an N-wide output: N16 = padded width, tile = CTA tile width (64/128/256).
@@ -135,7 +137,7 @@ template <int BN> struct TcGemmCfg {
 template <class Epi, int BN, int NEPI>
 __global__ void __launch_bounds__(128 + 32 * NEPI, 1)
 tc_conv_gemm_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__ CUtensorMap tmA1, const __grid_constant__ CUtensorMap tmA2,
-                    const __grid_constant__ CUtensorMap tmA3, const __grid_constant__ CUtensorMap tmW, const TcGemmParams p,
+                    const __grid_constant__ CUtensorMap tmA3, const __grid_constant__ CUtensorMap tmA4, const __grid_constant__ CUtensorMap tmW, const TcGemmParams p,
                     const typename Epi::Params ep) {
   using Cfg = TcGemmCfg<BN>;
   constexpr int STAGES = Cfg::STAGES;
@@ -153,6 +155,7 @@ tc_conv_gemm_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_const
     if (p.nseg > 1) tma_prefetch_desc(&tmA1);
     if (p.nseg > 2) tma_prefetch_desc(&tmA2);
     if (p.nseg > 3) tma_prefetch_desc(&tmA3);
+    if (p.nseg > 4) tma_prefetch_desc(&tmA4);
     tma_prefetch_desc(&tmW);
   }
   if (warp == 1 && lane == 0) {
@@ -176,7 +179,7 @@ tc_conv_gemm_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_const
         int wk = 0;
         for (int o = 0; o < p.n_outer; ++o) {
           for (int s = 0; s < p.nseg; ++s) {
-            const CUtensorMap* tm = s == 0 ? &tmA0 : (s == 1 ? &tmA1 : (s == 2 ? &tmA2 : &tmA3));
+            const CUtensorMap* tm = s == 0 ? &tmA0 : (s == 1 ? &tmA1 : (s == 2 ? &tmA2 : (s == 3 ? &tmA3 : &tmA4)));
             const int kseg = p.segK[s], tcoord = t0 + p.segShift[s];
             for (int k0 = 0; k0 < kseg; k0 += Cfg::BK) {
               mbar_wait(&empty_bar[stage], phase ^ 1);
@@ -293,7 +296,7 @@ static inline int tc_balanced_slots(int tiles, int slots) {
 template <class Epi, int BN, int NEPI>
 static int tc_conv_gemm_launch(TmapCache& tc, cudaStream_t st, const TcGemmDesc& d, const typename Epi::Params& ep) {
   using Cfg = TcGemmCfg<BN>;
-  const CUtensorMap* ma[TC_MAX_SEG] = {nullptr, nullptr, nullptr, nullptr};
+  const CUtensorMap* ma[TC_MAX_SEG] = {};
   for (int s = 0; s < d.nseg; ++s) {
     ma[s] = tc_act_map(tc, d.seg[s].A, d.seg[s].lda, d.seg[s].K, d.T, d.B, s == 0 ? d.n_outer : 1, d.outer_stride, 128);
     if (!ma[s]) return -10;
@@ -315,7 +318,7 @@ static int tc_conv_gemm_launch(TmapCache& tc, cudaStream_t st, const TcGemmDesc&
     if (e != cudaSuccess) { snprintf(g_tc_err, sizeof(g_tc_err), "cudaFuncSetAttribute(smem=%d): %s", Cfg::SMEM_BYTES, cudaGetErrorString(e)); return -12; }
   }
   const int grid = p.num_tiles < tc_num_sms() ? p.num_tiles : tc_num_sms();
-  kern<<<grid, 128 + 32 * NEPI, Cfg::SMEM_BYTES, st>>>(*ma[0], *ma[1], *ma[2], *ma[3], *mw, p, ep);
+  kern<<<grid, 128 + 32 * NEPI, Cfg::SMEM_BYTES, st>>>(*ma[0], *ma[1], *ma[2], *ma[3], *ma[4], *mw, p, ep);
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) { snprintf(g_tc_err, sizeof(g_tc_err), "conv_gemm launch: %s", cudaGetErrorString(e)); return -13; }
   return 0;
@@ -375,7 +378,7 @@ template <int BN, int NIN, int NOUT, int IN_PANELS, int OUT_SLOTS_, int CG = 1> 
 template <class Epi, int BN, int CG>
 __global__ void __launch_bounds__(384, 1)
 tc_conv_gemm_staged_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__ CUtensorMap tmA1, const __grid_constant__ CUtensorMap tmA2,
-                           const __grid_constant__ CUtensorMap tmA3, const __grid_constant__ CUtensorMap tmW,
+                           const __grid_constant__ CUtensorMap tmA3, const __grid_constant__ CUtensorMap tmA4, const __grid_constant__ CUtensorMap tmW,
                            const __grid_constant__ CUtensorMap tmI0, const __grid_constant__ CUtensorMap tmI1,
                            const __grid_constant__ CUtensorMap tmO0, const __grid_constant__ CUtensorMap tmO1, const __grid_constant__ CUtensorMap tmO2,
                            const TcGemmParams p, const TcStagedParams sp, const typename Epi::Params ep) {
@@ -450,7 +453,7 @@ tc_conv_gemm_staged_kernel(const __grid_constant__ CUtensorMap tmA0, const __gri
         int wk = 0;
         for (int o = 0; o < p.n_outer; ++o) {
           for (int s = 0; s < p.nseg; ++s) {
-            const CUtensorMap* tm = s == 0 ? &tmA0 : (s == 1 ? &tmA1 : (s == 2 ? &tmA2 : &tmA3));
+            const CUtensorMap* tm = s == 0 ? &tmA0 : (s == 1 ? &tmA1 : (s == 2 ? &tmA2 : (s == 3 ? &tmA3 : &tmA4)));
             const int kseg = p.segK[s], tcoord = t0 + p.segShift[s];
             const unsigned long long pol_as = sp.pol_seg[s];
             for (int k0 = 0; k0 < kseg; k0 += Cfg::BK) {
@@ -758,7 +761,7 @@ template <class Epi, int BN, int CG>
 static int tc_conv_gemm_staged_launch(TmapCache& tc, cudaStream_t st, const TcGemmDesc& d, const typename Epi::Params& ep, const TcEpiIo* ins,
                                       uint32_t in_mask, const TcEpiIo* outs) {
   using Cfg = TcStagedCfg<BN, Epi::NIN, Epi::NOUT, Epi::kInPanels, Epi::kOutSlots, CG>;
-  const CUtensorMap* ma[TC_MAX_SEG] = {nullptr, nullptr, nullptr, nullptr};
+  const CUtensorMap* ma[TC_MAX_SEG] = {};
   for (int s = 0; s < d.nseg; ++s) {
     ma[s] = tc_act_map(tc, d.seg[s].A, d.seg[s].lda, d.seg[s].K, d.T, d.B, s == 0 ? d.n_outer : 1, d.outer_stride, 128);
     if (!ma[s]) return -10;
@@ -807,7 +810,7 @@ static int tc_conv_gemm_staged_launch(TmapCache& tc, cudaStream_t st, const TcGe
   cfg.gridDim = dim3(grid); cfg.blockDim = dim3(384); cfg.dynamicSmemBytes = Cfg::SMEM_BYTES; cfg.stream = st;
   cudaLaunchAttribute attr[2];
   cfg.attrs = attr; cfg.numAttrs = tc_launch_attrs(attr, CG);
-  cudaError_t e = cudaLaunchKernelEx(&cfg, kern, *ma[0], *ma[1], *ma[2], *ma[3], *mw, *mi[0], *mi[1], *mo[0], *mo[1], *mo[2], p, sp, ep);
+  cudaError_t e = cudaLaunchKernelEx(&cfg, kern, *ma[0], *ma[1], *ma[2], *ma[3], *ma[4], *mw, *mi[0], *mi[1], *mo[0], *mo[1], *mo[2], p, sp, ep);
   if (e != cudaSuccess) { snprintf(g_tc_err, sizeof(g_tc_err), "staged conv_gemm launch (cta_group %d): %s", CG, cudaGetErrorString(e)); return -13; }
   return 0;
 }
@@ -877,7 +880,7 @@ template <int BN> struct TcWgradCfg {
 template <int BN, int CL>
 __global__ void __launch_bounds__(256, 1)
 tc_wgrad_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__ CUtensorMap tmA1, const __grid_constant__ CUtensorMap tmA2,
-                const __grid_constant__ CUtensorMap tmA3, const __grid_constant__ CUtensorMap tmG, const TcWgradParams p) {
+                const __grid_constant__ CUtensorMap tmA3, const __grid_constant__ CUtensorMap tmA4, const __grid_constant__ CUtensorMap tmG, const TcWgradParams p) {
   using Cfg = TcWgradCfg<BN>;
   constexpr int STAGES = Cfg::STAGES;
   extern __shared__ uint8_t smem_raw[];
@@ -928,7 +931,7 @@ tc_wgrad_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
 
   if (warp == 0) {
     if (lane == 0) {
-      const CUtensorMap* tm = s == 0 ? &tmA0 : (s == 1 ? &tmA1 : (s == 2 ? &tmA2 : &tmA3));
+      const CUtensorMap* tm = s == 0 ? &tmA0 : (s == 1 ? &tmA1 : (s == 2 ? &tmA2 : (s == 3 ? &tmA3 : &tmA4)));
       tma_prefetch_desc(tm);
       tma_prefetch_desc(&tmG);
       const int shift = p.segShift[s];
@@ -1086,7 +1089,7 @@ template <int BN, int NH = 1> struct TcWgradPairCfg {
 template <int BN, int NH>
 __global__ void __launch_bounds__(256, 1)
 tc_wgrad_pair_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__ CUtensorMap tmA1, const __grid_constant__ CUtensorMap tmA2,
-                     const __grid_constant__ CUtensorMap tmA3, const __grid_constant__ CUtensorMap tmG, const __grid_constant__ CUtensorMap tmP,
+                     const __grid_constant__ CUtensorMap tmA3, const __grid_constant__ CUtensorMap tmA4, const __grid_constant__ CUtensorMap tmG, const __grid_constant__ CUtensorMap tmP,
                      const TcWgradParams p) {
   using Cfg = TcWgradPairCfg<BN, NH>;
   constexpr int STAGES = Cfg::STAGES;
@@ -1140,7 +1143,7 @@ tc_wgrad_pair_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_cons
 
   if (warp == 0) {
     if (lane == 0) {
-      const CUtensorMap* tm = s == 0 ? &tmA0 : (s == 1 ? &tmA1 : (s == 2 ? &tmA2 : &tmA3));
+      const CUtensorMap* tm = s == 0 ? &tmA0 : (s == 1 ? &tmA1 : (s == 2 ? &tmA2 : (s == 3 ? &tmA3 : &tmA4)));
       tma_prefetch_desc(tm);
       tma_prefetch_desc(&tmG);
       const int shift = p.segShift[s];
@@ -1338,7 +1341,7 @@ tc_wgrad_pair_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_cons
 template <int BN, int NH>
 static int tc_wgrad_pair_launch(TmapCache& tc, cudaStream_t st, const TcWgradDesc& d, TcWgradPlan* plan) {
   using Cfg = TcWgradPairCfg<BN, NH>;
-  const CUtensorMap* ma[TC_MAX_SEG] = {nullptr, nullptr, nullptr, nullptr};
+  const CUtensorMap* ma[TC_MAX_SEG] = {};
   int mpairs = 0;
   for (int s = 0; s < d.nseg; ++s) {
     ma[s] = tc_atom_map(tc, d.seg[s].A, d.seg[s].lda, d.seg[s].K, d.T, d.B, 64, 2);
@@ -1379,7 +1382,7 @@ static int tc_wgrad_pair_launch(TmapCache& tc, cudaStream_t st, const TcWgradDes
   cfg.gridDim = dim3(2 * mpairs, ntiles, nsplit); cfg.blockDim = dim3(256); cfg.dynamicSmemBytes = Cfg::SMEM_BYTES; cfg.stream = st;
   cudaLaunchAttribute attr[2];
   cfg.attrs = attr; cfg.numAttrs = tc_launch_attrs(attr, 2);
-  cudaError_t e = cudaLaunchKernelEx(&cfg, kern, *ma[0], *ma[1], *ma[2], *ma[3], *mg, *mp, p);
+  cudaError_t e = cudaLaunchKernelEx(&cfg, kern, *ma[0], *ma[1], *ma[2], *ma[3], *ma[4], *mg, *mp, p);
   if (e != cudaSuccess) { snprintf(g_tc_err, sizeof(g_tc_err), "wgrad launch (cta pairs): %s", cudaGetErrorString(e)); return -13; }
   return 0;
 }
@@ -1421,7 +1424,7 @@ static int tc_wgrad_launch_cl(const CUtensorMap* const* ma, const CUtensorMap* m
   cfg.gridDim = grid; cfg.blockDim = dim3(256); cfg.dynamicSmemBytes = Cfg::SMEM_BYTES; cfg.stream = st;
   cudaLaunchAttribute attr[2];
   cfg.attrs = attr; cfg.numAttrs = tc_launch_attrs(attr, CL);
-  cudaError_t e = cudaLaunchKernelEx(&cfg, kern, *ma[0], *ma[1], *ma[2], *ma[3], *mg, p);
+  cudaError_t e = cudaLaunchKernelEx(&cfg, kern, *ma[0], *ma[1], *ma[2], *ma[3], *ma[4], *mg, p);
   if (e != cudaSuccess) { snprintf(g_tc_err, sizeof(g_tc_err), "wgrad launch (cluster %d): %s", CL, cudaGetErrorString(e)); return -13; }
   return 0;
 }
@@ -1429,7 +1432,7 @@ static int tc_wgrad_launch_cl(const CUtensorMap* const* ma, const CUtensorMap* m
 template <int BN>
 static int tc_wgrad_launch(TmapCache& tc, cudaStream_t st, const TcWgradDesc& d, TcWgradPlan* plan) {
   using Cfg = TcWgradCfg<BN>;
-  const CUtensorMap* ma[TC_MAX_SEG] = {nullptr, nullptr, nullptr, nullptr};
+  const CUtensorMap* ma[TC_MAX_SEG] = {};
   int mtiles = 0;
   for (int s = 0; s < d.nseg; ++s) {
     ma[s] = tc_act_map(tc, d.seg[s].A, d.seg[s].lda, d.seg[s].K, d.T, d.B, 1, 0, 64);

@@ -37,7 +37,7 @@ template <int NT1> __device__ __forceinline__ void blk_tile(int pos, int n, int&
 
 struct TcBlockParams {
   int B, T, tiles_t, num_mtiles;
-  int nseg, shift[TC_MAX_SEG];   // taps of the gated conv (all on the same input tensor)
+  int nseg, shift[TC_MAX_TAPS];   // taps of the gated conv (all on the same input tensor)
   int Cin, D, R, has_res;
   const float* bias_g; const float* cbias; const float* bias_r;   // [2D], [B][2D] or null, [R]
   unsigned long long pol_a, pol_w, pol_z, pol_g, pol_o;
@@ -408,7 +408,7 @@ tc_block_fwd_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
 }
 
 struct TcBlockDesc {
-  int B, T, nseg, shift[TC_MAX_SEG], Cin, D, R, has_res;
+  int B, T, nseg, shift[TC_MAX_TAPS], Cin, D, R, has_res;
   const bf16* A; int lda;            // input of the gated conv (B,T,Cin)
   const bf16* X; int ldx;            // residual / block input (B,T,R)
   const bf16* W1; int k1;            // gate weights, tile-interleaved [2D][nseg*Cin]
@@ -476,7 +476,7 @@ static int tc_block_fwd_launch(TmapCache& tc, cudaStream_t st, const TcBlockDesc
 // supported shapes: D in {128, 256}, R in {128, 256}, Cin % 64 == 0; returns -100 when the caller should use the
 // separate gate / conv1 kernels instead
 static inline int tc_block_fwd(TmapCache& tc, cudaStream_t st, const TcBlockDesc& d) {
-  if (d.Cin % 64 != 0 || d.nseg < 1 || d.nseg > TC_MAX_SEG) return -100;
+  if (d.Cin % 64 != 0 || d.nseg < 1 || d.nseg > TC_MAX_TAPS) return -100;
   if (d.D == 256 && d.R == 256) return tc_block_fwd_launch<256, 256>(tc, st, d);
   if (d.D == 128 && d.R == 128) return tc_block_fwd_launch<128, 128>(tc, st, d);
   return -100;

@@ -32,7 +32,7 @@
 #define TC_STACK_MAX_LAYERS 256
 struct alignas(128) TcStackLayer {
   CUtensorMap tmA, tmX, tmW1, tmW2, tmZf, tmZs, tmG, tmO, tmOd;
-  int shift[TC_MAX_SEG];
+  int shift[TC_MAX_TAPS];
   const float* bias_g; const float* cbias; const float* bias_r;
   const uint8_t* mask_next;      // dropout keep-mask of the next block's conv branch, or null (tmOd: its masked input)
   int kind;                      // 0: gated conv + gate + conv1 (+ residual) = block tail; 1: plain conv + bias + activation
@@ -587,7 +587,7 @@ static int tc_stack_build_t(TmapCache& tc, const std::vector<TcBlockDesc>& descs
         t.tmOd = *mOd; t.mask_next = d.mask_next;
       }
     }
-    for (int s = 0; s < TC_MAX_SEG; ++s) t.shift[s] = s < d.nseg ? d.shift[s] : 0;
+    for (int s = 0; s < TC_MAX_TAPS; ++s) t.shift[s] = s < d.nseg ? d.shift[s] : 0;
     t.bias_g = d.bias_g; t.cbias = d.cbias; t.bias_r = d.bias_r;
   }
   const TcBlockDesc& d0 = descs[0];

@@ -42,7 +42,7 @@
 
 struct alignas(128) TcStackBwdLayer {
   CUtensorMap tmDX, tmDS, tmWdg, tmZf, tmZs, tmDZ, tmWb, tmDXp, tmO;   // tmZf / tmZs: the cached gate derivative coefficients P / Q; tmDXp: d x_out as 32-column panels
-  int shift[TC_MAX_SEG];      // row shift of tap k (k < nseg - 1: positive; tap nseg - 1: 0)
+  int shift[TC_MAX_TAPS];      // row shift of tap k (k < nseg - 1: positive; tap nseg - 1: 0)
   int has_dx, has_ds, has_res;
   int wait_dx;                // d x_out_l is written by this launch (every block but the last): acquire its tile flag first
   const uint8_t* mask;        // dropout keep-mask of this block's conv branch [b*T+t][R], or null
@@ -730,7 +730,7 @@ tc_stack_bwd_kernel(const TcStackBwdLayer* __restrict__ layers, int* __restrict_
 
 // ---------------------------------------------------------------- host side
 struct TcStackBwdDesc {       // one block
-  int B, T, nseg, shift[TC_MAX_SEG], D, R, S;
+  int B, T, nseg, shift[TC_MAX_TAPS], D, R, S;
   const bf16* dxo;            // d x_out_l (B,T,R) or null (last block under use_skip)
   const bf16* dskip; int lds; // d skip (B,T,S) or null
   const bf16* z;              // cached gate pre-activations (B,T,2D)
@@ -770,7 +770,7 @@ static int tc_stack_bwd_build_t(TmapCache& tc, const std::vector<TcStackBwdDesc>
     const CUtensorMap* mWb = tc.get(d.Wb, 2, bd, bs, bb);
     if (!mO || !mWb) return -10;
     t.tmO = *mO; t.tmWb = *mWb; t.tmDXp = *mO;
-    for (int s = 0; s < TC_MAX_SEG; ++s) t.shift[s] = s < d.nseg ? d.shift[s] : 0;
+    for (int s = 0; s < TC_MAX_TAPS; ++s) t.shift[s] = s < d.nseg ? d.shift[s] : 0;
     t.mask = d.mask;
     t.kind = d.plain ? 1 : 0; t.out_mode = d.out_mode; t.act = d.act; t.in_flag_layer = d.out_mode == 1 ? d.ein_layer : -1;
     if (d.out_mode) {

@@ -300,7 +300,7 @@ __global__ void __launch_bounds__(256) tc_wgrad_group_finish(const TcWgFinParams
 
 // ---------------------------------------------------------------- host side: plan
 struct TcWgJobDesc {         // one weight-gradient problem dW[k * Cin + c, n] = sum_{b,t} A[(b, t + shift_k), c] * G[(b, t), n]
-  const bf16* A; int lda; int cin; int ntaps; int shift[TC_MAX_SEG];
+  const bf16* A; int lda; int cin; int ntaps; int shift[TC_MAX_TAPS];
   const bf16* G; int ldg; int N;
   float* dst; const float* w;            // [ntaps * cin][N] fp32 gradient (Keras layout), weights for L2 (or null)
   float* bias;                           // [N] column sums of G, or null

@@ -308,6 +308,15 @@ __global__ void convert_kernel(const TI* __restrict__ in, TO* __restrict__ out, 
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n) out[i] = from_f<TO>(to_f(in[i]));
 }
+// out[r][c] = in[r][c] for c < cin, 0 for cin <= c < cout: rows of width cin widened to cout (zero padding)
+template <class TI, class TO>
+__global__ void convert_pad_kernel(const TI* __restrict__ in, int cin, TO* __restrict__ out, int cout, long long rows) {
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= rows * cout) return;
+  const long long r = i / cout;
+  const int c = (int)(i % cout);
+  out[i] = from_f<TO>(c < cin ? to_f(in[r * cin + c]) : 0.f);
+}
 template <class T>
 __global__ void add2_kernel(const T* __restrict__ a, const T* __restrict__ b, T* __restrict__ out, long long n) {
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;

@@ -96,6 +96,12 @@ struct BlockP {
   // x_out = [g | x] . [Wr ; I] + b  (the x . I products are exact in the fp32 accumulator).  Takes the residual
   // read out of the epilogue, whose TMA input ring was the long pole of this kernel (3 k cycles per tile).
   bf16* Wres16 = nullptr;
+  // layer handles with conditioning: a conditioning SEQUENCE (B,T,Cc) enters the gated conv's contraction as one more
+  // segment (shift 0), so its weights follow the taps in the same packed operand
+  float* Wfc = nullptr;                   // fp32 [K*cin + Cc][Npad]: gated conv rows, then Wc rows (same interleaved columns)
+  float* Wct = nullptr; int Ccpad = 0;    // fp32 [2D][Ccpad]: Wc^T, operand of d cond = dz Wc^T
+  bf16* Wfc16 = nullptr; int Kfc16 = 0;   // bf16 [N16][K*cin + Ccs]: gated conv, then Wc zero-padded to Ccs columns
+  bf16* Wct16 = nullptr; int Cc16 = 0, tileCc16 = 0;   // bf16 [Cc16][2D]: Wc, B operand of d cond
 };
 
 struct Arena {
@@ -187,6 +193,13 @@ struct wn_handle {
   bool fwd_valid = false;
   bool layer_fwd_valid[WN_MAX_DILATIONS] = {};
   bool layer_drop[WN_MAX_DILATIONS] = {};     // wn_layer_forward_ex ran block l with dropout active (its adjoint must too)
+  // conditioning sequences of the layer API (wn_layer_forward_seq); buffers exist on layer handles with conditioning only
+  int Ccs = 0;                            // stored width of a sequence: Cc (fp32), Cc rounded up to 32 (bf16)
+  std::vector<void*> cseq;                // bf16: [block] zero-padded copy of the last sequence (rows, Ccs)
+  float* cseq_bias = nullptr;             // [L][2D] gated-conv bias + conv_cond bias
+  float* cseq_dw = nullptr;               // bf16: [Ccs][2D] weight gradient of the padded contraction (first Cc rows = d Wc)
+  const void* layer_cseq[WN_MAX_DILATIONS] = {};   // sequence (in T, width Ccs) of block l's last forward; null: time-constant
+  const void* cond_seq = nullptr;         // the sequence of the block being enqueued (null: time-constant or no conditioning)
   const float* last_cond = nullptr;
   long long launches = 0;
   // profiling
@@ -338,7 +351,7 @@ static int validate_config(const wn_config& c) {
   if (c.sampling_function == WN_CATEGORICAL && c.num_mixtures != 0) { set_err("Categorical sampling cannot be used with mixtures."); return WN_ERR_VALUE; }
   if (c.has_head && c.sampling_function != WN_CATEGORICAL && c.num_mixtures == 0) { set_err("mixture sampling needs num_mixtures"); return WN_ERR_VALUE; }
   if (c.channels < 1 || c.max_batch < 1 || c.max_time < 1) { set_err("channels / max_batch / max_time must be positive"); return WN_ERR_VALUE; }
-  if (c.kernel_size > WN_MAX_SEG) { set_err("kernel_size > %d not built", WN_MAX_SEG); return WN_ERR_UNSUPPORTED; }
+  if (c.kernel_size > WN_MAX_TAPS) { set_err("kernel_size > %d not built", WN_MAX_TAPS); return WN_ERR_UNSUPPORTED; }
   if (c.num_mixtures > WN_MAX_MIX) { set_err("num_mixtures > %d not built", WN_MAX_MIX); return WN_ERR_UNSUPPORTED; }
   if (c.blocks * c.layers_per_block > WN_MAX_DILATIONS) { set_err("too many dilated convs"); return WN_ERR_UNSUPPORTED; }
   if (c.n_mapping < 0 || c.n_mapping > WN_MAX_LIST || c.n_final < 0 || c.n_final > WN_MAX_LIST) { set_err("list too long"); return WN_ERR_VALUE; }
@@ -394,6 +407,19 @@ static void layout_buffers(wn_handle* h) {
       b.Dpad = n16;
       b.Wdg16 = (bf16*)P.take((size_t)n16 * rup(rs, 64) * 2);
       if (h->cfg.use_residual) b.Wres16 = (bf16*)P.take((size_t)b.conv1.N16 * (h->D + h->R) * 2);
+    }
+    if (b.has_cond && h->Ccs > 0) {
+      const ConvP& c = b.stack.back();
+      if (!bf) {
+        b.Wfc = (float*)P.take((size_t)(c.K * c.cin + h->Cc) * c.Npad * 4);
+        b.Ccpad = rup(h->Cc, 64);
+        b.Wct = (float*)P.take((size_t)c.cout * b.Ccpad * 4);
+      } else {
+        b.Kfc16 = c.K * c.cin + h->Ccs;
+        b.Wfc16 = (bf16*)P.take((size_t)c.N16 * b.Kfc16 * 2);
+        tc_pick_tile(h->Cc, false, &b.Cc16, &b.tileCc16);
+        b.Wct16 = (bf16*)P.take((size_t)b.Cc16 * c.cout * 2);
+      }
     }
   }
   for (auto& c : h->head) lay_conv(c);
@@ -476,6 +502,7 @@ static void layout_buffers(wn_handle* h) {
     for (auto& c : b.stack) upd((long long)c.K * c.cin, c.cout);
     upd(D, R);
     if (b.has_skip) upd(D, h->S);
+    if (b.has_cond && h->Ccs > 0) upd(h->Ccs, 2 * D);
   }
   for (auto& c : h->head) upd(c.cin, c.cout);
   h->wg_partial_elems = maxkn * WN_MAX_WGRAD_SPLITS;
@@ -486,6 +513,7 @@ static void layout_buffers(wn_handle* h) {
     int max_mt = 1;
     auto mt = [&](int K, int cin) { const int m = K * cdiv(cin, 128); if (m > max_mt) max_mt = m; };
     for (auto& b : h->blocks) { for (auto& c : b.stack) mt(c.K, c.cin); mt(1, D); }
+    if (h->Ccs > 0) mt(1, h->Ccs);
     for (auto& c : h->head) mt(1, c.cin);
     h->cs_partial = (float*)W.take((size_t)tc_wgrad_cs_rows(h->maxB, h->maxT, max_mt) * (size_t)rup(nmax, 4) * 4 * 2);
     h->cs_partial_side = (float*)W.take((size_t)tc_wgrad_cs_rows(h->maxB, h->maxT, max_mt) * (size_t)rup(nmax, 4) * 4 * 2);
@@ -501,6 +529,14 @@ static void layout_buffers(wn_handle* h) {
     h->cb = (float*)W.take((size_t)L * h->maxB * 2 * D * 4);
     h->dcb = (float*)W.take((size_t)L * h->maxB * 2 * D * 4);
     h->dcond = (float*)W.take((size_t)h->maxB * (h->Cc > 0 ? h->Cc : 1) * 4);
+  }
+  if (h->Ccs > 0) {
+    h->cseq.assign(L, nullptr);
+    if (bf) {
+      for (int l = 0; l < L; ++l) h->cseq[l] = W.take(rows * h->Ccs * 2);
+      h->cseq_dw = (float*)W.take((size_t)h->Ccs * 2 * D * 4);
+    }
+    h->cseq_bias = (float*)W.take((size_t)L * 2 * D * 4);
   }
   h->l2_sum = (float*)W.take(16);
   if (h->cfg.dropout > 0.f) {
@@ -546,6 +582,8 @@ extern "C" int wn_create(const wn_config* cfg, wn_handle** out) {
   h->Cout = c.num_mixtures > 0 ? 3 * c.num_mixtures : (1 << c.bits);
   h->Cc = 0;
   if (c.conditioning) h->Cc = c.n_mapping > 0 ? c.mapping_layers[c.n_mapping - 1] : c.cond_in;
+  // layer handles (no head) may be called with a conditioning sequence: model handles allocate nothing for it
+  if (c.conditioning && !c.has_head) h->Ccs = c.precision == WN_BF16 ? rup(h->Cc, 32) : h->Cc;
   h->maxB = c.max_batch;
   h->maxT = c.max_time;
   // dilation schedule (model.py:79-81) unless given explicitly (bare WaveNetLayer)
@@ -630,7 +668,7 @@ extern "C" int wn_create(const wn_config* cfg, wn_handle** out) {
   // ---- grouped weight gradients: bf16 tier, separate skip projection (or none), widths in whole 256-channel pair tiles
   if (c.precision == WN_BF16) {
     const char* e = getenv("WN_TC_GROUP_WGRAD");
-    bool ok = !(e && e[0] == '0') && h->R % 256 == 0 && h->D % 256 == 0 && h->K <= TC_MAX_SEG;
+    bool ok = !(e && e[0] == '0') && h->R % 256 == 0 && h->D % 256 == 0 && h->K <= TC_MAX_TAPS;
     for (auto& b : h->blocks) if (b.has_skip && h->S % 256 != 0) ok = false;
     if (ok) {
       // d z, d x_out (and d x_out + d skip when the skip aliases conv1, and the pre-stack gradients of multi-dilation
@@ -878,6 +916,21 @@ extern "C" int wn_params_changed(wn_handle* h, void* stream) {
         pack_emit(h, nullptr, 0, 0, b.Wres16 + h->D, h->D + h->R, 4, 0, 0, 0, h->R);
       }
     }
+    if (b.Wfc || b.Wfc16) {
+      // conditioning-sequence operands: [gated conv taps ; Wc] with the gated conv's column order, and Wc for d cond
+      const ConvP& c = b.stack.back();
+      const int ktot = c.K * c.cin, Cc = h->Cc;
+      const float* Wc = P + h->params[b.cw_idx].offset;
+      if (!bf) {
+        pack_launch<float>(h, st, W(c), ktot, c.cout, b.Wfc, c.Npad, 2, 64, c.cout / 2, c.Npad);
+        pack_launch<float>(h, st, Wc, Cc, c.cout, b.Wfc + (size_t)ktot * c.Npad, c.Npad, 2, 64, c.cout / 2, c.Npad);
+        pack_launch<float>(h, st, Wc, Cc, c.cout, b.Wct, b.Ccpad, 1, 0, 0, 0);
+      } else {
+        pack_emit(h, W(c), ktot, c.cout, b.Wfc16, b.Kfc16, 3, c.tileN16, c.cout / 2, c.N16, (long long)c.N16 * ktot);
+        pack_emit(h, Wc, Cc, c.cout, b.Wfc16 + ktot, b.Kfc16, 3, c.tileN16, c.cout / 2, c.N16, (long long)c.N16 * Cc);
+        pack_launch<bf16>(h, st, Wc, Cc, c.cout, b.Wct16, c.cout, 0, 0, 0, 0);
+      }
+    }
   }
   for (auto& c : h->head) pack_conv(c);
   CK(cudaMalloc(&h->d_pack_jobs, h->pack_jobs.size() * sizeof(PackJob)));
@@ -895,7 +948,7 @@ struct GemmH {
   const float* W32 = nullptr; int Npad = 0;     // fp32: [ktot][Npad]
   const bf16* W16 = nullptr; int ktot16 = 0; int N16 = 0; int tile16 = 0;  // bf16: [N16][ktot16]
   int l2_a = 0, l2_in[2] = {0, 0}, l2_out[3] = {0, 0, 0};   // bf16 tier: L2 policy codes (TC_L2_*), see tc_common.cuh
-  int l2_seg[WN_MAX_SEG] = {-1, -1, -1, -1};                // per-segment override of l2_a
+  int l2_seg[WN_MAX_SEG] = {-1, -1, -1, -1, -1};            // per-segment override of l2_a
 };
 
 // bf16 tier: map the generic epilogue description onto the TMA-staged tcgen05 kernel (tc_epilogues.cuh);
@@ -1189,7 +1242,7 @@ static int block_forward(wn_handle* h, cudaStream_t st, int l, const void* x_in,
     } else {
       if constexpr (sizeof(T) == 2) {
         // bf16 tier: gated conv + gate + conv1 (+ residual) as ONE kernel when the shapes allow (gemm_tc_block.cuh)
-        if (h->use_fused_fwd && b.Wres16 && h->cfg.use_residual && tc_cta_group() == 2 && c.K <= TC_MAX_SEG) {
+        if (h->use_fused_fwd && b.Wres16 && h->cfg.use_residual && tc_cta_group() == 2 && c.K <= TC_MAX_TAPS && !h->cond_seq) {
           TcBlockDesc d{};
           d.B = B; d.T = Tn; d.nseg = c.K; d.Cin = c.cin; d.D = h->D; d.R = h->R; d.has_res = 1;
           for (int k = 0; k < c.K; ++k) d.shift[k] = -(c.K - 1 - k) * c.dil;
@@ -1215,6 +1268,12 @@ static int block_forward(wn_handle* h, cudaStream_t st, int l, const void* x_in,
       ep.ldg = h->D; ep.bias = P_(h, c.b_idx);
       ep.cbias = has_cb ? h->cb + (size_t)l * h->maxB * 2 * h->D : nullptr;
       ep.D = h->D; ep.vec = vec_ok<T>(h->D);
+      if (h->cond_seq) {
+        // conditioning sequence: conv_cond is one more segment of the contraction (layers.py:203-204), bc joins the bias
+        g.seg[g.nseg++] = SegH{h->cond_seq, h->Ccs, 0, h->Ccs};
+        g.W32 = b.Wfc; g.W16 = b.Wfc16; g.ktot16 = b.Kfc16;
+        ep.bias = h->cseq_bias + (size_t)l * 2 * h->D;
+      }
       // z is not needed before the backward pass (streaming store); g feeds conv1 next; x_in is conv1's residual
       g.l2_a = depth == 1 ? TC_L2_LAST : TC_L2_NORMAL;
       g.l2_out[0] = g.l2_out[1] = TC_L2_FIRST; g.l2_out[2] = TC_L2_LAST;
@@ -1300,7 +1359,7 @@ static int model_forward(wn_handle* h, cudaStream_t st, const float* x, int ldx,
     for (auto& b : h->blocks) {
       if (!ok) break;
       const ConvP& cv = b.stack.back();
-      ok = b.Wres16 != nullptr && cv.tileN16 == 256 && cv.K <= TC_MAX_SEG && cv.cin % 64 == 0;
+      ok = b.Wres16 != nullptr && cv.tileN16 == 256 && cv.K <= TC_MAX_TAPS && cv.cin % 64 == 0;
       for (size_t j = 0; ok && j + 1 < b.stack.size(); ++j) {
         const ConvP& pc = b.stack[j];
         // plain layers run as one 256-wide tile per m tile: D = 256 only; all convs share K and the input width
@@ -1644,7 +1703,7 @@ static int block_backward(wn_handle* h, cudaStream_t st, int l, const void* x_in
     } else {
       WgradH w{};
       w.bias_dst = G_(h, c.b_idx);
-      if (j == depth - 1 && b.has_cond) { w.per_batch = h->dcb + (size_t)l * h->maxB * 2 * D; w.ldpb = 2 * D; }
+      if (j == depth - 1 && b.has_cond && !h->cond_seq) { w.per_batch = h->dcb + (size_t)l * h->maxB * 2 * D; w.ldpb = 2 * D; }
       w.B = B; w.T = Tn; w.N = c.cout; w.G = dcur; w.ldg = dcw; w.nseg = c.K;
       for (int k = 0; k < c.K; ++k) w.seg[k] = SegH{a_in, a_w, -(c.K - 1 - k) * c.dil, c.cin};
       w.dst = G_(h, c.w_idx); w.w = P_(h, c.w_idx); w.l2coef = l2coef;
@@ -1809,7 +1868,7 @@ static int model_backward(wn_handle* h, cudaStream_t st, const float* x, int ldx
   bool sb_ok = false;
   if constexpr (sizeof(T) == 2) {
     sb_ok = group && !cat && h->use_stack_bwd && tc_cta_group() == 2 && h->L >= 2 && h->D == h->R && (h->D == 256 || h->D == 128) &&
-            h->K <= TC_MAX_SEG && B * cdiv(Tn, 256) > tc_num_sms() / 2;
+            h->K <= TC_MAX_TAPS && B * cdiv(Tn, 256) > tc_num_sms() / 2;
     for (auto& b : h->blocks) {
       if (!sb_ok) break;
       // multi-dilation blocks (plain conv layers of the launch): all convs 256 wide
@@ -2808,8 +2867,8 @@ extern "C" int wn_train_step_host(wn_handle* h, const float* frames_host, const 
 
 // ---------------------------------------------------------------- layer-level API
 template <class T>
-static int layer_fwd_entry(wn_handle* h, int l, const float* x, const float* cond, int B, int Tn, int training, float* x_out, float* skip,
-                           cudaStream_t st) {
+static int layer_fwd_entry(wn_handle* h, int l, const float* x, const float* cond, bool seq, int B, int Tn, int training, float* x_out,
+                           float* skip, cudaStream_t st) {
   // WaveNetLayer.call(inputs, training): Keras Dropout is active only under training=True (layers.py:195-196)
   h->drop_active = training && h->cfg.dropout > 0.f;
   h->layer_drop[l] = h->drop_active;
@@ -2827,7 +2886,25 @@ static int layer_fwd_entry(wn_handle* h, int l, const float* x, const float* con
   }
   xin = slot;
   bool has_cb = false;
-  if (h->blocks[l].has_cond) {
+  h->layer_cseq[l] = nullptr;
+  if (seq) {
+    // (B,T,Cc) sequence: the bf16 tier contracts a zero-padded bf16 copy, the fp32 tier the caller's buffer itself
+    const BlockP& b = h->blocks[l];
+    const void* cs = cond;
+    if constexpr (sizeof(T) == 2) {
+      LaunchScope ls(h, st, CLS_MISC);
+      const long long rows = (long long)B * Tn;
+      convert_pad_kernel<float, bf16><<<cdiv(rows * h->Ccs, 256), 256, 0, st>>>(cond, h->Cc, (bf16*)h->cseq[l], h->Ccs, rows);
+      cs = h->cseq[l];
+    }
+    {
+      LaunchScope ls(h, st, CLS_MISC);
+      add2_kernel<float><<<cdiv(2 * h->D, 256), 256, 0, st>>>(P_(h, b.stack.back().b_idx), P_(h, b.cb_idx), h->cseq_bias + (size_t)l * 2 * h->D,
+                                                              2 * h->D);
+    }
+    h->layer_cseq[l] = cs;
+    h->cond_seq = cs;
+  } else if (h->blocks[l].has_cond) {
     if (!cond) { set_err("Conditioning must be provided."); return WN_ERR_VALUE; }
     h->last_cond = cond;
     cond_bias_block(h, st, l, cond, B);
@@ -2845,22 +2922,37 @@ static int layer_fwd_entry(wn_handle* h, int l, const float* x, const float* con
   return WN_OK;
 }
 
-extern "C" int wn_layer_forward_ex(wn_handle* h, int block, const float* x_dev, const float* cond_dev, int B, int T, int training, float* x_out_dev,
-                                   float* skip_dev, void* stream) {
-  RET(check_bt(h, B, T));
-  if (block < 0 || block >= h->L || !x_dev || !x_out_dev) { set_err("bad layer arguments"); return WN_ERR_VALUE; }
-  if (training && h->cfg.dropout >= 1.f) { set_err("dropout must be < 1 for training"); return WN_ERR_VALUE; }
+static int layer_forward_call(wn_handle* h, int block, const float* x_dev, const float* cond_dev, bool seq, int B, int T, int training,
+                              float* x_out_dev, float* skip_dev, void* stream) {
   CK(cudaSetDevice(h->cfg.device));
   h->launches = 0;
   cudaStream_t st = (cudaStream_t)stream;
-  int r = h->cfg.precision == WN_BF16 ? layer_fwd_entry<bf16>(h, block, x_dev, cond_dev, B, T, training, x_out_dev, skip_dev, st)
-                                      : layer_fwd_entry<float>(h, block, x_dev, cond_dev, B, T, training, x_out_dev, skip_dev, st);
+  int r = h->cfg.precision == WN_BF16 ? layer_fwd_entry<bf16>(h, block, x_dev, cond_dev, seq, B, T, training, x_out_dev, skip_dev, st)
+                                      : layer_fwd_entry<float>(h, block, x_dev, cond_dev, seq, B, T, training, x_out_dev, skip_dev, st);
   h->drop_active = false;
+  h->cond_seq = nullptr;
   RET(r);
   CK(cudaGetLastError());
   h->lastB = B; h->lastT = T;
   h->layer_fwd_valid[block] = true;
   return WN_OK;
+}
+extern "C" int wn_layer_forward_ex(wn_handle* h, int block, const float* x_dev, const float* cond_dev, int B, int T, int training, float* x_out_dev,
+                                   float* skip_dev, void* stream) {
+  RET(check_bt(h, B, T));
+  if (block < 0 || block >= h->L || !x_dev || !x_out_dev) { set_err("bad layer arguments"); return WN_ERR_VALUE; }
+  if (training && h->cfg.dropout >= 1.f) { set_err("dropout must be < 1 for training"); return WN_ERR_VALUE; }
+  return layer_forward_call(h, block, x_dev, cond_dev, false, B, T, training, x_out_dev, skip_dev, stream);
+}
+extern "C" int wn_layer_forward_seq(wn_handle* h, int block, const float* x_dev, const float* cond_dev, int B, int T, int training,
+                                    float* x_out_dev, float* skip_dev, void* stream) {
+  RET(check_bt(h, B, T));
+  if (block < 0 || block >= h->L || !x_dev || !x_out_dev) { set_err("bad layer arguments"); return WN_ERR_VALUE; }
+  if (!cond_dev) { set_err("conditioning sequence is NULL"); return WN_ERR_VALUE; }
+  if (!h->blocks[block].has_cond) { set_err("block %d was built without conditioning", block); return WN_ERR_VALUE; }
+  if (h->Ccs == 0) { set_err("conditioning sequences are built for layer handles (has_head = 0) only"); return WN_ERR_UNSUPPORTED; }
+  if (training && h->cfg.dropout >= 1.f) { set_err("dropout must be < 1 for training"); return WN_ERR_VALUE; }
+  return layer_forward_call(h, block, x_dev, cond_dev, true, B, T, training, x_out_dev, skip_dev, stream);
 }
 extern "C" int wn_layer_forward(wn_handle* h, int block, const float* x_dev, const float* cond_dev, int B, int T, float* x_out_dev, float* skip_dev,
                                 void* stream) {
@@ -2870,6 +2962,7 @@ extern "C" int wn_layer_forward(wn_handle* h, int block, const float* x_dev, con
 template <class T>
 static int layer_bwd_entry(wn_handle* h, int l, const float* dxo, const float* dsk, float* dx, float* dcond, cudaStream_t st) {
   h->drop_active = h->layer_drop[l];   // adjoint of the forward this block last ran (its keep-mask is still in drop_mask)
+  h->cond_seq = h->layer_cseq[l];      // ... and its conditioning sequence, if it had one
   const int B = h->lastB, Tn = h->lastT;
   const long long nR = (long long)B * Tn * h->R, nS = (long long)B * Tn * h->Sp;
   const void *dxo_t = nullptr, *dsk_t = nullptr;
@@ -2889,7 +2982,28 @@ static int layer_bwd_entry(wn_handle* h, int l, const float* dxo, const float* d
     LaunchScope ls(h, st, CLS_MISC);
     convert_kernel<T, float><<<cdiv(nR, 256), 256, 0, st>>>((const T*)h->dxB, dx, nR);
   }
-  if (h->blocks[l].has_cond) {
+  if (h->cond_seq) {
+    const BlockP& b = h->blocks[l];
+    const int n = 2 * h->D, Cc = h->Cc;
+    // d Wc = sum_{b,t} c^T dz and d bc = column sums of dz: the sequence against the gate adjoint block_backward left in h->dz
+    // (bf16: the contraction runs over the padded width, its first Cc rows are d Wc)
+    WgradH w{};
+    w.B = B; w.T = Tn; w.N = n; w.G = h->dz; w.ldg = n; w.nseg = 1; w.seg[0] = SegH{h->cond_seq, h->Ccs, 0, h->Ccs};
+    w.dst = sizeof(T) == 2 ? h->cseq_dw : G_(h, b.cw_idx); w.w = P_(h, b.cw_idx); w.l2coef = 0.f; w.bias_dst = G_(h, b.cb_idx);
+    RET(run_wgrad<T>(h, st, CLS_GEMM, w));
+    if (sizeof(T) == 2) CK(cudaMemcpyAsync(G_(h, b.cw_idx), h->cseq_dw, (size_t)Cc * n * 4, cudaMemcpyDeviceToDevice, st));
+    if (dcond) {
+      // d cond = dz Wc^T (B,T,Cc), fp32 straight into the caller's buffer
+      GemmH g;
+      g.B = B; g.T = Tn; g.N = Cc; g.nseg = 1;
+      g.seg[0] = SegH{h->dz, n, 0, n};
+      g.W32 = b.Wct; g.Npad = b.Ccpad;
+      g.W16 = b.Wct16; g.ktot16 = n; g.N16 = b.Cc16; g.tile16 = b.tileCc16;
+      typename EpiBiasActRes<T, float, sizeof(T) == 2>::Params ep{};
+      ep.out = dcond; ep.ldo = Cc; ep.bias = nullptr; ep.cbias = nullptr; ep.act = ACT_LINEAR; ep.res = nullptr; ep.N = Cc; ep.vec = vec_ok<float>(Cc);
+      RET((run_conv_gemm<T, EpiBiasActRes<T, float, sizeof(T) == 2>>(h, st, CLS_GEMM, g, ep)));
+    }
+  } else if (h->blocks[l].has_cond) {
     RET(cond_backward(h, st, nullptr, h->last_cond, B, l, 1, false, h->dcond, 0.f));
     if (dcond) CK(cudaMemcpyAsync(dcond, h->dcond, (size_t)B * h->Cc * 4, cudaMemcpyDeviceToDevice, st));
   }
@@ -2907,6 +3021,7 @@ extern "C" int wn_layer_backward(wn_handle* h, int block, const float* dx_out_de
   int r = h->cfg.precision == WN_BF16 ? layer_bwd_entry<bf16>(h, block, dx_out_dev, dskip_dev, dx_dev, dcond_dev, st)
                                       : layer_bwd_entry<float>(h, block, dx_out_dev, dskip_dev, dx_dev, dcond_dev, st);
   h->drop_active = false;
+  h->cond_seq = nullptr;
   RET(r);
   CK(cudaGetLastError());
   return WN_OK;

@@ -5,6 +5,12 @@ Mirrors /root/reference/src/layers.py: same constructor kwargs (:10-20), `build`
 (:178-224), same ValueErrors.  The arithmetic runs in libwavenet_b200.so (`wn_layer_forward` /
 `wn_layer_backward`); torch only holds the device buffers.  `generate` (:226-290) is
 inference-only and out of scope.
+
+Conditioning (`condition=True`) takes either form the reference accepts: a (B,Cc) vector, or a (B,T,Cc)
+sequence that is constant in time, runs as a per-batch bias of the gated conv; a (B,T,Cc) sequence that
+varies in time (local conditioning, one feature vector per sample) runs through `wn_layer_forward_seq`,
+where conv_cond is one more segment of the gated conv's contraction.  `backward` returns `dcond` in the
+shape of the conditioning that ran: (B,Cc) for the time-constant forms, (B,T,Cc) for a sequence.
 """
 from __future__ import annotations
 
@@ -83,6 +89,7 @@ class WaveNetLayer:
     cfg.conditioning = 1 if self.condition else 0
     cfg.n_mapping = 0
     cfg.cond_in = int(cond_shape[-1]) if self.condition else 0
+    self._cond_in = cfg.cond_in
     cfg.dilation_bound = 1
     cfg.num_mixtures = 0
     cfg.sampling_function = 0
@@ -178,14 +185,19 @@ class WaveNetLayer:
       raise ValueError('input must be (batch, samples, channels)')
     B, T, _ = x.shape
     cond2 = None
+    seq = None
     if self.condition:
       cond = as_dev(cond, dev)
       if cond.dim() == 3:
         if cond.shape[1] != T:
           raise ValueError('Condition tensor must have the same length as input')
         if T > 1 and not bool((cond == cond[:, :1, :]).all()):
-          raise NotImplementedError('time-varying (local) conditioning is untested/broken upstream and not built')
-        cond2 = cond[:, 0, :].contiguous()
+          # local conditioning: conv_cond(cond) joins the gated conv's pre-activation at every step (layers.py:203-204)
+          if self.built and cond.shape[2] != self._cond_in:
+            raise ValueError(f'Condition tensor has {cond.shape[2]} channels; the layer was built for {self._cond_in}')
+          seq = cond
+        else:
+          cond2 = cond[:, 0, :].contiguous()
       else:
         cond2 = cond
     if not self.built or (B, T) != self._built_for and (B > self._built_for[0] or T > self._built_for[1]):
@@ -196,9 +208,13 @@ class WaveNetLayer:
     skip = torch.empty((B, T, skip_ch), dtype=torch.float32, device=dev)
     # training=True: inverted dropout on the conv branch, residual from the un-masked input (layers.py:192-196); the keep-mask
     # is a fresh Philox draw unless one was injected with set_dropout_mask (TF's RNG stream is not reproducible)
-    _lib.check(h.lib.wn_layer_forward_ex(h.h, 0, h.ptr(x), h.ptr(cond2), B, T, 1 if (training and self.dropout is not None) else 0,
-                                         h.ptr(x_out), h.ptr(skip), h.stream_ptr()))
-    self._last = (x, cond2)
+    drop = 1 if (training and self.dropout is not None) else 0
+    if seq is not None:
+      _lib.check(h.lib.wn_layer_forward_seq(h.h, 0, h.ptr(x), h.ptr(seq), B, T, drop, h.ptr(x_out), h.ptr(skip), h.stream_ptr()))
+      self._last = (x, seq)   # the library reads the sequence again in backward
+    else:
+      _lib.check(h.lib.wn_layer_forward_ex(h.h, 0, h.ptr(x), h.ptr(cond2), B, T, drop, h.ptr(x_out), h.ptr(skip), h.stream_ptr()))
+      self._last = (x, cond2)
     return x_out, skip
 
   __call__ = call
