@@ -53,7 +53,7 @@ def _run(kw, B, T, group, env=None):
     outs = []
     for _ in range(3):   # eager (plan built), eager (side launches), graph replay
       out = m.train_step((x, cond) if cond is not None else x)
-      outs.append((out['loss'], m.get_grads()))
+      outs.append((out['loss'], m.get_grads(), int(m.handle.lib.wn_stack_backward_layers(m.handle.h))))
     return outs
   finally:
     for k, v in old.items():
@@ -114,6 +114,7 @@ def test_stack_backward_vs_per_block_chain():
   kw, B, T = CASES['side_launches']
   a = _run(kw, B, T, True, {'WN_TC_STACK_BWD': '1'})
   b = _run(kw, B, T, True)
+  assert a[0][2] > 0 and b[0][2] == 0, 'the stack-backward launch must be held against the per-block chain'
   assert a[0][0] == b[0][0]
   for i in (1, 2):
     assert a[i][0] == a[0][0]

@@ -34,7 +34,7 @@ from tests.util import oracle_config, rel_err, rel_l2
 TILE = 256
 COND_IN = 109
 B200_PAIRS = 74                 # 148 SMs
-SB_BAND = 128                   # default WN_TC_SB_BAND of the stack backward
+SB_BAND = 128                   # band target of the stack backward (m tiles per band)
 
 W256 = dict(channels=256, final_layers_channels=[256])
 W128 = dict(channels=128, final_layers_channels=[128])

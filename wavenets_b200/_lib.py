@@ -44,7 +44,7 @@ class WnConfig(C.Structure):
 
 
 def lib_path() -> str:
-  # WN_LIB selects an alternative build of the same library (ablation builds under scripts/exp.sh)
+  # WN_LIB selects an alternative build of the same library (another revision from scripts/build_rev.sh, the precise / tl flavours)
   return os.environ.get('WN_LIB') or os.path.join(os.path.dirname(os.path.abspath(__file__)), 'libwavenet_b200.so')
 
 

@@ -34,13 +34,7 @@
 struct TcSeg { const bf16* A; int lda; int shift; int K; };
 // L2 policy per tensor of a launch: 0 = normal, 1 = evict_first (streaming), 2 = evict_last (the next kernel reads it)
 enum { TC_L2_NORMAL = 0, TC_L2_FIRST = 1, TC_L2_LAST = 2 };
-static inline int tc_l2_hints_on() {
-  static int on = -1;
-  if (on < 0) { const char* e = getenv("WN_TC_L2_HINTS"); on = (e && e[0] == '0') ? 0 : 1; }
-  return on;
-}
 static inline unsigned long long tc_policy(int code) {
-  if (!tc_l2_hints_on()) return TC_POL_NORMAL;
   return code == TC_L2_FIRST ? TC_POL_FIRST : (code == TC_L2_LAST ? TC_POL_LAST : TC_POL_NORMAL);
 }
 struct TcGemmDesc {
@@ -93,23 +87,13 @@ static inline void tc_pack_gate_T(cudaStream_t st, const float* src, int ktot, i
   tc_pack_gate_T_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(src, ktot, cout, dst, ld, tile, D, n16);
 }
 
-// programmatic dependent launch of the GEMM-class kernels (WN_TC_PDL=0 turns it off for A/B runs)
-static inline int tc_pdl_on() {
-  static int on = -1;
-  if (on < 0) { const char* e = getenv("WN_TC_PDL"); on = (e && e[0] == '0') ? 0 : 1; }
-  return on;
-}
+// cluster shape + programmatic dependent launch of the GEMM-class kernels
 static inline int tc_launch_attrs(cudaLaunchAttribute* attr, int cluster) {
-  int n = 0;
-  attr[n].id = cudaLaunchAttributeClusterDimension;
-  attr[n].val.clusterDim.x = cluster; attr[n].val.clusterDim.y = 1; attr[n].val.clusterDim.z = 1;
-  ++n;
-  if (tc_pdl_on()) {
-    attr[n].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[n].val.programmaticStreamSerializationAllowed = 1;
-    ++n;
-  }
-  return n;
+  attr[0].id = cudaLaunchAttributeClusterDimension;
+  attr[0].val.clusterDim.x = cluster; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
+  attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr[1].val.programmaticStreamSerializationAllowed = 1;
+  return 2;
 }
 
 // ---------------------------------------------------------------- conv GEMM kernel
@@ -284,11 +268,10 @@ static inline const CUtensorMap* tc_atom_map(TmapCache& tc, const bf16* A, int l
 // The same 4 rounds fit on 64 pairs; the SMs left over can run other work (the side-stream weight gradients) meanwhile.
 // g_tc_balance: 0 = always the whole GPU, 1 = the fewest CTAs (pairs) that keep the number of rounds.
 // The switch belongs to the pass a host thread is enqueuing (set and cleared around the backward chain), so it is per thread:
-// handles driven from different threads do not see each other's setting.  WN_TC_BALANCE_GRID=1 forces it for every launch.
+// handles driven from different threads do not see each other's setting.
 static thread_local int g_tc_balance = 0;
-static int g_tc_balance_env = 0;
 static inline int tc_balanced_slots(int tiles, int slots) {
-  if (!(g_tc_balance || g_tc_balance_env) || tiles <= slots) return slots;
+  if (!g_tc_balance || tiles <= slots) return slots;
   const int rounds = (tiles + slots - 1) / slots;
   return (tiles + rounds - 1) / rounds;
 }
@@ -353,29 +336,26 @@ struct TcStagedParams {
 
 // IN_PANELS: capacity of the epilogue-input ring in half-panels (slots = IN_PANELS / active inputs, decided at
 // run time); OUT_SLOTS: output slots of NOUT half-panels each.
-// CG: CTAs per MMA (cta_group).  CG == 2: a CTA pair works on 256 rows x BN columns; each CTA stages its own
-// 128 rows of A and HALF of the W tile, so one k-step moves 32 KB per SM instead of 48 KB for the same FLOPs
-// (the conv GEMMs at cta_group::1 top out on L2 -> SM bandwidth, profiles/README.md).
-template <int BN, int NIN, int NOUT, int IN_PANELS, int OUT_SLOTS_, int CG = 1> struct TcStagedCfg {
+// CTA pairs (cta_group::2): a pair works on 256 rows x BN columns; each CTA stages its own 128 rows of A and HALF
+// of the W tile, so one k-step moves 32 KB per SM instead of 48 KB for the same FLOPs (the conv GEMMs at
+// cta_group::1 top out on L2 -> SM bandwidth, profiles/README.md).
+template <int BN, int NIN, int NOUT, int IN_PANELS, int OUT_SLOTS_> struct TcStagedCfg {
   static constexpr int BM = 128, BK = 64;
   static constexpr int A_BYTES = BM * BK * 2;
-  static constexpr int B_BYTES = (BN / CG) * BK * 2;
+  static constexpr int B_BYTES = (BN / 2) * BK * 2;
   static constexpr int STAGE_BYTES = A_BYTES + B_BYTES;
   static constexpr int PANEL = 128 * 64;                 // 128 rows x 32 bf16
   static constexpr int IN_MAX = IN_PANELS > 0 ? IN_PANELS : 1, OUT_SLOTS = OUT_SLOTS_;
   static constexpr int STAGING = (IN_PANELS + OUT_SLOTS * NOUT) * PANEL;
   static constexpr int MAX_SMEM = 232448;
   static constexpr int ST0 = (MAX_SMEM - 4096 - STAGING) / STAGE_BYTES;
-#ifndef TC_STAGES_CAP
-#define TC_STAGES_CAP 6
-#endif
-  static constexpr int STAGES = ST0 > TC_STAGES_CAP ? TC_STAGES_CAP : ST0;
+  static constexpr int STAGES = ST0 > 6 ? 6 : ST0;
   static constexpr int TMEM_COLS = 2 * BN < 32 ? 32 : 2 * BN;
   static constexpr int SMEM_BYTES = STAGES * STAGE_BYTES + STAGING + 1024 + 512 + 2048 /*bias tables (double-buffered)*/;
   static_assert(STAGES >= 2, "not enough shared memory for the mainloop ring");
 };
 
-template <class Epi, int BN, int CG>
+template <class Epi, int BN>
 __global__ void __launch_bounds__(384, 1)
 tc_conv_gemm_staged_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__ CUtensorMap tmA1, const __grid_constant__ CUtensorMap tmA2,
                            const __grid_constant__ CUtensorMap tmA3, const __grid_constant__ CUtensorMap tmA4, const __grid_constant__ CUtensorMap tmW,
@@ -383,21 +363,15 @@ tc_conv_gemm_staged_kernel(const __grid_constant__ CUtensorMap tmA0, const __gri
                            const __grid_constant__ CUtensorMap tmO0, const __grid_constant__ CUtensorMap tmO1, const __grid_constant__ CUtensorMap tmO2,
                            const TcGemmParams p, const TcStagedParams sp, const typename Epi::Params ep) {
   constexpr int NIN = Epi::NIN, NOUT = Epi::NOUT;
-  using Cfg = TcStagedCfg<BN, NIN, NOUT, Epi::kInPanels, Epi::kOutSlots, CG>;
+  using Cfg = TcStagedCfg<BN, NIN, NOUT, Epi::kInPanels, Epi::kOutSlots>;
   constexpr int STAGES = Cfg::STAGES;
   constexpr int NEPI = 8;
   constexpr int STEPS = Epi::kGate ? BN / 64 : BN / 32;   // 32 output columns per step
   // CTA pair: rank 0 leads (issues the MMAs, owns the barriers the pair synchronises on)
-  const uint32_t crank = CG == 2 ? cluster_ctarank() : 0u;
+  const uint32_t crank = cluster_ctarank();
   const bool leader = crank == 0;
-  const int tile_first = (int)blockIdx.x / CG, tile_stride = (int)gridDim.x / CG;
+  const int tile_first = (int)blockIdx.x / 2, tile_stride = (int)gridDim.x / 2;
   const int pair_row0 = (int)crank * Cfg::BM;     // first row of this CTA inside the pair's 256-row tile
-#ifdef TC_DEBUG_PAIR
-  if (threadIdx.x == 0) {
-    uint32_t nr; asm volatile("mov.u32 %0, %%cluster_nctarank;" : "=r"(nr));
-    printf("blk %d/%d crank %u nctarank %u CG %d tiles %d tiles_t %d\n", blockIdx.x, gridDim.x, crank, nr, CG, p.num_tiles, p.tiles_t);
-  }
-#endif
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
   uint8_t* in_ring = smem + STAGES * Cfg::STAGE_BYTES;
@@ -425,18 +399,15 @@ tc_conv_gemm_staged_kernel(const __grid_constant__ CUtensorMap tmA0, const __gri
   }
   if (warp == 1 && lane == 0) {
     for (int i = 0; i < STAGES; ++i) { mbar_init(&full_bar[i], 1); mbar_init(&empty_bar[i], 1); }
-    for (int i = 0; i < 2; ++i) { mbar_init(&tfull_bar[i], 1); mbar_init(&tempty_bar[i], NEPI * CG); }
+    for (int i = 0; i < 2; ++i) { mbar_init(&tfull_bar[i], 1); mbar_init(&tempty_bar[i], NEPI * 2); }
     for (int i = 0; i < Cfg::IN_MAX; ++i) { mbar_init(&in_full[i], 1); mbar_init(&in_empty[i], NEPI); }
     for (int i = 0; i < Cfg::OUT_SLOTS; ++i) mbar_init(&out_empty[i], 1);
     mbar_fence_init();
   }
-  if (warp == 2) {
-    if (CG == 2) tmem_alloc_pair<Cfg::TMEM_COLS>(tmem_ptr);
-    else tmem_alloc<Cfg::TMEM_COLS>(tmem_ptr);
-  }
+  if (warp == 2) tmem_alloc_pair<Cfg::TMEM_COLS>(tmem_ptr);
   tc_fence_before();
   __syncthreads();
-  if (CG == 2) cluster_sync_all();     // the peer's barriers are initialised before anything is signalled across the pair
+  cluster_sync_all();     // the peer's barriers are initialised before anything is signalled across the pair
   tc_fence_after();
   const uint32_t tmem_base = *tmem_ptr;
   // everything above touched only shared memory / TMEM; global data of the previous kernel is read below
@@ -449,7 +420,7 @@ tc_conv_gemm_staged_kernel(const __grid_constant__ CUtensorMap tmA0, const __gri
       int stage = 0; uint32_t phase = 0;
       for (int tile = tile_first; tile < p.num_tiles; tile += tile_stride) {
         const int nt = tile % p.n_tiles, mt = tile / p.n_tiles;
-        const int b = mt / p.tiles_t, t0 = (mt % p.tiles_t) * (Cfg::BM * CG) + pair_row0, n0 = nt * BN;
+        const int b = mt / p.tiles_t, t0 = (mt % p.tiles_t) * (Cfg::BM * 2) + pair_row0, n0 = nt * BN;
         int wk = 0;
         for (int o = 0; o < p.n_outer; ++o) {
           for (int s = 0; s < p.nseg; ++s) {
@@ -459,28 +430,10 @@ tc_conv_gemm_staged_kernel(const __grid_constant__ CUtensorMap tmA0, const __gri
             for (int k0 = 0; k0 < kseg; k0 += Cfg::BK) {
               mbar_wait(&empty_bar[stage], phase ^ 1);
               uint8_t* sa = smem + stage * Cfg::STAGE_BYTES;
-#ifdef TC_EXP_NO_TMA
-              mbar_arrive(&full_bar[stage]);
-#else
-              if (CG == 1) {
-                mbar_expect_tx(&full_bar[stage], Cfg::STAGE_BYTES);
-                tma_load_4d_h(sa, tm, &full_bar[stage], k0, tcoord, b, o, pol_as);
-                tma_load_2d_h(sa + Cfg::A_BYTES, &tmW, &full_bar[stage], wk + k0, n0, sp.pol_w);
-              } else {
-                // the leader's barrier counts the bytes of both CTAs' operand halves
-#if defined(TC_EXP_NO_W)
-                if (leader) mbar_expect_tx(&full_bar[stage], 2 * Cfg::A_BYTES);
-                tma_load_4d_pair_h(sa, tm, &full_bar[stage], k0, tcoord, b, o, pol_as);
-#elif defined(TC_EXP_NO_A)
-                if (leader) mbar_expect_tx(&full_bar[stage], 2 * Cfg::B_BYTES);
-                tma_load_2d_pair_h(sa + Cfg::A_BYTES, &tmW, &full_bar[stage], wk + k0, n0 + (int)crank * (BN / 2), sp.pol_w);
-#else
-                if (leader) mbar_expect_tx(&full_bar[stage], 2 * Cfg::STAGE_BYTES);
-                tma_load_4d_pair_h(sa, tm, &full_bar[stage], k0, tcoord, b, o, pol_as);
-                tma_load_2d_pair_h(sa + Cfg::A_BYTES, &tmW, &full_bar[stage], wk + k0, n0 + (int)crank * (BN / 2), sp.pol_w);
-#endif
-              }
-#endif
+              // the leader's barrier counts the bytes of both CTAs' operand halves
+              if (leader) mbar_expect_tx(&full_bar[stage], 2 * Cfg::STAGE_BYTES);
+              tma_load_4d_pair_h(sa, tm, &full_bar[stage], k0, tcoord, b, o, pol_as);
+              tma_load_2d_pair_h(sa + Cfg::A_BYTES, &tmW, &full_bar[stage], wk + k0, n0 + (int)crank * (BN / 2), sp.pol_w);
               if (++stage == STAGES) { stage = 0; phase ^= 1; }
             }
             wk += kseg;
@@ -490,7 +443,7 @@ tc_conv_gemm_staged_kernel(const __grid_constant__ CUtensorMap tmA0, const __gri
     }
   } else if (warp == 1) {
     // ===================== MMA issuer (leader CTA of a pair only) =====================
-    constexpr uint32_t idesc = umma_idesc_bf16(128 * CG, BN, 0, 0);
+    constexpr uint32_t idesc = umma_idesc_bf16(256, BN, 0, 0);
     if (leader) {
     int stage = 0; uint32_t phase = 0;
     int as = 0; uint32_t aphase = 0;
@@ -517,20 +470,11 @@ tc_conv_gemm_staged_kernel(const __grid_constant__ CUtensorMap tmA0, const __gri
           const uint32_t sa = smem_u32(smem + stage * Cfg::STAGE_BYTES);
           const uint64_t adesc = umma_smem_desc(sa, 16, 1024);
           const uint64_t bdesc = umma_smem_desc(sa + Cfg::A_BYTES, 16, 1024);
-#ifndef TC_EXP_NO_MMA
 #pragma unroll
-          for (int k = 0; k < Cfg::BK / 16; ++k) {
-            if (CG == 1) umma_bf16(d_tmem, adesc + (uint64_t)(2 * k), bdesc + (uint64_t)(2 * k), idesc, (ks | k) != 0);
-            else umma_bf16_pair(d_tmem, adesc + (uint64_t)(2 * k), bdesc + (uint64_t)(2 * k), idesc, (ks | k) != 0);
-          }
-#endif
-          if (CG == 1) {
-            umma_commit(&empty_bar[stage]);
-            if (ks == ksteps - 1) umma_commit(&tfull_bar[as]);
-          } else {
-            umma_commit_pair(&empty_bar[stage]);
-            if (ks == ksteps - 1) umma_commit_pair(&tfull_bar[as]);
-          }
+          for (int k = 0; k < Cfg::BK / 16; ++k)
+            umma_bf16_pair(d_tmem, adesc + (uint64_t)(2 * k), bdesc + (uint64_t)(2 * k), idesc, (ks | k) != 0);
+          umma_commit_pair(&empty_bar[stage]);
+          if (ks == ksteps - 1) umma_commit_pair(&tfull_bar[as]);
         }
         __syncwarp();
         if (++stage == STAGES) { stage = 0; phase ^= 1; }
@@ -549,11 +493,10 @@ tc_conv_gemm_staged_kernel(const __grid_constant__ CUtensorMap tmA0, const __gri
     // ===================== output store warp =====================
     // waits for the 8 epilogue warps to fill an output slot (named barrier per slot), issues its TMA stores, and
     // frees the slot of the previous step once those stores have read shared memory
-#ifndef TC_EXP_NO_EPI
     int oslot = 0, prev = -1;
     for (int tile = tile_first; tile < p.num_tiles; tile += tile_stride) {
       const int nt = tile % p.n_tiles, mt = tile / p.n_tiles;
-      const int b = mt / p.tiles_t, t0 = (mt % p.tiles_t) * (Cfg::BM * CG) + pair_row0;
+      const int b = mt / p.tiles_t, t0 = (mt % p.tiles_t) * (Cfg::BM * 2) + pair_row0;
       const int tile_col0 = Epi::kGate ? nt * (BN / 2) : nt * BN;
 #pragma unroll 1
       for (int step = 0; step < STEPS; ++step) {
@@ -561,15 +504,11 @@ tc_conv_gemm_staged_kernel(const __grid_constant__ CUtensorMap tmA0, const __gri
         named_bar_sync(3 + oslot, NEPI * 32 + 32);
         if (lane == 0) {
           const uint8_t* ob = out_ring + oslot * NOUT * Cfg::PANEL;
-#ifndef TC_EXP_NO_OUT
           tma_store_3d_h(ob, &tmO0, sp.out_col[0] + col0, t0, b, sp.pol_out[0]);
           if (NOUT > 1) tma_store_3d_h(ob + Cfg::PANEL, &tmO1, sp.out_col[1] + col0, t0, b, sp.pol_out[1]);
           if (NOUT > 2) tma_store_3d_h(ob + 2 * Cfg::PANEL, &tmO2, sp.out_col[2] + col0, t0, b, sp.pol_out[2]);
           bulk_commit_group();
           if (prev >= 0) { bulk_wait_group_read<1>(); mbar_arrive(&out_empty[prev]); }
-#else
-          if (prev >= 0) mbar_arrive(&out_empty[prev]);
-#endif
           prev = oslot;
         }
         __syncwarp();
@@ -577,44 +516,20 @@ tc_conv_gemm_staged_kernel(const __grid_constant__ CUtensorMap tmA0, const __gri
       }
     }
     if (lane == 0) bulk_wait_group<0>();
-#endif
   } else if (warp == 3) {
     // ===================== epilogue-input producer =====================
-#ifdef TC_EXP_NO_EPI
-    if (false) {
-#else
     if (NIN > 0 && use_in && lane == 0) {
-#endif
       int islot = 0; uint32_t iphase = 0;
       for (int tile = tile_first; tile < p.num_tiles; tile += tile_stride) {
         const int nt = tile % p.n_tiles, mt = tile / p.n_tiles;
-        const int b = mt / p.tiles_t, t0 = (mt % p.tiles_t) * (Cfg::BM * CG) + pair_row0;
+        const int b = mt / p.tiles_t, t0 = (mt % p.tiles_t) * (Cfg::BM * 2) + pair_row0;
         const int tile_col0 = Epi::kGate ? nt * (BN / 2) : nt * BN;
-#ifdef TC_L2_PREFETCH
-        {
-          // pull the NEXT tile's epilogue inputs into L2 while this tile is being computed
-          const int tn = tile + tile_stride;
-          if (tn < p.num_tiles) {
-            const int nt2 = tn % p.n_tiles, mt2 = tn / p.n_tiles;
-            const int b2 = mt2 / p.tiles_t, t2 = (mt2 % p.tiles_t) * (Cfg::BM * CG) + pair_row0;
-            const int c2 = Epi::kGate ? nt2 * (BN / 2) : nt2 * BN;
-            for (int step = 0; step < STEPS; ++step) {
-              if (sp.in_mask & 1u) tma_prefetch_l2_3d(&tmI0, sp.in_col[0] + c2 + step * 32, t2, b2);
-              if (NIN > 1 && (sp.in_mask & 2u)) tma_prefetch_l2_3d(&tmI1, sp.in_col[1] + c2 + step * 32, t2, b2);
-            }
-          }
-        }
-#endif
         for (int step = 0; step < STEPS; ++step) {
           mbar_wait(&in_empty[islot], iphase ^ 1);
-#ifdef TC_EXP_NO_IN
-          mbar_arrive(&in_full[islot]);
-#else
           mbar_expect_tx(&in_full[islot], (uint32_t)(nact * Cfg::PANEL));
           uint8_t* dst = in_ring + islot * nact * Cfg::PANEL;
           if (sp.in_mask & 1u) { tma_load_3d_h(dst, &tmI0, &in_full[islot], sp.in_col[0] + tile_col0 + step * 32, t0, b, sp.pol_in[0]); dst += Cfg::PANEL; }
           if (NIN > 1 && (sp.in_mask & 2u)) tma_load_3d_h(dst, &tmI1, &in_full[islot], sp.in_col[1] + tile_col0 + step * 32, t0, b, sp.pol_in[1]);
-#endif
           if (++islot == in_slots) { islot = 0; iphase ^= 1; }
         }
       }
@@ -640,7 +555,7 @@ tc_conv_gemm_staged_kernel(const __grid_constant__ CUtensorMap tmA0, const __gri
       const long long tl_a = clock64();
 #endif
       const int nt = tile % p.n_tiles, mt = tile / p.n_tiles;
-      const int b = mt / p.tiles_t, t0 = (mt % p.tiles_t) * (Cfg::BM * CG) + pair_row0;
+      const int b = mt / p.tiles_t, t0 = (mt % p.tiles_t) * (Cfg::BM * 2) + pair_row0;
       const int tile_col0 = Epi::kGate ? nt * (BN / 2) : nt * BN;
       const int bsafe = b < p.B ? b : p.B - 1;
       constexpr int NBIAS = Epi::kBiasFloats(BN);
@@ -659,11 +574,6 @@ tc_conv_gemm_staged_kernel(const __grid_constant__ CUtensorMap tmA0, const __gri
         named_bar_sync(2, NEPI * 32);
       }
       TmemAccRow acc{tmem_base + (uint32_t)(as * BN) + ((uint32_t)(quarter * 32) << 16), true};
-#ifdef TC_EXP_NO_EPI
-      constexpr int STEPS_RUN = 0;
-#else
-      constexpr int STEPS_RUN = STEPS;
-#endif
 #ifdef TC_TIMELINE
       long long ph[6] = {0, 0, 0, 0, 0, 0};
 #define TL_MARK(i) { const long long tl_now = clock64(); ph[i] += tl_now - tl_prev; tl_prev = tl_now; }
@@ -672,7 +582,7 @@ tc_conv_gemm_staged_kernel(const __grid_constant__ CUtensorMap tmA0, const __gri
 #define TL_MARK(i)
 #endif
 #pragma unroll 1
-      for (int step = 0; step < STEPS_RUN; ++step) {
+      for (int step = 0; step < STEPS; ++step) {
         const int col0 = tile_col0 + step * 32;
         float in[NIN > 0 ? NIN : 1][16];
         float out[NOUT][16];
@@ -729,10 +639,7 @@ tc_conv_gemm_staged_kernel(const __grid_constant__ CUtensorMap tmA0, const __gri
 #endif
       tc_fence_before();
       __syncwarp();
-      if (lane == 0) {
-        if (CG == 1) mbar_arrive(&tempty_bar[as]);
-        else mbar_arrive_remote_relaxed(&tempty_bar[as], 0u);      // the leader's MMA warp waits for both CTAs' epilogues
-      }
+      if (lane == 0) mbar_arrive_remote_relaxed(&tempty_bar[as], 0u);      // the leader's MMA warp waits for both CTAs' epilogues
       if (++as == 2) { as = 0; aphase ^= 1; }
     }
 #ifdef TC_TIMELINE
@@ -742,11 +649,8 @@ tc_conv_gemm_staged_kernel(const __grid_constant__ CUtensorMap tmA0, const __gri
   }
   tc_fence_before();
   __syncthreads();
-  if (CG == 2) cluster_sync_all();       // nobody leaves (or frees TMEM) while the pair may still signal / read
-  if (warp == 2) {
-    if (CG == 2) tmem_dealloc_pair<Cfg::TMEM_COLS>(tmem_base);
-    else tmem_dealloc<Cfg::TMEM_COLS>(tmem_base);
-  }
+  cluster_sync_all();       // nobody leaves (or frees TMEM) while the pair may still signal / read
+  if (warp == 2) tmem_dealloc_pair<Cfg::TMEM_COLS>(tmem_base);
 }
 
 // half-panel map over a (B,T,ld) bf16 tensor restricted to C columns: box (32 cols, 128 rows, 1), 64B swizzle
@@ -757,10 +661,10 @@ static inline const CUtensorMap* tc_panel_map(TmapCache& tc, const TcEpiIo& io, 
   return tc.get(io.base, 3, dims, str, box, 64);
 }
 
-template <class Epi, int BN, int CG>
+template <class Epi, int BN>
 static int tc_conv_gemm_staged_launch(TmapCache& tc, cudaStream_t st, const TcGemmDesc& d, const typename Epi::Params& ep, const TcEpiIo* ins,
                                       uint32_t in_mask, const TcEpiIo* outs) {
-  using Cfg = TcStagedCfg<BN, Epi::NIN, Epi::NOUT, Epi::kInPanels, Epi::kOutSlots, CG>;
+  using Cfg = TcStagedCfg<BN, Epi::NIN, Epi::NOUT, Epi::kInPanels, Epi::kOutSlots>;
   const CUtensorMap* ma[TC_MAX_SEG] = {};
   for (int s = 0; s < d.nseg; ++s) {
     ma[s] = tc_act_map(tc, d.seg[s].A, d.seg[s].lda, d.seg[s].K, d.T, d.B, s == 0 ? d.n_outer : 1, d.outer_stride, 128);
@@ -769,7 +673,7 @@ static int tc_conv_gemm_staged_launch(TmapCache& tc, cudaStream_t st, const TcGe
   for (int s = d.nseg; s < TC_MAX_SEG; ++s) ma[s] = ma[0];
   uint64_t wd[2] = {(uint64_t)d.ktot, (uint64_t)d.N16};
   uint64_t ws[1] = {(uint64_t)d.ktot * 2};
-  uint32_t wb[2] = {64, (uint32_t)(BN / CG)};
+  uint32_t wb[2] = {64, (uint32_t)(BN / 2)};
   const CUtensorMap* mw = tc.get(d.W, 2, wd, ws, wb);
   if (!mw) return -11;
   TcStagedParams sp{};
@@ -795,34 +699,24 @@ static int tc_conv_gemm_staged_launch(TmapCache& tc, cudaStream_t st, const TcGe
   }
   for (int k = 0; k < 2; ++k) if (!mi[k]) mi[k] = mo[0];
   TcGemmParams p{};
-  p.B = d.B; p.T = d.T; p.tiles_t = (d.T + 128 * CG - 1) / (128 * CG); p.n_tiles = d.N16 / BN; p.num_tiles = d.B * p.tiles_t * p.n_tiles;
+  p.B = d.B; p.T = d.T; p.tiles_t = (d.T + 255) / 256; p.n_tiles = d.N16 / BN; p.num_tiles = d.B * p.tiles_t * p.n_tiles;
   p.nseg = d.nseg; p.n_outer = d.n_outer > 0 ? d.n_outer : 1;
   for (int s = 0; s < d.nseg; ++s) { p.segK[s] = d.seg[s].K; p.segShift[s] = d.seg[s].shift; }
-  auto kern = tc_conv_gemm_staged_kernel<Epi, BN, CG>;
+  auto kern = tc_conv_gemm_staged_kernel<Epi, BN>;
   static unsigned long long attr_devs = 0ull;
   if (tc_first_use_on_device(&attr_devs)) {
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES);
     if (e != cudaSuccess) { snprintf(g_tc_err, sizeof(g_tc_err), "cudaFuncSetAttribute(smem=%d): %s", Cfg::SMEM_BYTES, cudaGetErrorString(e)); return -12; }
   }
-  const int slots = tc_balanced_slots(p.num_tiles, tc_num_sms() / CG);      // one CTA (or CTA pair) per SM (pair of SMs of a TPC)
-  const int grid = (p.num_tiles < slots ? p.num_tiles : slots) * CG;
+  const int slots = tc_balanced_slots(p.num_tiles, tc_num_sms() / 2);      // one CTA pair per pair of SMs (a TPC)
+  const int grid = (p.num_tiles < slots ? p.num_tiles : slots) * 2;
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3(grid); cfg.blockDim = dim3(384); cfg.dynamicSmemBytes = Cfg::SMEM_BYTES; cfg.stream = st;
   cudaLaunchAttribute attr[2];
-  cfg.attrs = attr; cfg.numAttrs = tc_launch_attrs(attr, CG);
+  cfg.attrs = attr; cfg.numAttrs = tc_launch_attrs(attr, 2);
   cudaError_t e = cudaLaunchKernelEx(&cfg, kern, *ma[0], *ma[1], *ma[2], *ma[3], *ma[4], *mw, *mi[0], *mi[1], *mo[0], *mo[1], *mo[2], p, sp, ep);
-  if (e != cudaSuccess) { snprintf(g_tc_err, sizeof(g_tc_err), "staged conv_gemm launch (cta_group %d): %s", CG, cudaGetErrorString(e)); return -13; }
+  if (e != cudaSuccess) { snprintf(g_tc_err, sizeof(g_tc_err), "staged conv_gemm launch: %s", cudaGetErrorString(e)); return -13; }
   return 0;
-}
-
-// cta_group of the conv GEMMs: 2 (CTA pairs) unless overridden (WN_TC_CTA_GROUP=1 in the environment, for A/B runs)
-static inline int tc_cta_group() {
-  static int cg = 0;
-  if (cg == 0) {
-    const char* e = getenv("WN_TC_CTA_GROUP");
-    cg = (e && e[0] == '1') ? 1 : 2;
-  }
-  return cg;
 }
 
 template <class Epi>
@@ -831,18 +725,10 @@ static int tc_conv_gemm_staged(TmapCache& tc, cudaStream_t st, const TcGemmDesc&
   int tile = d.tileN;
   if (tile == 0) tile = d.N16 % 256 == 0 ? 256 : (d.N16 % 128 == 0 ? 128 : 64);
   if (d.N16 % tile != 0 || d.nseg < 1 || d.nseg > TC_MAX_SEG) { snprintf(g_tc_err, sizeof(g_tc_err), "bad tiling N16=%d tile=%d nseg=%d", d.N16, tile, d.nseg); return -1; }
-  if (tc_cta_group() == 2) {
-    switch (tile) {
-      case 256: return tc_conv_gemm_staged_launch<Epi, 256, 2>(tc, st, d, ep, ins, in_mask, outs);
-      case 128: return tc_conv_gemm_staged_launch<Epi, 128, 2>(tc, st, d, ep, ins, in_mask, outs);
-      case 64: return tc_conv_gemm_staged_launch<Epi, 64, 2>(tc, st, d, ep, ins, in_mask, outs);
-    }
-    return -2;
-  }
   switch (tile) {
-    case 256: return tc_conv_gemm_staged_launch<Epi, 256, 1>(tc, st, d, ep, ins, in_mask, outs);
-    case 128: return tc_conv_gemm_staged_launch<Epi, 128, 1>(tc, st, d, ep, ins, in_mask, outs);
-    case 64: return tc_conv_gemm_staged_launch<Epi, 64, 1>(tc, st, d, ep, ins, in_mask, outs);
+    case 256: return tc_conv_gemm_staged_launch<Epi, 256>(tc, st, d, ep, ins, in_mask, outs);
+    case 128: return tc_conv_gemm_staged_launch<Epi, 128>(tc, st, d, ep, ins, in_mask, outs);
+    case 64: return tc_conv_gemm_staged_launch<Epi, 64>(tc, st, d, ep, ins, in_mask, outs);
   }
   return -2;
 }
@@ -874,10 +760,7 @@ template <int BN> struct TcWgradCfg {
 };
 
 // grid: x = 128-row tiles of the (seg, channel) axis, y = BN-wide tiles of N, z = row-range split
-// CL = cluster size along x: the CL CTAs of a cluster work on different m-tiles (channel blocks of A) against the
-// SAME G tile, so each loads 1/CL of its rows and multicasts them to all (L2 -> SM traffic per MMA step: 16 KB of A
-// + 32/CL KB of G instead of 48 KB).  Stage release is cluster-wide: every consumer arrives on every CTA's barrier.
-template <int BN, int CL>
+template <int BN>
 __global__ void __launch_bounds__(256, 1)
 tc_wgrad_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__ CUtensorMap tmA1, const __grid_constant__ CUtensorMap tmA2,
                 const __grid_constant__ CUtensorMap tmA3, const __grid_constant__ CUtensorMap tmA4, const __grid_constant__ CUtensorMap tmG, const TcWgradParams p) {
@@ -907,23 +790,16 @@ tc_wgrad_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
   // The otherwise idle epilogue warps also reduce the columns of G (bias / conditioning gradients)
   // straight from the TMA-staged G tiles in shared memory; the gridDim.x CTAs that share a G tile
   // split its 64 time rows between them so no CTA becomes the long pole.
-#ifdef TC_EXP_WG_NO_CS
-  const bool do_cs = false;
-#else
   const bool do_cs = p.cs_partial != nullptr;
-#endif
   const int cs_r0 = (Cfg::BKT * (int)blockIdx.x) / (int)gridDim.x, cs_r1 = (Cfg::BKT * ((int)blockIdx.x + 1)) / (int)gridDim.x;
-  const uint32_t crank = CL > 1 ? cluster_ctarank() : 0u;
-  constexpr uint16_t cmask = (uint16_t)((1u << CL) - 1u);
   if (warp == 1 && lane == 0) {
-    for (int i = 0; i < STAGES; ++i) { mbar_init(&full_bar[i], 1); mbar_init(&empty_bar[i], CL * (do_cs ? 5 : 1)); }
+    for (int i = 0; i < STAGES; ++i) { mbar_init(&full_bar[i], 1); mbar_init(&empty_bar[i], do_cs ? 5 : 1); }
     mbar_init(tfull_bar, 1);
     mbar_fence_init();
   }
   if (warp == 2) tmem_alloc<Cfg::TMEM_COLS>(tmem_ptr);
   tc_fence_before();
   __syncthreads();
-  if (CL > 1) cluster_sync_all();      // peers' barriers are initialised before anyone multicasts / arrives remotely
   tc_fence_after();
   const uint32_t tmem_base = *tmem_ptr;
   pdl_launch_dependents();
@@ -940,22 +816,11 @@ tc_wgrad_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
         const int b = ch / p.chunks_t, t0 = (ch % p.chunks_t) * Cfg::BKT;
         mbar_wait(&empty_bar[stage], phase ^ 1);
         uint8_t* sa = smem + stage * Cfg::STAGE_BYTES;
-#ifdef TC_EXP_WG_NO_TMA
-        mbar_arrive(&full_bar[stage]);
-#else
         mbar_expect_tx(&full_bar[stage], Cfg::STAGE_BYTES);
         tma_load_4d_h(sa, tm, &full_bar[stage], k0, t0 + shift, b, 0, p.pol_a);
         tma_load_4d_h(sa + 8192, tm, &full_bar[stage], k0 + 64, t0 + shift, b, 0, p.pol_a);
-        if (CL == 1) {
 #pragma unroll
-          for (int j = 0; j < BN / 64; ++j) tma_load_4d_h(sa + Cfg::A_BYTES + j * 8192, &tmG, &full_bar[stage], n0 + 64 * j, t0, b, 0, p.pol_g);
-        } else {
-          constexpr int RPC = Cfg::BKT / CL;          // time rows of every G atom this CTA fetches for the whole cluster
-#pragma unroll
-          for (int j = 0; j < BN / 64; ++j)
-            tma_load_4d_mc(sa + Cfg::A_BYTES + j * 8192 + crank * (RPC * 128), &tmG, &full_bar[stage], n0 + 64 * j, t0 + (int)crank * RPC, b, 0, cmask);
-        }
-#endif
+        for (int j = 0; j < BN / 64; ++j) tma_load_4d_h(sa + Cfg::A_BYTES + j * 8192, &tmG, &full_bar[stage], n0 + 64 * j, t0, b, 0, p.pol_g);
         if (++stage == STAGES) { stage = 0; phase ^= 1; }
       }
     }
@@ -970,13 +835,10 @@ tc_wgrad_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
         // MN-major, 128B swizzle: 64-wide channel atoms 8192 B apart (LBO), 8 time rows = 1024 B (SBO)
         const uint64_t adesc = umma_smem_desc(sa, 8192, 1024);
         const uint64_t bdesc = umma_smem_desc(sa + Cfg::A_BYTES, 8192, 1024);
-#ifndef TC_EXP_WG_NO_MMA
 #pragma unroll
         for (int k = 0; k < Cfg::BKT / 16; ++k)   // 16 time rows = 2048 bytes (>>4 = 128) per step
           umma_bf16(tmem_base, adesc + (uint64_t)(128 * k), bdesc + (uint64_t)(128 * k), idesc, (it | k) != 0);
-#endif
-        if (CL == 1) umma_commit(&empty_bar[stage]);
-        else umma_commit_mc(&empty_bar[stage], cmask);
+        umma_commit(&empty_bar[stage]);
         if (it == nchunks - 1) umma_commit(tfull_bar);
       }
       __syncwarp();
@@ -1016,8 +878,7 @@ tc_wgrad_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
           }
         }
         __syncwarp();
-        if (CL == 1) { if (lane == 0) mbar_arrive(&empty_bar[stage]); }
-        else if (lane < CL) mbar_arrive_remote(&empty_bar[stage], (uint32_t)lane);
+        if (lane == 0) mbar_arrive(&empty_bar[stage]);
         if (++stage == STAGES) { stage = 0; phase ^= 1; }
       }
       if (nchunks > 0 && act && n0 + c < p.N) {
@@ -1044,11 +905,7 @@ tc_wgrad_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
 #pragma unroll
         for (int i = 0; i < 16; ++i) v[i] = 0.f;
       }
-#ifdef TC_EXP_WG_NO_ST
-      if (valid && v[0] == 123.456f) {
-#else
       if (valid) {
-#endif
         const int nv = min(16, p.N - n);
         if (nv == 16 && ((p.N & 3) == 0)) {
 #pragma unroll
@@ -1062,7 +919,6 @@ tc_wgrad_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
   }
   tc_fence_before();
   __syncthreads();
-  if (CL > 1) cluster_sync_all();      // nobody leaves while a peer may still signal its barriers
   if (warp == 2) tmem_dealloc<Cfg::TMEM_COLS>(tmem_base);
 }
 
@@ -1072,8 +928,7 @@ tc_wgrad_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
 // bandwidth: 387 MB per dilated wgrad launch).  The leader's barrier counts both CTAs' TMA bytes; the column sums
 // read the local G half after the MMAs of the stage have completed (mma_done), then release the stage.
 // Requires every segment width to be a multiple of 256 (pair tiles never straddle a segment).
-// NH: BN-wide column blocks per pair (1 or 2).  NH = 2 (N = 512 per pair, all 512 TMEM columns): the A tile of a stage is
-// used for two MMAs, 48 KB per SM per 2 x the products instead of 32 KB per 1 x -> a third less L2 -> SM traffic per FLOP.
+// NH: BN-wide column blocks per pair: 1 here, 2 in the two-accumulator units of the grouped kernel (gemm_tc_wgroup.cuh).
 template <int BN, int NH = 1> struct TcWgradPairCfg {
   static constexpr int BKT = 64;
   static constexpr int A_BYTES = 2 * 64 * BKT * 2;               // two 64-channel atoms: 16 KB
@@ -1086,12 +941,12 @@ template <int BN, int NH = 1> struct TcWgradPairCfg {
   static constexpr int SMEM_BYTES = STAGES * STAGE_BYTES + 1024 + 1024 + 2048;   // align slack, barriers, column-sum scratch
 };
 
-template <int BN, int NH>
+template <int BN>
 __global__ void __launch_bounds__(256, 1)
 tc_wgrad_pair_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__ CUtensorMap tmA1, const __grid_constant__ CUtensorMap tmA2,
                      const __grid_constant__ CUtensorMap tmA3, const __grid_constant__ CUtensorMap tmA4, const __grid_constant__ CUtensorMap tmG, const __grid_constant__ CUtensorMap tmP,
                      const TcWgradParams p) {
-  using Cfg = TcWgradPairCfg<BN, NH>;
+  using Cfg = TcWgradPairCfg<BN>;
   constexpr int STAGES = Cfg::STAGES;
   constexpr int HALF = BN / 2;
   extern __shared__ uint8_t smem_raw[];
@@ -1101,7 +956,7 @@ tc_wgrad_pair_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_cons
   uint64_t* mma_done = empty_bar + STAGES;
   uint64_t* tfull_bar = mma_done + STAGES;
   uint32_t* tmem_ptr = (uint32_t*)(tfull_bar + 1);
-  float* cs_s = (float*)(smem + STAGES * Cfg::STAGE_BYTES + 1024);      // [RH][NH * HALF] column-sum hand-over between row halves
+  float* cs_s = (float*)(smem + STAGES * Cfg::STAGE_BYTES + 1024);      // [RH][HALF] column-sum hand-over between row halves
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const uint32_t crank = cluster_ctarank();
@@ -1117,8 +972,8 @@ tc_wgrad_pair_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_cons
     mp -= nt; koff += p.segK[s]; ++s;
   }
   const int k0 = (mp << 8) + (int)crank * 128;
-  const int n0 = blockIdx.y * (BN * NH);
-  const int gcol0 = n0 + (int)crank * HALF;           // first column of this CTA's half of column block 0 (block h: + h * BN)
+  const int n0 = blockIdx.y * BN;
+  const int gcol0 = n0 + (int)crank * HALF;           // first column of this CTA's half of the column block
   const int c_begin = blockIdx.z * p.chunks_per_split;
   const int c_end = min(p.total_chunks, c_begin + p.chunks_per_split);
   const int nchunks = c_end - c_begin;
@@ -1164,9 +1019,7 @@ tc_wgrad_pair_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_cons
         if (leader) mbar_expect_tx(&full_bar[stage], 2 * Cfg::STAGE_BYTES);
         // one op per operand: boxes of 2 (A) and G_ATOMS (G) 64-channel atoms (tc_atom_map)
         tma_load_4d_pair_h(sa, tm, &full_bar[stage], 0, t0 + shift, k0 >> 6, b, p.pol_a);
-#pragma unroll
-        for (int hh = 0; hh < NH; ++hh)
-          tma_load_4d_pair_h(sa + Cfg::A_BYTES + hh * Cfg::GH_BYTES, &tmG, &full_bar[stage], 0, t0, (gcol0 + hh * BN) >> 6, b, p.pol_g);
+        tma_load_4d_pair_h(sa + Cfg::A_BYTES, &tmG, &full_bar[stage], 0, t0, gcol0 >> 6, b, p.pol_g);
         if (++stage == STAGES) { stage = 0; phase ^= 1; }
       }
 #ifdef TC_TIMELINE
@@ -1192,13 +1045,10 @@ tc_wgrad_pair_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_cons
         if (elect_one()) {
           const uint32_t sa = smem_u32(smem + stage * Cfg::STAGE_BYTES);
           const uint64_t adesc = umma_smem_desc(sa, 8192, 1024);
+          const uint64_t bdesc = umma_smem_desc(sa + Cfg::A_BYTES, 8192, 1024);
 #pragma unroll
-          for (int hh = 0; hh < NH; ++hh) {
-            const uint64_t bdesc = umma_smem_desc(sa + Cfg::A_BYTES + hh * Cfg::GH_BYTES, 8192, 1024);
-#pragma unroll
-            for (int k = 0; k < Cfg::BKT / 16; ++k)
-              umma_bf16_pair(tmem_base + (uint32_t)(hh * BN), adesc + (uint64_t)(128 * k), bdesc + (uint64_t)(128 * k), idesc, (it | k) != 0);
-          }
+          for (int k = 0; k < Cfg::BKT / 16; ++k)
+            umma_bf16_pair(tmem_base, adesc + (uint64_t)(128 * k), bdesc + (uint64_t)(128 * k), idesc, (it | k) != 0);
           // with column sums the stage is released by the summing warps, which first wait for these MMAs
           umma_commit_pair(do_cs ? &mma_done[stage] : &empty_bar[stage]);
           if (it == nchunks - 1) umma_commit_pair(tfull_bar);
@@ -1223,30 +1073,24 @@ tc_wgrad_pair_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_cons
       const uint32_t chunk = (uint32_t)(cc >> 3);
       const int len = cs_r1 - cs_r0;
       const int r_lo = cs_r0 + (len * rh) / RH, r_hi = cs_r0 + (len * (rh + 1)) / RH;
-      float s0[NH], s1[NH];
-#pragma unroll
-      for (int hh = 0; hh < NH; ++hh) s0[hh] = s1[hh] = 0.f;
+      float s0 = 0.f, s1 = 0.f;
       int stage = 0; uint32_t phase = 0;
       int cur_b = c_begin / p.chunks_t;
       const int b_first = cur_b;
       auto flush = [&](int slot) {
         // combine the row halves in a fixed order, write this CTA's columns and zero the peer's half
-#pragma unroll
-        for (int hh = 0; hh < NH; ++hh) { cs_s[(rh * NH + hh) * HALF + c] = s0[hh]; cs_s[(rh * NH + hh) * HALF + c + 1] = s1[hh]; }
+        cs_s[rh * HALF + c] = s0; cs_s[rh * HALF + c + 1] = s1;
         named_bar_sync(7, 128);
         if (rh == 0) {
           float* o = p.cs_partial + (((long long)blockIdx.z * gridDim.x + blockIdx.x) * p.slots + slot) * p.N;
+          float t0 = 0.f, t1 = 0.f;
 #pragma unroll
-          for (int hh = 0; hh < NH; ++hh) {
-            float t0 = 0.f, t1 = 0.f;
-#pragma unroll
-            for (int h2 = 0; h2 < RH; ++h2) { t0 += cs_s[(h2 * NH + hh) * HALF + c]; t1 += cs_s[(h2 * NH + hh) * HALF + c + 1]; }
-            const int mine = gcol0 + hh * BN + c, other = n0 + hh * BN + (1 - (int)crank) * HALF + c;
-            if (mine < p.N) o[mine] = t0;
-            if (mine + 1 < p.N) o[mine + 1] = t1;
-            if (other < p.N) o[other] = 0.f;
-            if (other + 1 < p.N) o[other + 1] = 0.f;
-          }
+          for (int h2 = 0; h2 < RH; ++h2) { t0 += cs_s[h2 * HALF + c]; t1 += cs_s[h2 * HALF + c + 1]; }
+          const int mine = gcol0 + c, other = n0 + (1 - (int)crank) * HALF + c;
+          if (mine < p.N) o[mine] = t0;
+          if (mine + 1 < p.N) o[mine + 1] = t1;
+          if (other < p.N) o[other] = 0.f;
+          if (other + 1 < p.N) o[other + 1] = 0.f;
         }
         named_bar_sync(7, 128);
       };
@@ -1254,20 +1098,16 @@ tc_wgrad_pair_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_cons
         const int b = ch / p.chunks_t;
         if (b != cur_b) {
           flush(cur_b - b_first);
-#pragma unroll
-          for (int hh = 0; hh < NH; ++hh) s0[hh] = s1[hh] = 0.f;
+          s0 = s1 = 0.f;
           cur_b = b;
         }
         mbar_wait(&mma_done[stage], phase);
-#pragma unroll
-        for (int hh = 0; hh < NH; ++hh) {
-          const uint8_t* g = smem + stage * Cfg::STAGE_BYTES + Cfg::A_BYTES + hh * Cfg::GH_BYTES + col_off;
+        const uint8_t* g = smem + stage * Cfg::STAGE_BYTES + Cfg::A_BYTES + col_off;
 #pragma unroll 8
-          for (int r = r_lo; r < r_hi; ++r) {
-            const uint32_t w = *reinterpret_cast<const uint32_t*>(g + r * 128 + ((chunk ^ (uint32_t)(r & 7)) << 4));
-            s0[hh] += __uint_as_float(w << 16);
-            s1[hh] += __uint_as_float(w & 0xffff0000u);
-          }
+        for (int r = r_lo; r < r_hi; ++r) {
+          const uint32_t w = *reinterpret_cast<const uint32_t*>(g + r * 128 + ((chunk ^ (uint32_t)(r & 7)) << 4));
+          s0 += __uint_as_float(w << 16);
+          s1 += __uint_as_float(w & 0xffff0000u);
         }
         __syncwarp();
         if (lane == 0) mbar_arrive(&empty_bar[stage]);
@@ -1296,35 +1136,27 @@ tc_wgrad_pair_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_cons
       const int r = quarter * 32 + lane;
       const uint32_t rsw = (uint32_t)(r & 7);
       uint8_t* const rowp = smem + (uint32_t)r * 128u;
-#pragma unroll 1
-      for (int hh = 0; hh < NH; ++hh) {
-        if (hh > 0) {
-          // the staging area is reused: its TMA stores must have read it
-          if (threadIdx.x == 128) bulk_wait_group_read<0>();
-          named_bar_sync(6, 128);
-        }
-        for (int c = 0; c < BN; c += 16) {
-          float v[16];
-          if (nchunks > 0) tmem_ld16(taddr + (uint32_t)(hh * BN + c), v);
-          else {
+      for (int c = 0; c < BN; c += 16) {
+        float v[16];
+        if (nchunks > 0) tmem_ld16(taddr + (uint32_t)c, v);
+        else {
 #pragma unroll
-            for (int i = 0; i < 16; ++i) v[i] = 0.f;
-          }
-          uint8_t* const boxp = rowp + (c >> 5) * 16384;
-          const uint32_t j0 = (uint32_t)((c & 31) >> 2);
-#pragma unroll
-          for (int i = 0; i < 4; ++i)
-            *reinterpret_cast<float4*>(boxp + (((j0 + i) ^ rsw) << 4)) = make_float4(v[4 * i], v[4 * i + 1], v[4 * i + 2], v[4 * i + 3]);
+          for (int i = 0; i < 16; ++i) v[i] = 0.f;
         }
-        fence_proxy_async();
-        named_bar_sync(6, 128);
-        if (threadIdx.x == 128) {
-          const int row0 = koff + k0;
+        uint8_t* const boxp = rowp + (c >> 5) * 16384;
+        const uint32_t j0 = (uint32_t)((c & 31) >> 2);
 #pragma unroll
-          for (int bx = 0; bx < BN / 32; ++bx)
-            if (n0 + hh * BN + bx * 32 < p.N) tma_store_3d_h(smem + bx * 16384, &tmP, n0 + hh * BN + bx * 32, row0, (int)blockIdx.z, TC_POL_LAST);
-          bulk_commit_group();
-        }
+        for (int i = 0; i < 4; ++i)
+          *reinterpret_cast<float4*>(boxp + (((j0 + i) ^ rsw) << 4)) = make_float4(v[4 * i], v[4 * i + 1], v[4 * i + 2], v[4 * i + 3]);
+      }
+      fence_proxy_async();
+      named_bar_sync(6, 128);
+      if (threadIdx.x == 128) {
+        const int row0 = koff + k0;
+#pragma unroll
+        for (int bx = 0; bx < BN / 32; ++bx)
+          if (n0 + bx * 32 < p.N) tma_store_3d_h(smem + bx * 16384, &tmP, n0 + bx * 32, row0, (int)blockIdx.z, TC_POL_LAST);
+        bulk_commit_group();
       }
       if (threadIdx.x == 128) bulk_wait_group<0>();
     }
@@ -1338,9 +1170,9 @@ tc_wgrad_pair_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_cons
   if (warp == 2) tmem_dealloc_pair<Cfg::TMEM_COLS>(tmem_base);
 }
 
-template <int BN, int NH>
+template <int BN>
 static int tc_wgrad_pair_launch(TmapCache& tc, cudaStream_t st, const TcWgradDesc& d, TcWgradPlan* plan) {
-  using Cfg = TcWgradPairCfg<BN, NH>;
+  using Cfg = TcWgradPairCfg<BN>;
   const CUtensorMap* ma[TC_MAX_SEG] = {};
   int mpairs = 0;
   for (int s = 0; s < d.nseg; ++s) {
@@ -1356,7 +1188,7 @@ static int tc_wgrad_pair_launch(TmapCache& tc, cudaStream_t st, const TcWgradDes
   for (int s = 0; s < d.nseg; ++s) { p.segK[s] = d.seg[s].K; p.segShift[s] = d.seg[s].shift; }
   p.partial = d.partial;
   p.pol_a = tc_policy(d.l2_a); p.pol_g = tc_policy(d.l2_g);
-  const int ntiles = (d.N + BN * NH - 1) / (BN * NH);
+  const int ntiles = (d.N + BN - 1) / BN;
   int nsplit = (tc_num_sms() / 2) / (mpairs * ntiles);     // one wave of CTA pairs
   if (nsplit < 1) nsplit = 1;
   if (nsplit > WN_MAX_WGRAD_SPLITS) nsplit = WN_MAX_WGRAD_SPLITS;
@@ -1372,7 +1204,7 @@ static int tc_wgrad_pair_launch(TmapCache& tc, cudaStream_t st, const TcWgradDes
   uint32_t pb[3] = {32, 128, 1};
   const CUtensorMap* mp = tc.get(d.partial, 3, pd, ps, pb, 128, true);
   if (!mp) return -14;
-  auto kern = tc_wgrad_pair_kernel<BN, NH>;
+  auto kern = tc_wgrad_pair_kernel<BN>;
   static unsigned long long attr_devs = 0ull;
   if (tc_first_use_on_device(&attr_devs)) {
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES);
@@ -1387,48 +1219,6 @@ static int tc_wgrad_pair_launch(TmapCache& tc, cudaStream_t st, const TcWgradDes
   return 0;
 }
 
-// CTAs of one wave for cluster size CL (clusters must fit inside a GPC, so fewer than #SMs may be usable)
-template <int BN, int CL>
-static int tc_wgrad_wave_ctas() {
-  using Cfg = TcWgradCfg<BN>;
-  static int cached = 0;
-  if (cached) return cached;
-  auto kern = tc_wgrad_kernel<BN, CL>;
-  cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES);
-  int n = 0;
-  if (CL > 1) {
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3(CL * tc_num_sms()); cfg.blockDim = dim3(256); cfg.dynamicSmemBytes = Cfg::SMEM_BYTES;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = CL; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr; cfg.numAttrs = 1;
-    if (cudaOccupancyMaxActiveClusters(&n, kern, &cfg) != cudaSuccess) { n = 0; cudaGetLastError(); }
-    n *= CL;
-  }
-  if (n <= 0 || n > tc_num_sms()) n = CL > 1 ? (tc_num_sms() / CL) * CL * 7 / 8 : tc_num_sms();
-  cached = n;
-  return n;
-}
-
-template <int BN, int CL>
-static int tc_wgrad_launch_cl(const CUtensorMap* const* ma, const CUtensorMap* mg, const TcWgradParams& p, dim3 grid, cudaStream_t st) {
-  using Cfg = TcWgradCfg<BN>;
-  auto kern = tc_wgrad_kernel<BN, CL>;
-  static unsigned long long attr_devs = 0ull;
-  if (tc_first_use_on_device(&attr_devs)) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES);
-    if (e != cudaSuccess) { snprintf(g_tc_err, sizeof(g_tc_err), "cudaFuncSetAttribute(smem=%d): %s", Cfg::SMEM_BYTES, cudaGetErrorString(e)); return -12; }
-  }
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = grid; cfg.blockDim = dim3(256); cfg.dynamicSmemBytes = Cfg::SMEM_BYTES; cfg.stream = st;
-  cudaLaunchAttribute attr[2];
-  cfg.attrs = attr; cfg.numAttrs = tc_launch_attrs(attr, CL);
-  cudaError_t e = cudaLaunchKernelEx(&cfg, kern, *ma[0], *ma[1], *ma[2], *ma[3], *ma[4], *mg, p);
-  if (e != cudaSuccess) { snprintf(g_tc_err, sizeof(g_tc_err), "wgrad launch (cluster %d): %s", CL, cudaGetErrorString(e)); return -13; }
-  return 0;
-}
-
 template <int BN>
 static int tc_wgrad_launch(TmapCache& tc, cudaStream_t st, const TcWgradDesc& d, TcWgradPlan* plan) {
   using Cfg = TcWgradCfg<BN>;
@@ -1440,16 +1230,10 @@ static int tc_wgrad_launch(TmapCache& tc, cudaStream_t st, const TcWgradDesc& d,
     mtiles += (d.seg[s].K + 127) / 128;
   }
   for (int s = d.nseg; s < TC_MAX_SEG; ++s) ma[s] = ma[0];
-  // cluster along the m-tiles that share a G tile (multicast): 4, 2 or 1
-  // Measured on B200 (C2 dilated wgrad, profiles/README.md): multicast clusters of 4 are SLOWER (43 vs 37 us
-  // in isolation, +1.9 ms per step in situ: lock-step coupling, 2 KB boxes, remote barrier arrivals, and only
-  // 132 SMs host 4-clusters) — L2 already coalesces same-line requests of neighbouring SMs.  Off by default.
-#ifdef TC_WGRAD_CLUSTER
-  const int cl = mtiles % 4 == 0 ? 4 : (mtiles % 2 == 0 ? 2 : 1);
-#else
-  const int cl = 1;
-#endif
-  const CUtensorMap* mg = tc_act_map(tc, d.G, d.ldg, d.N, d.T, d.B, 1, 0, 64 / cl);
+  // No clusters along the m-tiles that share a G tile.  Measured on B200 (C2 dilated wgrad, profiles/README.md): multicasting
+  // the G tile to clusters of 4 is SLOWER (43 vs 37 us in isolation, +1.9 ms per step in situ: lock-step coupling, 2 KB boxes,
+  // remote barrier arrivals, and only 132 SMs host 4-clusters) — L2 already coalesces same-line requests of neighbouring SMs.
+  const CUtensorMap* mg = tc_act_map(tc, d.G, d.ldg, d.N, d.T, d.B, 1, 0, 64);
   if (!mg) return -11;
   TcWgradParams p{};
   p.B = d.B; p.T = d.T; p.N = d.N; p.chunks_t = (d.T + 63) / 64; p.total_chunks = d.B * p.chunks_t; p.ktot = d.ktot; p.nseg = d.nseg;
@@ -1457,8 +1241,7 @@ static int tc_wgrad_launch(TmapCache& tc, cudaStream_t st, const TcWgradDesc& d,
   p.partial = d.partial;
   p.pol_a = tc_policy(d.l2_a); p.pol_g = tc_policy(d.l2_g);
   const int ntiles = (d.N + BN - 1) / BN;
-  const int wave = cl == 4 ? tc_wgrad_wave_ctas<BN, 4>() : (cl == 2 ? tc_wgrad_wave_ctas<BN, 2>() : tc_num_sms());
-  int nsplit = wave / (mtiles * ntiles);   // one wave: never more CTAs than can be resident
+  int nsplit = tc_num_sms() / (mtiles * ntiles);   // one wave: never more CTAs than can be resident
   if (nsplit < 1) nsplit = 1;
   if (nsplit > WN_MAX_WGRAD_SPLITS) nsplit = WN_MAX_WGRAD_SPLITS;
   if (nsplit > p.total_chunks) nsplit = p.total_chunks;
@@ -1467,29 +1250,31 @@ static int tc_wgrad_launch(TmapCache& tc, cudaStream_t st, const TcWgradDesc& d,
   p.slots = (p.chunks_per_split + p.chunks_t - 2) / p.chunks_t + 1;
   p.cs_partial = d.cs_partial;
   plan->nsplit = nsplit; plan->chunks_per_split = p.chunks_per_split; plan->chunks_t = p.chunks_t; plan->slots = p.slots; plan->mtiles = mtiles;
-  const dim3 grid(mtiles, ntiles, nsplit);
-  if (cl == 4) return tc_wgrad_launch_cl<BN, 4>(ma, mg, p, grid, st);
-  if (cl == 2) return tc_wgrad_launch_cl<BN, 2>(ma, mg, p, grid, st);
-  return tc_wgrad_launch_cl<BN, 1>(ma, mg, p, grid, st);
+  auto kern = tc_wgrad_kernel<BN>;
+  static unsigned long long attr_devs = 0ull;
+  if (tc_first_use_on_device(&attr_devs)) {
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES);
+    if (e != cudaSuccess) { snprintf(g_tc_err, sizeof(g_tc_err), "cudaFuncSetAttribute(smem=%d): %s", Cfg::SMEM_BYTES, cudaGetErrorString(e)); return -12; }
+  }
+  cudaLaunchConfig_t cfg{};
+  cfg.gridDim = dim3(mtiles, ntiles, nsplit); cfg.blockDim = dim3(256); cfg.dynamicSmemBytes = Cfg::SMEM_BYTES; cfg.stream = st;
+  cudaLaunchAttribute attr[2];
+  cfg.attrs = attr; cfg.numAttrs = tc_launch_attrs(attr, 1);
+  cudaError_t e = cudaLaunchKernelEx(&cfg, kern, *ma[0], *ma[1], *ma[2], *ma[3], *ma[4], *mg, p);
+  if (e != cudaSuccess) { snprintf(g_tc_err, sizeof(g_tc_err), "wgrad launch: %s", cudaGetErrorString(e)); return -13; }
+  return 0;
 }
 
 static inline int tc_wgrad(TmapCache& tc, cudaStream_t st, const TcWgradDesc& d, TcWgradPlan* plan) {
   if (d.nseg < 1 || d.nseg > TC_MAX_SEG) return -1;
-  // CTA pairs when the pair's 256-channel tiles fit the segments exactly (WN_TC_WGRAD_PAIR=0: A/B switch)
-  static int pair_on = -1;
-  if (pair_on < 0) { const char* e = getenv("WN_TC_WGRAD_PAIR"); pair_on = (e && e[0] == '0') ? 0 : 1; }
-  bool pair_ok = pair_on && d.N > 64 && d.N % 64 == 0;
+  // CTA pairs when the pair's 256-channel tiles fit the segments exactly
+  bool pair_ok = d.N > 64 && d.N % 64 == 0;
   for (int s = 0; s < d.nseg; ++s) pair_ok = pair_ok && d.seg[s].K % 256 == 0;
   if (pair_ok) {
-    // two 256-column blocks per pair (N = 512, all of TMEM): a third less L2 -> SM traffic per FLOP, but twice the splits
-    // (37 instead of 18) and therefore twice the partial bytes to write and to reduce: measured SLOWER on C2 (7.41 vs
-    // 7.31 ms/step), off unless WN_TC_WGRAD_NH2=1
-    static int nh2_on = -1;
-    if (nh2_on < 0) { const char* e = getenv("WN_TC_WGRAD_NH2"); nh2_on = (e && e[0] == '1') ? 1 : 0; }
-    int mp = 0;
-    for (int s = 0; s < d.nseg; ++s) mp += d.seg[s].K / 256;
-    if (nh2_on && d.N % 512 == 0 && mp >= 2) return tc_wgrad_pair_launch<256, 2>(tc, st, d, plan);
-    return d.N > 128 ? tc_wgrad_pair_launch<256, 1>(tc, st, d, plan) : tc_wgrad_pair_launch<128, 1>(tc, st, d, plan);
+    // one column block per pair.  Two 256-column blocks (N = 512, all of TMEM) move a third less L2 -> SM traffic per FLOP,
+    // but need twice the splits (37 instead of 18) and therefore twice the partial bytes to write and to reduce: measured
+    // SLOWER on C2 (7.41 vs 7.31 ms/step)
+    return d.N > 128 ? tc_wgrad_pair_launch<256>(tc, st, d, plan) : tc_wgrad_pair_launch<128>(tc, st, d, plan);
   }
   if (d.N > 128) return tc_wgrad_launch<256>(tc, st, d, plan);
   if (d.N > 64) return tc_wgrad_launch<128>(tc, st, d, plan);
@@ -1570,13 +1355,4 @@ __global__ void __launch_bounds__(256) tc_wgrad_finish(const TcWgradFinish f) {
   pdl_launch_dependents();
   pdl_wait();
   tc_wgrad_finish_body(f, (int)blockIdx.x, red);
-}
-// the finishes of two weight-gradient launches (the [conv1|skip] and the dilated-conv wgrad of one block) in one launch:
-// blocks [0, n0) work on f0, the rest on f1
-__global__ void __launch_bounds__(256) tc_wgrad_finish2(const TcWgradFinish f0, const TcWgradFinish f1, const int n0) {
-  __shared__ float red[8][33];
-  pdl_launch_dependents();
-  pdl_wait();
-  if ((int)blockIdx.x < n0) tc_wgrad_finish_body(f0, (int)blockIdx.x, red);
-  else tc_wgrad_finish_body(f1, (int)blockIdx.x - n0, red);
 }

@@ -6,12 +6,12 @@
 //
 //   dg   = [d x_out_l | d skip] . [Wr^T ; Ws^T]                      DG tile   (M = 256, N = D, K = R + S)
 //   d z  = gate'(z_l) * dg                                           DG epilogue: z_f / z_s panels arrive by TMA, d z goes
-//                                                                    into a K-major 128B-swizzled operand buffer in shared
+//                                                                    K-major, 128B-swizzled into the operand ring in shared
 //                                                                    memory (and from there, by TMA, to HBM once: the
 //                                                                    grouped weight gradients read it later)
 //   d x_out_{l-1} = d x_out_l                                        OUT tile: the residual gradient is added in the OUT epilogue
 //                                                                    (d x_out panels arrive by TMA in the ring the P, Q panels use)
-//                 + d z[t]       . W_{K-1}^T                         ... the un-shifted tap straight from the operand buffer
+//                 + d z[t]       . W_{K-1}^T                         ... the un-shifted tap straight from the operand ring
 //                 + d z[t + s_k] . W_k^T,  k < K-1                   ... the anti-causal taps by TMA from HBM / L2 (rows of
 //                                                                    LATER tiles of the same block, and the peer's half)
 //
@@ -62,47 +62,44 @@ struct TcStackBwdParams {
   int kb_dx, kb_ds;           // 64-wide k blocks of the DG contraction over d x_out (R) and d skip (S)
   unsigned long long pol_dx, pol_ds, pol_w, pol_z, pol_dz_ld, pol_dz_st, pol_o;
   float drop_scale;           // 1 / (1 - rate)
-  int relaxed_handoff;        // the peer CTA's slab hand-off arrives without the cluster-scope release (see warp 12)
   int band, nbands;           // tile order: bands of `band` m tiles (the last one may be shorter); within a band all layers, last to first
 };
 
-// V2 (round 2, the default; WN_TC_STACK_BWD=1 selects the first version): no separate d z operand buffer.  An un-shifted-tap k-step only loads weights, the A half of its ring
-// stage is idle — the DG epilogue writes the d z slab straight into it (and the TMA store to HBM reads it from there).  The 64 KB of
-// the operand buffer become two more ring stages (5 instead of 3): up to five slabs in flight between epilogue and MMA instead of two
-// slab pairs, and a deeper ring for the DG / shifted-tap k-steps.  Measured (in-kernel phase accounting, C2): DG k-steps 9.3 k -> 7.0 k
-// cycles per tile, but the pair hand-off chain (epilogue -> hand-off warp -> cluster-scope arrive -> MMA) still paces the
-// un-shifted tap at ~10 k cycles per tile: step -0.3 .. -0.9 % same-box.  WN_TC_HANDOFF_RELAXED=1 drops the cluster-scope release
-// from the peer's hand-off arrive (hand-off waits -25 %, step within noise; off by default: it leans on shared-memory writes being
-// physically complete before the local barrier that the hand-off warp acquires, not on the PTX memory model).
-template <int D_, int R_, bool V2 = false> struct TcStackBwdCfg {
+// No separate d z operand buffer: an un-shifted-tap k-step only loads weights, so the A half of its ring stage is idle — the DG
+// epilogue writes the d z slab straight into it (and the TMA store to HBM reads it from there).  Against a 64 KB operand buffer
+// beside a 3-stage ring, the same shared memory as 5 ring stages holds up to five slabs in flight between epilogue and MMA instead
+// of two slab pairs, and deepens the ring for the DG / shifted-tap k-steps.  Measured (in-kernel phase accounting, C2): DG k-steps
+// 9.3 k -> 7.0 k cycles per tile, step -0.3 .. -0.9 % same-box; the pair hand-off chain (epilogue -> hand-off warp ->
+// cluster-scope arrive -> MMA) still paces the un-shifted tap at ~10 k cycles per tile.  The peer's hand-off arrive keeps its
+// cluster-scope release: without it the hand-off waits drop by 25 % but the step stays within noise, and the hand-off would lean
+// on shared-memory writes being physically complete before the local barrier that the hand-off warp acquires, not on the PTX
+// memory model.
+template <int D_, int R_> struct TcStackBwdCfg {
   static constexpr int BM = 128, BK = 64;
   static constexpr int A_BYTES = BM * BK * 2;                  // 16 KB
   static constexpr int B_BYTES = 128 * BK * 2;                 // this CTA's half of a 256-row weight tile: 16 KB
   static constexpr int STAGE_BYTES = A_BYTES + B_BYTES;
-  static constexpr int STAGES = V2 ? 5 : 3;
+  static constexpr int STAGES = 5;
   static constexpr int NSLAB = 2 * D_ / 64;                    // 64-column slabs of d z (filter slabs first, then gate slabs)
   static constexpr int NPAIR = D_ / 64;                        // slab pairs (f_p, s_p) = two 32-channel epilogue steps each
-  static constexpr int DZ_SLOTS = V2 ? 0 : 4;                  // operand buffer: two slab pairs
-  static constexpr int DZ_BYTES = DZ_SLOTS * A_BYTES;          // 64 KB
   static constexpr int PANEL = 128 * 64;                       // 128 rows x 32 bf16
   static constexpr int IN_SLOTS = 3, OUT_SLOTS = 2;            // z ring: (z_f, z_s) panels per slot; out ring: one d x panel per slot
   static constexpr int TMEM_COLS = 512;
-  static constexpr int SMEM_BYTES = STAGES * STAGE_BYTES + DZ_BYTES + IN_SLOTS * 2 * PANEL + OUT_SLOTS * PANEL + 512;
+  static constexpr int SMEM_BYTES = STAGES * STAGE_BYTES + IN_SLOTS * 2 * PANEL + OUT_SLOTS * PANEL + 512;
   static_assert(D_ % 128 == 0 && D_ <= 256 && R_ % 64 == 0 && R_ <= 256, "stack backward kernel: D in {128,256}, R <= 256");
   static_assert(SMEM_BYTES <= 232448, "stack backward kernel does not fit shared memory");
 };
 
-template <int D_, int R_, bool V2>
+template <int D_, int R_>
 __global__ void __launch_bounds__(416, 1)
 tc_stack_bwd_kernel(const TcStackBwdLayer* __restrict__ layers, int* __restrict__ flags_dx, int* __restrict__ flags_dz, const TcStackBwdParams p) {
-  using Cfg = TcStackBwdCfg<D_, R_, V2>;
+  using Cfg = TcStackBwdCfg<D_, R_>;
   constexpr int STAGES = Cfg::STAGES, NEPI = 8, NPAIR = Cfg::NPAIR;
   constexpr int KB_Z = Cfg::NSLAB;
   extern __shared__ __align__(1024) uint8_t smem_sb[];
   uint8_t* smem = smem_sb;
   if ((smem_u32(smem) & 1023u) != 0u) { if (threadIdx.x == 0) printf("libwavenet_b200: dynamic shared memory is not 1024-byte aligned\n"); __trap(); }
-  uint8_t* dzbuf = smem + STAGES * Cfg::STAGE_BYTES;                    // [4 slots][128 rows][128 B], 128B swizzle
-  uint8_t* in_ring = dzbuf + Cfg::DZ_BYTES;
+  uint8_t* in_ring = smem + STAGES * Cfg::STAGE_BYTES;
   uint8_t* out_ring = in_ring + Cfg::IN_SLOTS * 2 * Cfg::PANEL;
   uint64_t* full_bar = (uint64_t*)(out_ring + Cfg::OUT_SLOTS * Cfg::PANEL);
   uint64_t* empty_bar = full_bar + STAGES;
@@ -113,13 +110,9 @@ tc_stack_bwd_kernel(const TcStackBwdLayer* __restrict__ layers, int* __restrict_
   uint64_t* in_full = out_empty + 1;                 // [IN_SLOTS]
   uint64_t* in_empty = in_full + Cfg::IN_SLOTS;
   uint64_t* oslot_empty = in_empty + Cfg::IN_SLOTS;  // [OUT_SLOTS] output panel has been read by its TMA store
-  uint64_t* slab_done = oslot_empty + Cfg::OUT_SLOTS;   // [2] local: this CTA's epilogue has written (and fenced) slab pair slot ps
-  uint64_t* slab_full = slab_done + 2;               // [2] leader's: both CTAs' slabs of pair slot ps are complete
-  uint64_t* slab_cons = slab_full + 2;               // [2] local: the MMAs reading pair slot ps have completed
-  uint64_t* slab_free = slab_cons + 2;               // [2] local: the TMA stores of pair slot ps have read the buffer
-  // V2: per ring stage — a_done (local, 8 epilogue warps: this CTA's d z slab is in the stage's A half), a_ready (leader's, both CTAs),
+  // per ring stage — a_done (local, 8 epilogue warps: this CTA's d z slab is in the stage's A half), a_ready (leader's, both CTAs),
   // sfree (local: the TMA store of the slab has read the stage)
-  uint64_t* a_done = slab_free + 2;
+  uint64_t* a_done = oslot_empty + Cfg::OUT_SLOTS;
   uint64_t* a_ready = a_done + STAGES;
   uint64_t* sfree = a_ready + STAGES;
   uint32_t* tmem_ptr = (uint32_t*)(sfree + STAGES);
@@ -166,7 +159,6 @@ tc_stack_bwd_kernel(const TcStackBwdLayer* __restrict__ layers, int* __restrict_
     mbar_init(dg_full, 1); mbar_init(dg_empty, NEPI * 2); mbar_init(out_full, 1); mbar_init(out_empty, NEPI * 2);
     for (int i = 0; i < Cfg::IN_SLOTS; ++i) { mbar_init(&in_full[i], 1); mbar_init(&in_empty[i], NEPI); }
     for (int i = 0; i < Cfg::OUT_SLOTS; ++i) mbar_init(&oslot_empty[i], 1);
-    for (int i = 0; i < 2; ++i) { mbar_init(&slab_done[i], NEPI); mbar_init(&slab_full[i], 2); mbar_init(&slab_cons[i], 1); mbar_init(&slab_free[i], 1); }
     for (int i = 0; i < STAGES; ++i) { mbar_init(&a_done[i], NEPI); mbar_init(&a_ready[i], 2); mbar_init(&sfree[i], 1); }
     mbar_fence_init();
   }
@@ -192,12 +184,12 @@ tc_stack_bwd_kernel(const TcStackBwdLayer* __restrict__ layers, int* __restrict_
     if (lane == 0) {
       int stage = 0; uint32_t phase = 0;
       auto next = [&]() { if (++stage == STAGES) { stage = 0; phase ^= 1; } };
-      // V2: a stage whose last use carried a d z slab is free again once the slab's TMA store has read it (bit per stage:
+      // a stage whose last use carried a d z slab is free again once the slab's TMA store has read it (bit per stage:
       // un_pend = that wait is outstanding, un_wpar = parity to wait for, un_npar = parity of the stage's next slab use)
       uint32_t un_pend = 0u, un_wpar = 0u, un_npar = 0u;
       auto stage_wait = [&]() {
         mbar_wait(&empty_bar[stage], phase ^ 1);
-        if (V2 && ((un_pend >> stage) & 1u)) { mbar_wait(&sfree[stage], (un_wpar >> stage) & 1u); un_pend &= ~(1u << stage); }
+        if ((un_pend >> stage) & 1u) { mbar_wait(&sfree[stage], (un_wpar >> stage) & 1u); un_pend &= ~(1u << stage); }
       };
       SBT_DECL(4)
       constexpr int WDG_BYTES = (D_ / 2) * 64 * 2, WB_BYTES = (R_ / 2) * 64 * 2;
@@ -258,7 +250,7 @@ tc_stack_bwd_kernel(const TcStackBwdLayer* __restrict__ layers, int* __restrict_
             next();
           }
         }
-        // ---- OUT, un-shifted tap: only the weights (the A operand is the d z buffer), slab pairs in production order
+        // ---- OUT, un-shifted tap: only the weights (the A half receives a d z slab from the epilogue), slab pairs in production order
         const int kloc = (p.nseg - 1) * 2 * D_;
         for (int pr = 0; pr < NPAIR; ++pr) {
           for (int hh = 0; hh < 2; ++hh) {
@@ -267,10 +259,8 @@ tc_stack_bwd_kernel(const TcStackBwdLayer* __restrict__ layers, int* __restrict_
             uint8_t* sa = smem + stage * Cfg::STAGE_BYTES;
             if (leader) mbar_expect_tx(&full_bar[stage], 2 * WB_BYTES);
             tma_load_2d_pair_h(sa + Cfg::A_BYTES, &Ly.tmWb, &full_bar[stage], kloc + slab * 64, (int)crank * (R_ / 2), p.pol_w);
-            if (V2) {      // this stage's A half receives a d z slab from the epilogue
-              un_wpar = (un_wpar & ~(1u << stage)) | (((un_npar >> stage) & 1u) << stage);
-              un_npar ^= 1u << stage; un_pend |= 1u << stage;
-            }
+            un_wpar = (un_wpar & ~(1u << stage)) | (((un_npar >> stage) & 1u) << stage);
+            un_npar ^= 1u << stage; un_pend |= 1u << stage;
             next();
           }
         }
@@ -307,11 +297,10 @@ tc_stack_bwd_kernel(const TcStackBwdLayer* __restrict__ layers, int* __restrict_
       constexpr uint32_t idesc_o = umma_idesc_bf16(256, R_, 0, 0);
       const uint32_t t_dg = tmem_base, t_out = tmem_base + 256u;
       int stage = 0; uint32_t phase = 0;
-      uint32_t n_sf[2] = {0u, 0u};       // completed waits on slab_full[ps]
       uint32_t ng = 0u;                  // gated tiles so far
-      uint32_t ar_par = 0u;              // V2: per stage, parity of its next a_ready phase
+      uint32_t ar_par = 0u;              // per stage, parity of its next a_ready phase
       SBT_DECL(10)
-      auto kstep = [&](uint32_t d_tmem, uint32_t idesc, bool a_from_dz, int slot, bool first, uint64_t* extra0, uint64_t* extra1) {
+      auto kstep = [&](uint32_t d_tmem, uint32_t idesc, bool first, uint64_t* extra) {
 #ifdef TC_TIMELINE
         const long long w0 = clock64();
 #endif
@@ -322,15 +311,13 @@ tc_stack_bwd_kernel(const TcStackBwdLayer* __restrict__ layers, int* __restrict_
         tc_fence_after();
         if (elect_one()) {
           const uint32_t sa = smem_u32(smem + stage * Cfg::STAGE_BYTES);
-          const uint32_t a_addr = a_from_dz ? smem_u32(dzbuf) + (uint32_t)slot * (uint32_t)Cfg::A_BYTES : sa;
-          const uint64_t adesc = umma_smem_desc(a_addr, 16, 1024);
+          const uint64_t adesc = umma_smem_desc(sa, 16, 1024);
           const uint64_t bdesc = umma_smem_desc(sa + Cfg::A_BYTES, 16, 1024);
 #pragma unroll
           for (int k = 0; k < Cfg::BK / 16; ++k)
             umma_bf16_pair(d_tmem, adesc + (uint64_t)(2 * k), bdesc + (uint64_t)(2 * k), idesc, (first && k == 0) ? 0u : 1u);
           umma_commit_pair(&empty_bar[stage]);
-          if (extra0) umma_commit_pair(extra0);
-          if (extra1) umma_commit_pair(extra1);
+          if (extra) umma_commit_pair(extra);
         }
         __syncwarp();
         if (++stage == STAGES) { stage = 0; phase ^= 1; }
@@ -347,7 +334,7 @@ tc_stack_bwd_kernel(const TcStackBwdLayer* __restrict__ layers, int* __restrict_
           SBT(3)
           tc_fence_after();
           const int ks_p = p.nseg * Ly.kb_tap;
-          for (int ks = 0; ks < ks_p; ++ks) kstep(t_out, idesc_o, false, 0, ks == 0, ks == ks_p - 1 ? out_full : nullptr, nullptr);
+          for (int ks = 0; ks < ks_p; ++ks) kstep(t_out, idesc_o, ks == 0, ks == ks_p - 1 ? out_full : nullptr);
           SBT(7)
           continue;
         }
@@ -358,41 +345,28 @@ tc_stack_bwd_kernel(const TcStackBwdLayer* __restrict__ layers, int* __restrict_
         SBT(1)
         tc_fence_after();
         const int ks_dg = (Ly.has_dx ? p.kb_dx : 0) + (Ly.has_ds ? p.kb_ds : 0);
-        for (int ks = 0; ks < ks_dg; ++ks) kstep(t_dg, idesc_g, false, 0, ks == 0, ks == ks_dg - 1 ? dg_full : nullptr, nullptr);
+        for (int ks = 0; ks < ks_dg; ++ks) kstep(t_dg, idesc_g, ks == 0, ks == ks_dg - 1 ? dg_full : nullptr);
         // ---- OUT
         SBT(2)
         mbar_wait(out_empty, par ^ 1);
         SBT(3)
         tc_fence_after();
         const int ks_sh = (p.nseg - 1) * KB_Z;
-        bool first = true;
-        if constexpr (V2) {
-          for (int q = 0; q < KB_Z; ++q) {
-            // one hand-off per slab PAIR, on the barrier of the filter slab's stage: both CTAs' two slabs are in their stages' A halves
-            if ((q & 1) == 0) { mbar_wait(&a_ready[stage], (ar_par >> stage) & 1u); ar_par ^= 1u << stage; }
-            SBT(5)
-            tc_fence_after();
-            const bool last = ks_sh == 0 && q == KB_Z - 1;
-            kstep(t_out, idesc_o, false, 0, first, last ? out_full : nullptr, nullptr); first = false;
-            SBT(6)
-          }
-        } else
-        for (int pr = 0; pr < NPAIR; ++pr) {
-          const int ps = pr & 1;
-          mbar_wait(&slab_full[ps], n_sf[ps] & 1u); ++n_sf[ps];     // both CTAs' slab pair is in shared memory
+        for (int q = 0; q < KB_Z; ++q) {
+          // one hand-off per slab PAIR, on the barrier of the filter slab's stage: both CTAs' two slabs are in their stages' A halves
+          if ((q & 1) == 0) { mbar_wait(&a_ready[stage], (ar_par >> stage) & 1u); ar_par ^= 1u << stage; }
           SBT(5)
           tc_fence_after();
-          const bool last = ks_sh == 0 && pr == NPAIR - 1;
-          kstep(t_out, idesc_o, true, 2 * ps, first, nullptr, nullptr); first = false;
-          kstep(t_out, idesc_o, true, 2 * ps + 1, false, &slab_cons[ps], last ? out_full : nullptr);
+          const bool last = ks_sh == 0 && q == KB_Z - 1;
+          kstep(t_out, idesc_o, q == 0, last ? out_full : nullptr);
           SBT(6)
         }
-        for (int ks = 0; ks < ks_sh; ++ks) kstep(t_out, idesc_o, false, 0, false, ks == ks_sh - 1 ? out_full : nullptr, nullptr);
+        for (int ks = 0; ks < ks_sh; ++ks) kstep(t_out, idesc_o, false, ks == ks_sh - 1 ? out_full : nullptr);
         SBT(7)
       }
 #ifdef TC_TIMELINE
       if (lane == 0 && (blockIdx.x == 0 || blockIdx.x == 40))
-        printf("SBWD cta %d mma: tiles %d  wait_dg_empty %lld  DG ksteps %lld  wait_out_empty %lld  wait_slab_full %lld  unshifted %lld  shifted %lld  (of the ksteps: wait_full_bar %lld)\n",
+        printf("SBWD cta %d mma: tiles %d  wait_dg_empty %lld  DG ksteps %lld  wait_out_empty %lld  wait_a_ready %lld  unshifted %lld  shifted %lld  (of the ksteps: wait_full_bar %lld)\n",
                blockIdx.x, n_tiles, sbt[1], sbt[2], sbt[3], sbt[5], sbt[6], sbt[7], sbt[9]);
 #endif
     }
@@ -406,7 +380,7 @@ tc_stack_bwd_kernel(const TcStackBwdLayer* __restrict__ layers, int* __restrict_
       if (pend) { bulk_wait_group_read<1>(); mbar_arrive(pend); if (pend2) mbar_arrive(pend2); }
       pend = rel; pend2 = rel2;
     };
-    int s_rs = 0; uint32_t s_rp = 0u;      // V2: ring position at the start of the current tile
+    int s_rs = 0; uint32_t s_rp = 0u;      // ring position at the start of the current tile
     auto publish = [&](int* flag) {
       // every store of this thread so far has landed -> visible to the async proxy of other SMs -> count this CTA in
       bulk_wait_group<0>();
@@ -424,25 +398,15 @@ tc_stack_bwd_kernel(const TcStackBwdLayer* __restrict__ layers, int* __restrict_
       tile_ksteps(Ly, n_dg, n_un, n_sh);
       if (!Ly.kind) {
       int u_rs = s_rs; uint32_t u_rp = s_rp;
-      ring_adv(u_rs, u_rp, n_dg);      // V2: stage of the first un-shifted-tap k-step
+      ring_adv(u_rs, u_rp, n_dg);      // stage of the first un-shifted-tap k-step
       for (int pr = 0; pr < NPAIR; ++pr) {
-        const int ps = pr & 1;
-        if constexpr (V2) {
-          named_bar_sync(8 + pr, NEPI * 32 + 32);
-          const int sf = u_rs; ring_adv(u_rs, u_rp, 1);
-          const int ss = u_rs; ring_adv(u_rs, u_rp, 1);
-          if (lane == 0) {
-            tma_store_3d_h(smem + sf * Cfg::STAGE_BYTES, &Ly.tmDZ, pr * 64, t0, b, p.pol_dz_st);
-            tma_store_3d_h(smem + ss * Cfg::STAGE_BYTES, &Ly.tmDZ, D_ + pr * 64, t0, b, p.pol_dz_st);
-            committed(&sfree[sf], &sfree[ss]);
-          }
-        } else {
-        named_bar_sync(8 + ps, NEPI * 32 + 32);
+        named_bar_sync(8 + pr, NEPI * 32 + 32);
+        const int sf = u_rs; ring_adv(u_rs, u_rp, 1);
+        const int ss = u_rs; ring_adv(u_rs, u_rp, 1);
         if (lane == 0) {
-          tma_store_3d_h(dzbuf + (2 * ps) * Cfg::A_BYTES, &Ly.tmDZ, pr * 64, t0, b, p.pol_dz_st);
-          tma_store_3d_h(dzbuf + (2 * ps + 1) * Cfg::A_BYTES, &Ly.tmDZ, D_ + pr * 64, t0, b, p.pol_dz_st);
-          committed(&slab_free[ps]);
-        }
+          tma_store_3d_h(smem + sf * Cfg::STAGE_BYTES, &Ly.tmDZ, pr * 64, t0, b, p.pol_dz_st);
+          tma_store_3d_h(smem + ss * Cfg::STAGE_BYTES, &Ly.tmDZ, D_ + pr * 64, t0, b, p.pol_dz_st);
+          committed(&sfree[sf], &sfree[ss]);
         }
         __syncwarp();
       }
@@ -500,32 +464,19 @@ tc_stack_bwd_kernel(const TcStackBwdLayer* __restrict__ layers, int* __restrict_
   } else if (warp == 12) {
     // ===================== pair hand-off of the d z slabs =====================
     if (lane == 0) {
-      uint32_t n_sd[2] = {0u, 0u};
-      int h_rs = 0; uint32_t h_rp = 0u, ad_par = 0u;      // V2: ring position, per-stage parity of the next a_done phase
+      int h_rs = 0; uint32_t h_rp = 0u, ad_par = 0u;      // ring position, per-stage parity of the next a_done phase
       for (int j = 0; j < n_tiles; ++j) {
         int n_dg, n_un, n_sh;
         { int ly, mt, b, tb; locate(j, ly, mt, b, tb); tile_ksteps(layers[ly], n_dg, n_un, n_sh); }
-        if constexpr (V2) {
-          int u_rs = h_rs; uint32_t u_rp = h_rp;
-          ring_adv(u_rs, u_rp, n_dg);
-          for (int q = 0; q < n_un; q += 2) {
-            mbar_wait(&a_done[u_rs], (ad_par >> u_rs) & 1u); ad_par ^= 1u << u_rs;
-            if (leader) mbar_arrive(&a_ready[u_rs]);
-            else if (p.relaxed_handoff) mbar_arrive_remote_relaxed(&a_ready[u_rs], 0u);
-            else mbar_arrive_remote(&a_ready[u_rs], 0u);
-            ring_adv(u_rs, u_rp, 2);
-          }
-          ring_adv(h_rs, h_rp, n_dg + n_un + n_sh);
-          continue;
+        int u_rs = h_rs; uint32_t u_rp = h_rp;
+        ring_adv(u_rs, u_rp, n_dg);
+        for (int q = 0; q < n_un; q += 2) {
+          mbar_wait(&a_done[u_rs], (ad_par >> u_rs) & 1u); ad_par ^= 1u << u_rs;
+          if (leader) mbar_arrive(&a_ready[u_rs]);
+          else mbar_arrive_remote(&a_ready[u_rs], 0u);
+          ring_adv(u_rs, u_rp, 2);
         }
-        if (n_un == 0) continue;
-        for (int pr = 0; pr < NPAIR; ++pr) {
-          const int ps = pr & 1;
-          mbar_wait(&slab_done[ps], n_sd[ps] & 1u); ++n_sd[ps];
-          if (leader) mbar_arrive(&slab_full[ps]);
-          else if (p.relaxed_handoff) mbar_arrive_remote_relaxed(&slab_full[ps], 0u);
-          else mbar_arrive_remote(&slab_full[ps], 0u);
-        }
+        ring_adv(h_rs, h_rp, n_dg + n_un + n_sh);
       }
     }
   } else if (warp >= 4 && warp < 12) {
@@ -541,11 +492,10 @@ tc_stack_bwd_kernel(const TcStackBwdLayer* __restrict__ layers, int* __restrict_
     const uint32_t grow = (uint32_t)row * 128u, gsw = (uint32_t)(row & 7);
     int islot = 0; uint32_t iphase = 0;
     int oslot = 0; uint32_t ophase = 0;
-    uint32_t n_use[2] = {0u, 0u};      // fills of slab pair slot ps so far
     uint32_t nge = 0u;                 // gated tiles so far
-    int e_rs = 0; uint32_t e_rp = 0u;                              // V2: ring position at the start of the current tile
-    uint32_t eu_pend = 0u, eu_wpar = 0u, eu_npar = 0u;             // V2: per-stage slab-store bookkeeping (see the producer)
-    uint8_t* slab_dst[2] = {nullptr, nullptr};                     // V2: A halves of the stages the current slab pair goes to
+    int e_rs = 0; uint32_t e_rp = 0u;                              // ring position at the start of the current tile
+    uint32_t eu_pend = 0u, eu_wpar = 0u, eu_npar = 0u;             // per-stage slab-store bookkeeping (see the producer)
+    uint8_t* slab_dst[2] = {nullptr, nullptr};                     // A halves of the stages the current slab pair goes to
     int slab_st[2] = {0, 0};
     const TcEpiGateBwd<true>::Params pg{D_};
     const uint32_t lane_base = (uint32_t)(quarter * 32) << 16;
@@ -565,18 +515,18 @@ tc_stack_bwd_kernel(const TcStackBwdLayer* __restrict__ layers, int* __restrict_
       }
       if (!kind) {
       const uint32_t gpar = nge & 1u; ++nge;      // the DG accumulator hand-shakes count gated tiles only
-      // ---- DG epilogue: d z = d g * [P | Q] -> operand buffer
+      // ---- DG epilogue: d z = d g * [P | Q] -> operand ring
       SBT(0)
       mbar_wait(dg_full, gpar);
       SBT(1)
       tc_fence_after();
       int u_rs = e_rs; uint32_t u_rp = e_rp;
-      ring_adv(u_rs, u_rp, n_dg);          // V2: stage of the first un-shifted-tap k-step of this tile
+      ring_adv(u_rs, u_rp, n_dg);          // stage of the first un-shifted-tap k-step of this tile
       {
         TmemAccRow acc{tmem_base + lane_base, true};
 #pragma unroll 1
         for (int step = 0; step < D_ / 32; ++step) {
-          const int pr = step >> 1, ps = pr & 1;
+          const int pr = step >> 1;
           float in[2][16];
           float out[2][16];
           SBT(2)
@@ -601,25 +551,18 @@ tc_stack_bwd_kernel(const TcStackBwdLayer* __restrict__ layers, int* __restrict_
           if (++islot == Cfg::IN_SLOTS) { islot = 0; iphase ^= 1; }
           TcEpiGateBwd<true>::chunk(pg, acc, 0, step * 32 + q * 16, 0, 0, 3u, in, out, nullptr);
           SBT(2)
-          if constexpr (V2) {
-            if ((step & 1) == 0) {
-              // the two ring stages of this slab pair (filter slab, gate slab): free once the MMAs of their previous use have completed
-              // and, if that use carried a slab, its TMA store has read it
+          if ((step & 1) == 0) {
+            // the two ring stages of this slab pair (filter slab, gate slab): free once the MMAs of their previous use have completed
+            // and, if that use carried a slab, its TMA store has read it
 #pragma unroll
-              for (int k = 0; k < 2; ++k) {
-                mbar_wait(&empty_bar[u_rs], u_rp ^ 1u);
-                if ((eu_pend >> u_rs) & 1u) { mbar_wait(&sfree[u_rs], (eu_wpar >> u_rs) & 1u); eu_pend &= ~(1u << u_rs); }
-                eu_wpar = (eu_wpar & ~(1u << u_rs)) | (((eu_npar >> u_rs) & 1u) << u_rs);
-                eu_npar ^= 1u << u_rs; eu_pend |= 1u << u_rs;
-                slab_st[k] = u_rs; slab_dst[k] = smem + u_rs * Cfg::STAGE_BYTES;
-                ring_adv(u_rs, u_rp, 1);
-              }
+            for (int k = 0; k < 2; ++k) {
+              mbar_wait(&empty_bar[u_rs], u_rp ^ 1u);
+              if ((eu_pend >> u_rs) & 1u) { mbar_wait(&sfree[u_rs], (eu_wpar >> u_rs) & 1u); eu_pend &= ~(1u << u_rs); }
+              eu_wpar = (eu_wpar & ~(1u << u_rs)) | (((eu_npar >> u_rs) & 1u) << u_rs);
+              eu_npar ^= 1u << u_rs; eu_pend |= 1u << u_rs;
+              slab_st[k] = u_rs; slab_dst[k] = smem + u_rs * Cfg::STAGE_BYTES;
+              ring_adv(u_rs, u_rp, 1);
             }
-          } else
-          if ((step & 1) == 0 && n_use[ps] > 0) {
-            // the slot still holds an earlier slab pair: its MMAs must have completed and its TMA stores read the buffer
-            mbar_wait(&slab_cons[ps], (n_use[ps] - 1u) & 1u);
-            mbar_wait(&slab_free[ps], (n_use[ps] - 1u) & 1u);
           }
           SBT(4)
           {
@@ -628,7 +571,7 @@ tc_stack_bwd_kernel(const TcStackBwdLayer* __restrict__ layers, int* __restrict_
             const uint32_t j0 = (uint32_t)(ch >> 3);
 #pragma unroll
             for (int k = 0; k < 2; ++k) {
-              uint8_t* gs = (V2 ? slab_dst[k] : dzbuf + (2 * ps + k) * Cfg::A_BYTES) + grow;
+              uint8_t* gs = slab_dst[k] + grow;
               uint4 a, c;
               a.x = pack_bf16x2(out[k][0], out[k][1]); a.y = pack_bf16x2(out[k][2], out[k][3]);
               a.z = pack_bf16x2(out[k][4], out[k][5]); a.w = pack_bf16x2(out[k][6], out[k][7]);
@@ -641,14 +584,9 @@ tc_stack_bwd_kernel(const TcStackBwdLayer* __restrict__ layers, int* __restrict_
           if (step & 1) {
             // slab pair complete in this CTA: store warp (HBM copy) and, through the hand-off warp, the MMA side
             fence_proxy_async();
-            named_bar_arrive(8 + (V2 ? pr : ps), NEPI * 32 + 32);
+            named_bar_arrive(8 + pr, NEPI * 32 + 32);
             __syncwarp();
-            if constexpr (V2) {
-              if (lane == 0) mbar_arrive(&a_done[slab_st[0]]);      // (the pair's hand-off rides on the filter slab's stage)
-            } else {
-              if (lane == 0) mbar_arrive(&slab_done[ps]);
-            }
-            ++n_use[ps];
+            if (lane == 0) mbar_arrive(&a_done[slab_st[0]]);      // (the pair's hand-off rides on the filter slab's stage)
           }
         }
       }
@@ -823,15 +761,15 @@ static int tc_stack_bwd_build_t(TmapCache& tc, const std::vector<TcStackBwdDesc>
   return 0;
 }
 
-template <int D_, int R_, bool V2>
+template <int D_, int R_>
 static int tc_stack_bwd_launch_t(cudaStream_t st, const TcStackBwdPlan& plan, const TcStackBwdDesc& d0) {
-  using Cfg = TcStackBwdCfg<D_, R_, V2>;
+  using Cfg = TcStackBwdCfg<D_, R_>;
   TcStackBwdParams p{};
   p.B = d0.B; p.T = d0.T; p.tiles_t = (d0.T + 255) / 256; p.num_mtiles = d0.B * p.tiles_t; p.L = plan.L;
   p.nseg = d0.nseg; p.kb_dx = d0.R / 64; p.kb_ds = d0.S / 64; p.drop_scale = d0.drop_scale;
   p.pol_dx = tc_policy(TC_L2_NORMAL); p.pol_ds = tc_policy(TC_L2_LAST); p.pol_w = tc_policy(TC_L2_LAST); p.pol_z = tc_policy(TC_L2_FIRST);
   p.pol_dz_ld = tc_policy(TC_L2_NORMAL); p.pol_dz_st = tc_policy(TC_L2_LAST); p.pol_o = tc_policy(TC_L2_LAST);
-  auto kern = tc_stack_bwd_kernel<D_, R_, V2>;
+  auto kern = tc_stack_bwd_kernel<D_, R_>;
   static unsigned long long attr_devs = 0ull;
   if (tc_first_use_on_device(&attr_devs)) {
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES);
@@ -840,16 +778,12 @@ static int tc_stack_bwd_launch_t(cudaStream_t st, const TcStackBwdPlan& plan, co
   const int pairs = tc_num_sms() / 2;
   if (p.num_mtiles <= pairs) return -100;
   {
-    // bands of ~WN_TC_SB_BAND m tiles (default 128; 0: one band = layer-major order), every band longer than the launch has pairs
-    // (a tile then never waits for a tile of the round its own pair is in).
+    // bands of ~128 m tiles, every band longer than the launch has pairs (a tile then never waits for a tile of the round its own
+    // pair is in).
     // (Tried and dropped: issuing DG of a pair's next tile between the un-shifted and the shifted taps of the current one, to
     // fill the d z round trip through L2 — the OUT epilogue then no longer runs under those DG products: 1.79 -> 2.03 ms.)
-    static int relaxed = -1;
-    if (relaxed < 0) { const char* e = getenv("WN_TC_HANDOFF_RELAXED"); relaxed = (e && e[0] == '1') ? 1 : 0; }
-    p.relaxed_handoff = relaxed;
-    static int band_target = -1;
-    if (band_target < 0) { const char* e = getenv("WN_TC_SB_BAND"); band_target = e ? atoi(e) : 128; }
-    int nb = band_target > 0 ? p.num_mtiles / band_target : 1;
+    constexpr int band_target = 128;
+    int nb = p.num_mtiles / band_target;
     if (nb < 1) nb = 1;
     for (; nb > 1; --nb) {
       const int bw = (p.num_mtiles + nb - 1) / nb;
@@ -889,12 +823,9 @@ static int tc_stack_bwd_launch_t(cudaStream_t st, const TcStackBwdPlan& plan, co
 static inline int tc_stack_bwd_build(TmapCache& tc, const std::vector<TcStackBwdDesc>& descs, TcStackBwdPlan* plan) {
   const TcStackBwdDesc& d = descs[0];
   if (d.D == 256 && d.R == 256) return tc_stack_bwd_build_t<256, 256>(tc, descs, plan);
-  if (d.D == 128 && d.R == 128) return tc_stack_bwd_build_t<128, 128>(tc, descs, plan);
   return -100;
 }
-// v2: d z slabs through the operand ring's A halves (5 stages, no separate operand buffer) — see TcStackBwdCfg
-static inline int tc_stack_bwd_launch(cudaStream_t st, const TcStackBwdPlan& plan, const TcStackBwdDesc& d, bool v2) {
-  if (d.D == 256 && d.R == 256) return v2 ? tc_stack_bwd_launch_t<256, 256, true>(st, plan, d) : tc_stack_bwd_launch_t<256, 256, false>(st, plan, d);
-  if (d.D == 128 && d.R == 128) return v2 ? tc_stack_bwd_launch_t<128, 128, true>(st, plan, d) : tc_stack_bwd_launch_t<128, 128, false>(st, plan, d);
+static inline int tc_stack_bwd_launch(cudaStream_t st, const TcStackBwdPlan& plan, const TcStackBwdDesc& d) {
+  if (d.D == 256 && d.R == 256) return tc_stack_bwd_launch_t<256, 256>(st, plan, d);
   return -100;
 }

@@ -99,22 +99,6 @@ __device__ __forceinline__ void tma_load_4d_pair(void* dst, const CUtensorMap* m
       "l"(m), "r"(smem_u32(bar) & 0xFEFFFFFFu), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
       : "memory");
 }
-// multicast variant: the box lands at the same shared-memory offset of every CTA in `mask`, and each
-// destination CTA's mbarrier (same offset) receives the complete_tx
-__device__ __forceinline__ void tma_load_4d_mc(void* dst, const CUtensorMap* m, uint64_t* bar, int c0, int c1, int c2, int c3, uint16_t mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%3, %4, %5, %6}], [%2], %7;" ::"r"(
-          smem_u32(dst)),
-      "l"(m), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "h"(mask)
-      : "memory");
-}
-__device__ __forceinline__ void tma_load_2d_mc(void* dst, const CUtensorMap* m, uint64_t* bar, int c0, int c1, uint16_t mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%3, %4}], [%2], %5;" ::"r"(
-          smem_u32(dst)),
-      "l"(m), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "h"(mask)
-      : "memory");
-}
 // ---------------------------------------------------------------- thread-block clusters
 __device__ __forceinline__ uint32_t cluster_ctarank() {
   uint32_t r;
@@ -149,12 +133,6 @@ __device__ __forceinline__ void mbar_arrive_remote_relaxed(uint64_t* bar, uint32
 #define TC_POL_NORMAL 0x1000000000000000ull
 #define TC_POL_FIRST 0x12F0000000000000ull
 #define TC_POL_LAST 0x14F0000000000000ull
-__device__ __forceinline__ void tma_load_2d_h(void* dst, const CUtensorMap* m, uint64_t* bar, int c0, int c1, uint64_t pol) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1, {%3, %4}], [%2], %5;" ::"r"(smem_u32(dst)),
-      "l"(m), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "l"(pol)
-      : "memory");
-}
 __device__ __forceinline__ void tma_load_3d_h(void* dst, const CUtensorMap* m, uint64_t* bar, int c0, int c1, int c2, uint64_t pol) {
   asm volatile(
       "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1, {%3, %4, %5}], [%2], %6;" ::"r"(smem_u32(dst)),
@@ -193,10 +171,6 @@ __device__ __forceinline__ void tma_store_3d_h(const void* src, const CUtensorMa
   asm volatile("cp.async.bulk.tensor.3d.global.shared::cta.bulk_group.L2::cache_hint [%0, {%2, %3, %4}], [%1], %5;" ::"l"(m), "r"(smem_u32(src)),
                "r"(c0), "r"(c1), "r"(c2), "l"(pol)
                : "memory");
-}
-// L2 prefetch of a tile (no shared memory, no barrier)
-__device__ __forceinline__ void tma_prefetch_l2_3d(const CUtensorMap* m, int c0, int c1, int c2) {
-  asm volatile("cp.async.bulk.prefetch.tensor.3d.L2.global [%0, {%1, %2, %3}];" ::"l"(m), "r"(c0), "r"(c1), "r"(c2) : "memory");
 }
 // smem -> global tile store (bulk async group); rows / columns outside the tensor are clipped
 __device__ __forceinline__ void tma_store_3d(const void* src, const CUtensorMap* m, int c0, int c1, int c2) {
@@ -262,11 +236,6 @@ __device__ __forceinline__ void umma_commit_pair(uint64_t* bar) {
 // all previously issued tcgen05.mma of this thread arrive on `bar` when complete
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-// same, arriving on the barrier at that offset in every CTA of `mask`
-__device__ __forceinline__ void umma_commit_mc(uint64_t* bar, uint16_t mask) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(smem_u32(bar)), "h"(mask)
-               : "memory");
 }
 // 32 lanes x 16 consecutive fp32 columns: thread i of the warp gets lane (lane_base + i)
 __device__ __forceinline__ void tmem_ld16(uint32_t taddr, float* v) {

@@ -31,12 +31,9 @@ __device__ __forceinline__ void ld_bias16(const float* p, float* v) {   // share
 // out = act(acc + bias[n] + cbias[b][n]) + res      (layers.py:66-74,213,222-223; model.py:105-119,236)
 // (2 input half-panels: the skip sum and the head convs have no epilogue input at all and get 5 mainloop stages; the unfused
 // conv1 with a residual input keeps a 2-slot ring.  C2: 6.10 -> 6.00 ms/step, same box)
-#ifndef TC_BIASACTRES_IN_PANELS
-#define TC_BIASACTRES_IN_PANELS 2
-#endif
 template <bool FAST> struct TcEpiBiasActRes {
   static constexpr int NIN = 1, NOUT = 1;
-  static constexpr int kInPanels = TC_BIASACTRES_IN_PANELS, kOutSlots = 4;
+  static constexpr int kInPanels = 2, kOutSlots = 4;
   static constexpr bool kGate = false;
   struct Params { const float* bias; const float* cbias; int ldcb; int act; int N; };
   static constexpr int kBiasFloats(int BN) { return BN; }
@@ -126,24 +123,12 @@ template <bool FAST> struct TcEpiGate {
 };
 
 // adjoint of the gate: acc = dg; inputs the cached derivative coefficients P, Q (see TcEpiGate); outputs dz_f, dz_s
-#ifndef TC_GATEBWD_IN_PANELS
-#define TC_GATEBWD_IN_PANELS 8
-#endif
-#ifndef TC_GATEBWD_OUT_SLOTS
-#define TC_GATEBWD_OUT_SLOTS 2
-#endif
 // Ring depths trade against mainloop stages (every 4 half-panels = one 32 KB operand stage).  Measured on C2 (same box, ms/step):
 // dgrad with 4 input half-panels (4 mainloop stages instead of 3) 6.10 vs 6.25; gate adjoint with 4 instead of 8: 6.36 (its
 // epilogue streams z from HBM and wants the deep ring).
-#ifndef TC_ACTBWD_IN_PANELS
-#define TC_ACTBWD_IN_PANELS 4
-#endif
-#ifndef TC_ACTBWD_OUT_SLOTS
-#define TC_ACTBWD_OUT_SLOTS 4
-#endif
 template <bool FAST> struct TcEpiGateBwd {
   static constexpr int NIN = 2, NOUT = 2;
-  static constexpr int kInPanels = TC_GATEBWD_IN_PANELS, kOutSlots = TC_GATEBWD_OUT_SLOTS;
+  static constexpr int kInPanels = 8, kOutSlots = 2;
   static constexpr bool kGate = false;
   struct Params { int D; };
   static constexpr int kBiasFloats(int BN) { return 0; }
@@ -164,7 +149,7 @@ template <bool FAST> struct TcEpiGateBwd {
 // dgrad: out = (acc + add) * act'(y)    (residual pass-through; activation adjoint from its cached output)
 struct TcEpiActBwd {
   static constexpr int NIN = 2, NOUT = 1;
-  static constexpr int kInPanels = TC_ACTBWD_IN_PANELS, kOutSlots = TC_ACTBWD_OUT_SLOTS;
+  static constexpr int kInPanels = 4, kOutSlots = 4;
   static constexpr bool kGate = false;
   struct Params { int act; };
   static constexpr int kBiasFloats(int BN) { return 0; }

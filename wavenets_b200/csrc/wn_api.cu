@@ -221,16 +221,12 @@ struct wn_handle {
   // backward on two streams: the weight-gradient kernels of a block run beside its dgrad chain
   cudaStream_t side_stream = nullptr;
   std::vector<cudaEvent_t> ev_blk_in, ev_blk_dz, ev_blk_done;
-  int use_side = 1;
-  int use_res_gemm = 1;     // WN_TC_RES_GEMM=0: residual added in the epilogue (A/B switch)
-  int use_fused_fwd = 1;    // WN_TC_FUSED_FWD=0: gated conv and conv1 as separate launches (A/B switch)
   int stack_fwd_layers = 0;   // layers of the last forward inside the stack launch
   int use_stack_fwd = 1;    // WN_TC_STACK_FWD=0: one fused launch per block instead of one for the whole stack (gemm_tc_stack.cuh)
   std::vector<TcStackPlan> stack_plans;
   // backward chain (gate adjoint + dgrad of every block) as one persistent launch (gemm_tc_stack_bwd.cuh); WN_TC_STACK_BWD=0: per-block launches
-  int use_stack_bwd = 2, stack_bwd_layers = 0;   // 2: d z slabs through the operand ring's A halves (5 stages), 1: separate operand buffer, 0: per-block chain
+  int use_stack_bwd = 1, stack_bwd_layers = 0;
   std::vector<TcStackBwdPlan> stack_bwd_plans;
-  int tile_gate_bwd = 0, tile_dgrad = 0;   // forced CTA tile widths of the two backward conv GEMMs (0 = widest that divides N)
   int fused_fwd_launches = 0;  // fused block-forward launches of the last step (0: separate gate / conv1 kernels)
   // grouped weight gradients (gemm_tc_wgroup.cuh): d z and d x_out of EVERY block are kept (no ping-pong) and all block
   // weight gradients run as one launch behind the dgrad chain.  WN_TC_GROUP_WGRAD=0 switches back to per-block launches.
@@ -242,15 +238,12 @@ struct wn_handle {
   struct WgPlan { int B, T; bool drop; bool sb; int nb; TcWgGroupPlan plan; };
   std::vector<WgPlan> wg_plans;
   std::vector<TcWgJobDesc> wg_jobs;   // collected by block_backward while a pass is enqueued
-  int dskip_l2_last = 0;
   int wg_last_tiles = 0, wg_last_side = 0;   // grouped tiles / side launches of the last backward pass
   int wg_last_partials = 0;                  // fp32 partial tiles (tiles x row splits) its finish launch reads
   int wg_cur_group = -1;              // side group of the jobs block_backward appends (-1: final launch)
   int wg_side_every = 5;              // every n-th block hands its weight gradients to a side launch (WN_TC_GROUP_SIDE_EVERY, 0 = off)
   cudaEvent_t ev_wg_side = nullptr;
   int wg_force_split = 0, wg_pair_tiles = 1;   // WN_TC_GROUP_SPLIT=n / WN_TC_GROUP_NH2=0: A/B switches
-  int use_merged_finish = 0;  // WN_TC_MERGED_FINISH=1: one finish launch for both wgrads of a block. Measured SLOWER on C2 (7.48 vs
-                              // 7.38 ms/step: the deferred partials fall out of L2 before the merged finish reads them) -> off
   // every weight re-pack as one launch: job table recorded on the first wn_params_changed (buffers never move)
   // autoregressive generation state (wn_generate): histories of every dilated conv's input, scratch, step graphs
   struct Gen {
@@ -260,8 +253,6 @@ struct wn_handle {
     std::vector<float*> wcat, bcat;          // per block [D][R+S] = [Wr | Ws], [R+S]: conv1 and conv_skip as one product
     std::vector<void*> allocs;
   } gen;
-  // deferred wgrad finish (see WgradH::defer_finish)
-  TcWgradFinish pend_finish{}; bool pend_valid = false; int pend_blocks = 0; long long pend_partial_elems = 0, pend_cs_elems = 0;
   std::vector<PackJob> pack_jobs;
   PackJob* d_pack_jobs = nullptr; long long pack_blocks = 0; bool pack_ready = false;
   // data parallelism (train.py:203): NCCL communicator of the replicas; the gradient all-reduce is the only collective
@@ -506,17 +497,16 @@ static void layout_buffers(wn_handle* h) {
   }
   for (auto& c : h->head) upd(c.cin, c.cout);
   h->wg_partial_elems = maxkn * WN_MAX_WGRAD_SPLITS;
-  // x2: a deferred finish keeps one problem's partials in place while the next wgrad writes behind them
-  h->wg_partial = (float*)W.take((size_t)h->wg_partial_elems * 4 * 2);
-  h->wg_partial_side = (float*)W.take((size_t)h->wg_partial_elems * 4 * 2);
+  h->wg_partial = (float*)W.take((size_t)h->wg_partial_elems * 4);
+  h->wg_partial_side = (float*)W.take((size_t)h->wg_partial_elems * 4);
   if (bf) {
     int max_mt = 1;
     auto mt = [&](int K, int cin) { const int m = K * cdiv(cin, 128); if (m > max_mt) max_mt = m; };
     for (auto& b : h->blocks) { for (auto& c : b.stack) mt(c.K, c.cin); mt(1, D); }
     if (h->Ccs > 0) mt(1, h->Ccs);
     for (auto& c : h->head) mt(1, c.cin);
-    h->cs_partial = (float*)W.take((size_t)tc_wgrad_cs_rows(h->maxB, h->maxT, max_mt) * (size_t)rup(nmax, 4) * 4 * 2);
-    h->cs_partial_side = (float*)W.take((size_t)tc_wgrad_cs_rows(h->maxB, h->maxT, max_mt) * (size_t)rup(nmax, 4) * 4 * 2);
+    h->cs_partial = (float*)W.take((size_t)tc_wgrad_cs_rows(h->maxB, h->maxT, max_mt) * (size_t)rup(nmax, 4) * 4);
+    h->cs_partial_side = (float*)W.take((size_t)tc_wgrad_cs_rows(h->maxB, h->maxT, max_mt) * (size_t)rup(nmax, 4) * 4);
   }
   h->loss_parts_cap = cdiv((long long)rows, 8) + 8;
   h->loss_partial = (float*)W.take((size_t)h->loss_parts_cap * 4);
@@ -555,7 +545,6 @@ static void layout_buffers(wn_handle* h) {
 extern "C" int wn_create(const wn_config* cfg, wn_handle** out) {
   if (!cfg || !out) { set_err("null argument"); return WN_ERR_VALUE; }
   *out = nullptr;
-  const char* env_res = getenv("WN_TC_RES_GEMM");
   RET(validate_config(*cfg));
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
@@ -712,16 +701,8 @@ extern "C" int wn_create(const wn_config* cfg, wn_handle** out) {
   cudaEventCreateWithFlags(&h->ev_in, cudaEventDisableTiming);
   cudaEventCreateWithFlags(&h->ev_out, cudaEventDisableTiming);
   { const char* e = getenv("WN_CUDA_GRAPH"); if (e && e[0] == '0') h->use_graphs = 0; }
-  { const char* e = getenv("WN_SIDE_STREAM"); if (e && e[0] == '0') h->use_side = 0; }
-  if (env_res && env_res[0] == '0') h->use_res_gemm = 0;
-  { const char* e = getenv("WN_TC_FUSED_FWD"); if (e && e[0] == '0') h->use_fused_fwd = 0; }
   { const char* e = getenv("WN_TC_STACK_FWD"); if (e && e[0] == '0') h->use_stack_fwd = 0; }
-  { const char* e = getenv("WN_TC_STACK_BWD"); if (e) h->use_stack_bwd = atoi(e); }      // 0: per-block chain, 1: first version, 2: slabs through the ring
-  { const char* e = getenv("WN_TC_TILE_GATE_BWD"); if (e) h->tile_gate_bwd = atoi(e); }
-  { const char* e = getenv("WN_TC_TILE_DGRAD"); if (e) h->tile_dgrad = atoi(e); }
-  { const char* e = getenv("WN_TC_MERGED_FINISH"); if (e && e[0] == '1') h->use_merged_finish = 1; }
-  { const char* e = getenv("WN_TC_BALANCE_GRID"); if (e) g_tc_balance_env = atoi(e); }
-  { const char* e = getenv("WN_TC_DSKIP_LAST"); if (e) h->dskip_l2_last = atoi(e); }
+  { const char* e = getenv("WN_TC_STACK_BWD"); if (e && e[0] == '0') h->use_stack_bwd = 0; }
   cudaStreamCreateWithFlags(&h->side_stream, cudaStreamNonBlocking);
   cudaEventCreateWithFlags(&h->ev_wg_side, cudaEventDisableTiming);
   {
@@ -1026,9 +1007,6 @@ struct WgradH {
   int N0 = 0; float* dst1 = nullptr; const float* w1 = nullptr; float* bias1 = nullptr;
   bool side = false;   // issued on the side stream: uses the side copies of the partial buffers
   int l2_a = 0, l2_g = 0;   // bf16 tier: L2 policy codes of the two operands
-  // bf16 tier: `defer_finish` leaves the split partials in place (no finish launch); the next wgrad on the same stream
-  // with `merge_prev` writes its partials behind them and finishes both problems with ONE launch
-  bool defer_finish = false, merge_prev = false;
 };
 
 template <class T>
@@ -1075,15 +1053,8 @@ static int run_wgrad(wn_handle* h, cudaStream_t st, int cls, const WgradH& g) {
     d.B = g.B; d.T = g.T; d.N = g.N; d.G = (const bf16*)g.G; d.ldg = g.ldg; d.nseg = g.nseg; d.ktot = ktot;
     for (int s = 0; s < g.nseg; ++s) d.seg[s] = TcSeg{(const bf16*)g.seg[s].A, g.seg[s].lda, g.seg[s].shift, g.seg[s].K};
     d.l2_a = g.l2_a; d.l2_g = g.l2_g;
-    if (h->pend_valid && !g.merge_prev) {
-      // a deferred finish that nobody merged (should not happen): run it on its own before its partials are reused
-      LaunchScope ls(h, st, cls);
-      tc_wgrad_finish<<<h->pend_blocks, 256, 0, st>>>(h->pend_finish);
-      h->pend_valid = false;
-    }
-    const bool merging = g.merge_prev && h->pend_valid;
-    float* const wgp = (g.side ? h->wg_partial_side : h->wg_partial) + (merging ? h->pend_partial_elems : 0);
-    float* const csp = (g.side ? h->cs_partial_side : h->cs_partial) + (merging ? h->pend_cs_elems : 0);
+    float* const wgp = g.side ? h->wg_partial_side : h->wg_partial;
+    float* const csp = g.side ? h->cs_partial_side : h->cs_partial;
     d.partial = wgp;
     const bool want_cs = g.bias_dst || g.per_batch || g.bias1;
     d.cs_partial = want_cs ? csp : nullptr;
@@ -1101,29 +1072,14 @@ static int run_wgrad(wn_handle* h, cudaStream_t st, int cls, const WgradH& g) {
     f.bias0 = g.bias_dst; f.bias1 = g.bias1; f.per_batch = g.per_batch; f.ldpb = g.ldpb;
     f.wblocks = cdiv((long long)ktot * g.N, 256);
     const int nblocks = f.wblocks + (want_cs ? cdiv(g.N, 32) : 0);
-    const long long part_elems = (long long)plan.nsplit * ktot * g.N;
-    const long long cs_elems = (long long)plan.nsplit * plan.mtiles * plan.slots * g.N;
-    if (g.defer_finish && !merging) {
-      // keep the partials; the next wgrad of this stream finishes both
-      h->pend_finish = f; h->pend_valid = true; h->pend_blocks = nblocks;
-      h->pend_partial_elems = (part_elems + 63) / 64 * 64; h->pend_cs_elems = (cs_elems + 63) / 64 * 64;
-      return WN_OK;
-    }
+    // one finish per weight gradient: one finish launch for both wgrads of a block measured SLOWER on C2 (7.48 vs 7.38 ms/step:
+    // the deferred partials fall out of L2 before the merged finish reads them)
     LaunchScope ls(h, st, cls);
-    {
-      cudaLaunchConfig_t cfg{};
-      cfg.blockDim = dim3(256); cfg.dynamicSmemBytes = 0; cfg.stream = st;
-      cudaLaunchAttribute attr[2];
-      cfg.attrs = attr; cfg.numAttrs = tc_launch_attrs(attr, 1);
-      if (merging) {
-        cfg.gridDim = dim3(h->pend_blocks + nblocks);
-        h->pend_valid = false;
-        CK(cudaLaunchKernelEx(&cfg, tc_wgrad_finish2, h->pend_finish, f, h->pend_blocks));
-      } else {
-        cfg.gridDim = dim3(nblocks);
-        CK(cudaLaunchKernelEx(&cfg, tc_wgrad_finish, f));
-      }
-    }
+    cudaLaunchConfig_t cfg{};
+    cfg.gridDim = dim3(nblocks); cfg.blockDim = dim3(256); cfg.dynamicSmemBytes = 0; cfg.stream = st;
+    cudaLaunchAttribute attr[2];
+    cfg.attrs = attr; cfg.numAttrs = tc_launch_attrs(attr, 1);
+    CK(cudaLaunchKernelEx(&cfg, tc_wgrad_finish, f));
     return WN_OK;
   }
   {
@@ -1161,11 +1117,10 @@ static void fill_w(GemmH& g, const ConvP& c, bool dgrad) {
 
 // conditioning: mapping MLP (model.py:141-148,222) and the per-block time-constant bias
 // cb[l][b][:] = cond[b] @ Wc_l + bc_l  (layers.py:203-204 with cond constant in time)
-// one single-block launch each way for the conditioning MLP while it is as small as it really is (WN_FUSED_MAPPING=0: per layer)
+// one single-block launch each way for the conditioning MLP while it is as small as it really is (above 2^20 MACs: per layer)
 static bool mapping_args(wn_handle* h, const float* cond_in, int B, float l2coef, MapArgs* a) {
-  static const int enabled = [] { const char* e = getenv("WN_FUSED_MAPPING"); return e ? atoi(e) : 1; }();
   const int nl = (int)h->map_w.size();
-  if (!enabled || nl < 1 || nl > WN_MAX_LIST) return false;
+  if (nl < 1 || nl > WN_MAX_LIST) return false;
   long long macs = 0;
   int k = h->cfg.cond_in;
   for (int i = 0; i < nl; ++i) { macs += (long long)B * k * h->map_width[i]; k = h->map_width[i]; }
@@ -1242,7 +1197,7 @@ static int block_forward(wn_handle* h, cudaStream_t st, int l, const void* x_in,
     } else {
       if constexpr (sizeof(T) == 2) {
         // bf16 tier: gated conv + gate + conv1 (+ residual) as ONE kernel when the shapes allow (gemm_tc_block.cuh)
-        if (h->use_fused_fwd && b.Wres16 && h->cfg.use_residual && tc_cta_group() == 2 && c.K <= TC_MAX_TAPS && !h->cond_seq) {
+        if (b.Wres16 && h->cfg.use_residual && c.K <= TC_MAX_TAPS && !h->cond_seq) {
           TcBlockDesc d{};
           d.B = B; d.T = Tn; d.nseg = c.K; d.Cin = c.cin; d.D = h->D; d.R = h->R; d.has_res = 1;
           for (int k = 0; k < c.K; ++k) d.shift[k] = -(c.K - 1 - k) * c.dil;
@@ -1290,7 +1245,7 @@ static int block_forward(wn_handle* h, cudaStream_t st, int l, const void* x_in,
     typename EpiBiasActRes<T, T, sizeof(T) == 2>::Params ep{};
     ep.out = (T*)h->xout[l]; ep.ldo = h->R; ep.bias = P_(h, c.b_idx); ep.act = ACT_LINEAR;
     ep.res = h->cfg.use_residual ? (const T*)x_in : nullptr; ep.ldr = h->R; ep.N = h->R; ep.vec = vec_ok<T>(h->R);
-    if (sizeof(T) == 2 && b.Wres16 && h->use_res_gemm) {
+    if (sizeof(T) == 2 && b.Wres16) {
       // residual through the contraction: second segment x_in against the identity block of [Wr^T | I]
       g.nseg = 2;
       g.seg[1] = SegH{x_in, h->R, 0, h->R};
@@ -1354,7 +1309,7 @@ static int model_forward(wn_handle* h, cudaStream_t st, const float* x, int ldx,
     // the whole residual stack as ONE persistent launch (gemm_tc_stack.cuh) when every block takes the fused forward
     // and a layer has more 256-row tiles than the GPU has CTA pairs.  Multi-dilation blocks (layers.py:64-88): every conv in
     // front of the gated conv is a PLAIN layer of the same launch (its output is kept for the backward pass, as before).
-    bool ok = h->use_stack_fwd && h->use_fused_fwd && tc_cta_group() == 2 && c.use_residual && h->L >= 2 && h->D == h->R &&
+    bool ok = h->use_stack_fwd && c.use_residual && h->L >= 2 && h->D == h->R &&
               (h->D == 256 || h->D == 128) && B * cdiv(Tn, 256) > tc_num_sms() / 2;
     for (auto& b : h->blocks) {
       if (!ok) break;
@@ -1626,7 +1581,6 @@ static int block_backward(wn_handle* h, cudaStream_t st, int l, const void* x_in
     w.N0 = R; w.dst1 = G_(h, b.conv_skip.w_idx); w.w1 = P_(h, b.conv_skip.w_idx); w.bias1 = G_(h, b.conv_skip.b_idx);
     w.side = side1;
     w.l2_a = TC_L2_FIRST;   // last use of g_l
-    w.defer_finish = side1 && h->use_merged_finish;   // finished together with the gated conv's wgrad below (same stream)
     RET(run_wgrad<T>(h, s1, CLS_GEMM, w));
   } else if (d_o) {
     WgradH w{};
@@ -1664,14 +1618,12 @@ static int block_backward(wn_handle* h, cudaStream_t st, int l, const void* x_in
       if (use_o) g.seg[g.nseg++] = SegH{d_o, ld_o, 0, R};
       else koff = R;
       if (use_s) {
-        // d skip is the same tensor for every block (model.py:236): ask L2 to keep it between the blocks' launches
-        if (group && h->dskip_l2_last) g.l2_seg[g.nseg] = TC_L2_LAST;
         g.seg[g.nseg++] = SegH{dskip, ldsk, 0, S};
       }
     }
     const int rs = R + (b.has_skip ? S : 0);
     g.W32 = b.Wdg ? b.Wdg + (size_t)koff * b.Dpad : nullptr; g.Npad = b.Dpad;
-    g.W16 = b.Wdg16 ? b.Wdg16 + koff : nullptr; g.ktot16 = rup(rs, 64); g.N16 = b.Dpad; g.tile16 = h->tile_gate_bwd;
+    g.W16 = b.Wdg16 ? b.Wdg16 + koff : nullptr; g.ktot16 = rup(rs, 64); g.N16 = b.Dpad; g.tile16 = 0;
     typename EpiGateBwd<T, sizeof(T) == 2>::Params ep{};
     ep.z = (const T*)h->zbuf[l]; ep.dz = (T*)dzbuf; ep.D = D; ep.vec = vec_ok<T>(D);
     // last use of z; dz is read next by the dgrad and the weight-gradient kernels
@@ -1711,7 +1663,6 @@ static int block_backward(wn_handle* h, cudaStream_t st, int l, const void* x_in
       const bool side2 = sd != nullptr && j == depth - 1;
       if (side2) CK(cudaStreamWaitEvent(sd->side, sd->ev_dz, 0));
       w.side = side2;
-      w.merge_prev = side2 && h->pend_valid;
       w.l2_a = TC_L2_FIRST;   // last use of this forward activation
       RET(run_wgrad<T>(h, side2 ? sd->side : st, CLS_DILATED, w));
     }
@@ -1727,7 +1678,6 @@ static int block_backward(wn_handle* h, cudaStream_t st, int l, const void* x_in
       g.B = B; g.T = Tn; g.N = c.cin; g.nseg = c.K;
       for (int k = 0; k < c.K; ++k) g.seg[k] = SegH{dcur, dcw, +(c.K - 1 - k) * c.dil, c.cout};
       fill_w(g, c, true);
-      g.tile16 = h->tile_dgrad;
       typename EpiActBwd<T, T>::Params ep{};
       ep.N = c.cin;
       if (j > 0) {
@@ -1756,12 +1706,6 @@ static int block_backward(wn_handle* h, cudaStream_t st, int l, const void* x_in
         RET((run_conv_gemm<T, EpiActBwd<T, T>>(h, st, CLS_DILATED, g, ep)));
       }
     }
-  }
-  if (h->pend_valid) {
-    // deferred finish that found no partner in this block: run it on the stream its wgrad used
-    LaunchScope ls(h, s1, CLS_GEMM);
-    tc_wgrad_finish<<<h->pend_blocks, 256, 0, s1>>>(h->pend_finish);
-    h->pend_valid = false;
   }
   if (sd) CK(cudaEventRecord(sd->ev_done, sd->side));
   return WN_OK;
@@ -1850,7 +1794,7 @@ static int model_backward(wn_handle* h, cudaStream_t st, const float* x, int ldx
   const wn_config& c = h->cfg;
   // (bf16 tier only: the fp32 tier's wgrad / column-sum scratch buffers are not duplicated for a second stream)
   const bool group = sizeof(T) == 2 && h->use_group_wgrad;
-  const bool use_side = sizeof(T) == 2 && h->use_side && h->prof_tag == 0 && h->side_stream != nullptr && !group;
+  const bool use_side = sizeof(T) == 2 && h->prof_tag == 0 && h->side_stream != nullptr && !group;
   const bool cat = sizeof(T) == 2 && h->dcatA != nullptr;
   const int ldc = h->R + h->S;
   const size_t rows_cap = (size_t)h->maxB * h->maxT;
@@ -1862,12 +1806,12 @@ static int model_backward(wn_handle* h, cudaStream_t st, const float* x, int ldx
   // (256 tiles: 4 rounds on 74 or on 64 pairs), and the pairs left over run the weight gradients of every n-th block
   // beside the chain.  The plan (unit ranges per side group) exists from the second call on; the first call launches
   // every group at the end.
-  // Backward chain as ONE persistent launch (gemm_tc_stack_bwd.cuh): single-dilation blocks, D = R in {128, 256}, d z / d x_out
+  // Backward chain as ONE persistent launch (gemm_tc_stack_bwd.cuh): D = R = 256, d z / d x_out
   // of every block kept (grouped weight gradients), more 256-row tiles per layer than CTA pairs.  It takes every SM for the
   // whole chain, so the weight gradients all run in the one grouped launch behind it (no side launches).
   bool sb_ok = false;
   if constexpr (sizeof(T) == 2) {
-    sb_ok = group && !cat && h->use_stack_bwd && tc_cta_group() == 2 && h->L >= 2 && h->D == h->R && (h->D == 256 || h->D == 128) &&
+    sb_ok = group && !cat && h->use_stack_bwd && h->L >= 2 && h->D == h->R && h->D == 256 &&
             h->K <= TC_MAX_TAPS && B * cdiv(Tn, 256) > tc_num_sms() / 2;
     for (auto& b : h->blocks) {
       if (!sb_ok) break;
@@ -1879,7 +1823,7 @@ static int model_backward(wn_handle* h, cudaStream_t st, const float* x, int ldx
   }
   h->stack_bwd_layers = 0;
   int side_pairs = 0;
-  if (group && !sb_ok && h->use_side && h->side_stream != nullptr && h->wg_side_every > 0) {
+  if (group && !sb_ok && h->side_stream != nullptr && h->wg_side_every > 0) {
     const int pairs = tc_num_sms() / 2, tiles = B * cdiv(Tn, 256);
     if (tiles > pairs) {
       const int rounds = cdiv(tiles, pairs);
@@ -2052,7 +1996,7 @@ static int model_backward(wn_handle* h, cudaStream_t st, const float* x, int ldx
         if (sp) {
           struct Label { wn_handle* h; Label(wn_handle* h_) : h(h_) { h->cur_label = "stack_bwd"; } ~Label() { h->cur_label = "misc"; } } lab(h);
           LaunchScope ls(h, st, CLS_DILATED);
-          r = tc_stack_bwd_launch(st, *sp, bdescs[0], h->use_stack_bwd >= 2);
+          r = tc_stack_bwd_launch(st, *sp, bdescs[0]);
           if (r == 0) { stacked = true; h->stack_bwd_layers = h->L; }
           else if (r == -100) h->launches--;
           else { set_err("stack backward launch failed (%d): %s", r, tc_last_error()); return WN_ERR_CUDA; }
@@ -2114,7 +2058,7 @@ static int model_backward(wn_handle* h, cudaStream_t st, const float* x, int ldx
   };
   // (the stack-backward path has no side launches, but the same trick applies: d h0 is final behind the chain launch, and the
   // three small launches run beside the grouped weight-gradient launch instead of behind it)
-  const bool icb_side = !side_now && h->stack_bwd_layers > 0 && h->use_side && h->side_stream != nullptr && h->prof_tag == 0 && group && !h->wg_jobs.empty();
+  const bool icb_side = !side_now && h->stack_bwd_layers > 0 && h->side_stream != nullptr && h->prof_tag == 0 && group && !h->wg_jobs.empty();
   if (side_now || icb_side) {
     CK(cudaEventRecord(h->ev_blk_in[0], st));
     CK(cudaStreamWaitEvent(h->side_stream, h->ev_blk_in[0], 0));
@@ -2191,7 +2135,7 @@ static int model_backward(wn_handle* h, cudaStream_t st, const float* x, int ldx
         {
           LaunchScope ls(h, st, CLS_DILATED);
           h->wg_last_tiles = plan->ntiles; h->wg_last_partials = plan->npartial;
-          // without side launches (first call of a shape, profiling passes, WN_SIDE_STREAM=0) the side groups' units, which
+          // without side launches (first call of a shape, profiling passes, WN_TC_GROUP_SIDE_EVERY=0) the side groups' units, which
           // follow the final group's in the table, run in the same launch
           int r = tc_wgrad_group_launch(st, *plan, 0, side_now ? plan->final_units : plan->nunits);
           if (r != 0) { set_err("grouped wgrad launch failed (%d): %s", r, tc_last_error()); return WN_ERR_CUDA; }
