@@ -4,6 +4,8 @@ import numpy as np
 import pytest
 import torch
 
+from tests.util import env_vars
+
 pytestmark = pytest.mark.gpu
 
 
@@ -72,20 +74,6 @@ def test_fullsize_batch_permutation(c2):
   assert num <= 2e-3 * den, num / den
 
 
-def _with_env(env, fn):
-  import os
-  old = {k: os.environ.get(k) for k in env}
-  os.environ.update(env)
-  try:
-    return fn()
-  finally:
-    for k, v in old.items():
-      if v is None:
-        os.environ.pop(k, None)
-      else:
-        os.environ[k] = v
-
-
 def _debug_tensor(m, name, index, rows, width):
   import ctypes as C
   out = np.empty((rows, width), np.float32)
@@ -120,7 +108,7 @@ def test_fullsize_schedules_agree(c2):
   dz_a = _debug_tensor(m, 'dz', 29, rows, 512)
 
   def other(env):
-    def make():
+    with env_vars(env):
       kw = model_kwargs(dict(CONFIGS['c2']))
       m2 = WaveNet(**kw, precision='bf16', max_batch=B, max_time=T)     # the switches are read at wn_create
       m2.build(((B, T, 1), (B, 109)))
@@ -128,7 +116,6 @@ def test_fullsize_schedules_agree(c2):
       for _ in range(3):
         l2 = m2.train_step((x, c))['loss']
       return m2, l2
-    return _with_env(env, make)
 
   m_b, l_b = other({'WN_TC_STACK_BWD': '0'})
   g_b = m_b.get_grads()

@@ -6,12 +6,11 @@ is bit-equal (same forward), every gradient agrees to fp32 summation order (the 
 path is bit-reproducible across eager calls and CUDA-graph replays (no atomics).  `side_launches` has enough 256-row
 tiles (96 > 74 CTA pairs) for the side-stream launches beside the dgrad chain (reference: the filter gradients of
 `tape.gradient`, model.py:335)."""
-import os
 
 import numpy as np
 import pytest
 
-from tests.util import make_inputs
+from tests.util import env_vars, make_inputs
 
 pytestmark = pytest.mark.gpu
 
@@ -37,11 +36,8 @@ def _run(kw, B, T, group, env=None):
   from wavenets_b200 import WaveNet
   # (these tests hold the WEIGHT-GRADIENT schedules against each other on the same backward chain: the persistent
   # stack-backward launch, which replaces the chain and the side launches, is switched off unless a test asks for it)
-  env = dict({'WN_TC_STACK_BWD': '0'}, **(env or {}))
-  old = {k: os.environ.get(k) for k in ['WN_TC_GROUP_WGRAD'] + list(env)}
-  os.environ['WN_TC_GROUP_WGRAD'] = '1' if group else '0'
-  os.environ.update(env)
-  try:
+  env = dict({'WN_TC_STACK_BWD': '0', 'WN_TC_GROUP_WGRAD': '1' if group else '0'}, **(env or {}))
+  with env_vars(env):
     cond_in = 9 if kw.get('conditioning') else 0
     m = WaveNet(**kw, precision='bf16')   # the switches are read at wn_create
     x, cond = make_inputs(B, T, cond_in)
@@ -55,12 +51,6 @@ def _run(kw, B, T, group, env=None):
       out = m.train_step((x, cond) if cond is not None else x)
       outs.append((out['loss'], m.get_grads(), int(m.handle.lib.wn_stack_backward_layers(m.handle.h))))
     return outs
-  finally:
-    for k, v in old.items():
-      if v is None:
-        os.environ.pop(k, None)
-      else:
-        os.environ[k] = v
 
 
 @pytest.mark.parametrize('name', sorted(CASES))
@@ -159,21 +149,13 @@ def test_stack_backward_multi_dilation_vs_per_block_chain_and_oracle():
   x, _ = make_inputs(B, T, 0)
 
   def run(env):
-    old = {k: os.environ.get(k) for k in env}
-    os.environ.update(env)
-    try:
+    with env_vars(env):
       m = WaveNet(**kw, precision='bf16')
       m.build(x[:, :-1].shape)
       m.set_weights({k: v.astype(np.float32) for k, v in p.items()})
       for _ in range(3):
         out = m.train_step(x)
       return m, out['loss'], m.get_grads(), int(m.handle.lib.wn_stack_backward_layers(m.handle.h))
-    finally:
-      for k, v in old.items():
-        if v is None:
-          os.environ.pop(k, None)
-        else:
-          os.environ[k] = v
 
   m_a, l_a, g_a, n_a = run({})
   m_b, l_b, g_b, n_b = run({'WN_TC_STACK_BWD': '0'})

@@ -19,17 +19,15 @@ field and batch isolation around tile boundaries for the longest taps and for th
 measured errors.
 
 The 128-wide models run the stack forward, but their backward is the per-block chain: the stack backward needs the grouped
-weight-gradient mode, which needs R, D and S to be multiples of 256 (`wn_api.cu`, use_group_wgrad and sb_ok)."""
-import contextlib
+weight-gradient mode, which needs R, D and S to be multiples of 256 (`wn_api.cu`, use_group_wgrad and BwdSchedule::sb)."""
 import json
 import math
-import os
 
 import numpy as np
 import pytest
 
 from oracle import wavenet_oracle as wo
-from tests.util import oracle_config, rel_err, rel_l2
+from tests.util import env_vars, oracle_config, rel_err, rel_l2
 
 TILE = 256
 COND_IN = 109
@@ -160,20 +158,6 @@ def edge(name, T):
 
 
 # ----------------------------------------------------------------------------------------------------------- GPU
-@contextlib.contextmanager
-def _env(env):
-  old = {k: os.environ.get(k) for k in env}
-  os.environ.update(env)
-  try:
-    yield
-  finally:
-    for k, v in old.items():
-      if v is None:
-        os.environ.pop(k, None)
-      else:
-        os.environ[k] = v
-
-
 def _pairs():
   import torch
   return torch.cuda.get_device_properties(0).multi_processor_count // 2
@@ -198,7 +182,7 @@ def _setup(name):
 
 def _model(kw, p, B, T, cond, env=None):
   from wavenets_b200 import WaveNet
-  with _env(env or {}):                                    # the switches are read at wn_create
+  with env_vars(env or {}):                                    # the switches are read at wn_create
     m = WaveNet(**kw, precision='bf16', max_batch=B, max_time=T)
     m.build(((B, T, 1), (B, cond.shape[1])) if cond is not None else (B, T, 1))
   m.set_weights({k: v.astype(np.float32) for k, v in p.items()})

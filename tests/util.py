@@ -1,4 +1,7 @@
 """Shared helpers for the parity tests: one set of kwargs drives both the oracle and the product."""
+import contextlib
+import os
+
 import numpy as np
 
 from oracle import wavenet_oracle as wo
@@ -6,6 +9,21 @@ from oracle import wavenet_oracle as wo
 
 def oracle_config(kw: dict, cond_in: int = 0) -> wo.Config:
   return wo.config_from_kwargs(kw, cond_in)
+
+
+@contextlib.contextmanager
+def env_vars(env):
+  """sets the environment variables in env (the library reads its switches at wn_create), restores them on exit"""
+  old = {k: os.environ.get(k) for k in env}
+  os.environ.update(env)
+  try:
+    yield
+  finally:
+    for k, v in old.items():
+      if v is None:
+        os.environ.pop(k, None)
+      else:
+        os.environ[k] = v
 
 
 def make_inputs(B, T, cond_in=0, seed=0):

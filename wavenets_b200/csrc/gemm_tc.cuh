@@ -267,14 +267,19 @@ static inline const CUtensorMap* tc_atom_map(TmapCache& tc, const bf16* A, int l
 // Persistent kernels walk their tiles round-robin: with 256 tiles on 74 CTA pairs the last of 4 rounds keeps 34 pairs busy.
 // The same 4 rounds fit on 64 pairs; the SMs left over can run other work (the side-stream weight gradients) meanwhile.
 // g_tc_balance: 0 = always the whole GPU, 1 = the fewest CTAs (pairs) that keep the number of rounds.
-// The switch belongs to the pass a host thread is enqueuing (set and cleared around the backward chain), so it is per thread:
-// handles driven from different threads do not see each other's setting.
+// The switch belongs to the pass a host thread is enqueuing (set by a TcBalanceScope around the backward chain), so it is per
+// thread: handles driven from different threads do not see each other's setting.
 static thread_local int g_tc_balance = 0;
 static inline int tc_balanced_slots(int tiles, int slots) {
   if (!g_tc_balance || tiles <= slots) return slots;
   const int rounds = (tiles + slots - 1) / slots;
   return (tiles + rounds - 1) / rounds;
 }
+// sets the switch for one phase of a pass; every exit of the phase, an error return too, restores the whole GPU
+struct TcBalanceScope {
+  explicit TcBalanceScope(bool on) { g_tc_balance = on ? 1 : 0; }
+  ~TcBalanceScope() { g_tc_balance = 0; }
+};
 
 template <class Epi, int BN, int NEPI>
 static int tc_conv_gemm_launch(TmapCache& tc, cudaStream_t st, const TcGemmDesc& d, const typename Epi::Params& ep) {

@@ -182,7 +182,6 @@ struct wn_handle {
   float* opt_partial = nullptr; float* opt_scale = nullptr; float* opt_norms = nullptr;
   float opt_lr = 1e-3f, opt_b1 = 0.9f, opt_b2 = 0.999f, opt_eps = 1e-7f, opt_clipnorm = 0.f;
   long long opt_t = 0;
-  float* layer_xin = nullptr;             // layer API staging (fp32 in -> T)
   void* layer_in = nullptr;
   float* d_loss = nullptr;                // for the host-buffer entry point
   float* d_frames = nullptr; float* d_cond_in = nullptr;
@@ -235,12 +234,11 @@ struct wn_handle {
   void* dx_all = nullptr;     // [L][rows][R]: d x_out of block l
   void* do_all = nullptr;     // [L][rows][R]: d x_out + d skip of block l (skip_channels=None with use_skip: skip = conv1 output)
   std::vector<std::vector<void*>> dp_keep;   // [block][j]: gradient wrt the output of pre-stack conv j (B,T,D)
-  struct WgPlan { int B, T; bool drop; bool sb; int nb; TcWgGroupPlan plan; };
+  struct WgPlan { int B, T; bool drop; bool sb; int nb; TcWgGroupPlan plan; void release() { plan.release(); } };
   std::vector<WgPlan> wg_plans;
   std::vector<TcWgJobDesc> wg_jobs;   // collected by block_backward while a pass is enqueued
   int wg_last_tiles = 0, wg_last_side = 0;   // grouped tiles / side launches of the last backward pass
   int wg_last_partials = 0;                  // fp32 partial tiles (tiles x row splits) its finish launch reads
-  int wg_cur_group = -1;              // side group of the jobs block_backward appends (-1: final launch)
   int wg_side_every = 5;              // every n-th block hands its weight gradients to a side launch (WN_TC_GROUP_SIDE_EVERY, 0 = off)
   cudaEvent_t ev_wg_side = nullptr;
   int wg_force_split = 0, wg_pair_tiles = 1;   // WN_TC_GROUP_SPLIT=n / WN_TC_GROUP_NH2=0: A/B switches
@@ -269,9 +267,7 @@ struct wn_handle {
   cudaStream_t comm_stream = nullptr;
   cudaEvent_t ev_bucket[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
   cudaEvent_t ev_comm_done = nullptr;
-  int wg_cur_bucket = 0;
   int last_ar_buckets = 0;        // gradient slices the last training step all-reduced EARLY (beside the next bucket's kernels)
-  bool cond_wgrad_done = false;   // the per-bucket launches of this pass already wrote the conditioning filter gradients
 };
 
 enum { CLS_DILATED = 1, CLS_GEMM = 2, CLS_LOSS = 3, CLS_MISC = 4 };
@@ -307,6 +303,43 @@ struct OuterLabel {
   OuterLabel(wn_handle* h_, const char* l) : h(h_), prev(h_->outer_label) { h->outer_label = l; }
   ~OuterLabel() { h->outer_label = prev; }
 };
+
+// names the launches of one kernel kind (when no OuterLabel is set)
+struct LaunchLabel {
+  wn_handle* h;
+  LaunchLabel(wn_handle* h_, const char* l) : h(h_) { h->cur_label = l; }
+  ~LaunchLabel() { h->cur_label = "misc"; }
+};
+
+// captured step graphs bake in the launch sequence and the plans' tables: anything that changes either drops them
+static void drop_graphs(wn_handle* h) {
+  for (auto& g : h->graphs) if (g.exec) cudaGraphExecDestroy(g.exec);
+  h->graphs.clear();
+}
+
+// Plans of the persistent launches are built per shape on first use and kept, at most 4 of a kind.  Building allocates and
+// copies synchronously, so nothing is built while st is being captured: *out stays null then, and when the kernel does not take
+// the shape (the build returns -100).
+template <class Plan, class Build>
+static int new_plan(wn_handle* h, cudaStream_t st, std::vector<Plan>& plans, const Plan& fresh, const char* what, Build build, Plan** out) {
+  *out = nullptr;
+  cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+  cudaStreamIsCapturing(st, &cs);
+  if (cs != cudaStreamCaptureStatusNone) return WN_OK;
+  if (plans.size() >= 4) {
+    CK(cudaDeviceSynchronize());
+    drop_graphs(h);
+    for (auto& q : plans) q.release();
+    plans.clear();
+  }
+  plans.push_back(fresh);
+  const int r = build(plans.back());
+  if (r == 0) { *out = &plans.back(); return WN_OK; }
+  plans.pop_back();
+  if (r == -100) return WN_OK;
+  set_err("%s plan failed (%d): %s", what, r, tc_last_error());
+  return WN_ERR_CUDA;
+}
 
 // ============================================================================ build
 static int add_param(wn_handle* h, const std::string& name, std::initializer_list<int> shape) {
@@ -751,7 +784,7 @@ extern "C" void wn_destroy(wn_handle* h) {
   cudaDeviceSynchronize();
   if (h->comm && h->comm_owned && g_nccl.CommDestroy) g_nccl.CommDestroy(h->comm);
   for (auto& p : h->prof_events) { cudaEventDestroy(p.first); cudaEventDestroy(p.second); }
-  for (auto& g : h->graphs) if (g.exec) cudaGraphExecDestroy(g.exec);
+  drop_graphs(h);
   for (auto e : h->ev_blk_in) cudaEventDestroy(e);
   for (auto e : h->ev_blk_dz) cudaEventDestroy(e);
   for (auto e : h->ev_blk_done) cudaEventDestroy(e);
@@ -763,7 +796,7 @@ extern "C" void wn_destroy(wn_handle* h) {
   if (h->ev_in) cudaEventDestroy(h->ev_in);
   if (h->ev_out) cudaEventDestroy(h->ev_out);
   for (void* a : h->gen.allocs) cudaFree(a);
-  for (auto& wp : h->wg_plans) wp.plan.release();
+  for (auto& wp : h->wg_plans) wp.release();
   for (auto& sp : h->stack_plans) sp.release();
   for (auto& sp : h->stack_bwd_plans) sp.release();
   cudaFree(h->d_pack_jobs);
@@ -972,7 +1005,7 @@ int tc_dispatch<EpiActBwd<bf16, bf16>>(wn_handle* h, cudaStream_t st, const TcGe
 
 template <class T, class Epi>
 static int run_conv_gemm(wn_handle* h, cudaStream_t st, int cls, const GemmH& g, const typename Epi::Params& ep) {
-  struct Label { wn_handle* h; Label(wn_handle* h_, const char* l) : h(h_) { h->cur_label = l; } ~Label() { h->cur_label = "misc"; } } lab(h, Epi::kLabel);
+  LaunchLabel lab(h, Epi::kLabel);
   LaunchScope ls(h, st, cls);
   if constexpr (sizeof(T) == 4) {
     ConvGemmArgsF a;
@@ -1014,7 +1047,7 @@ static void run_colsum(wn_handle* h, cudaStream_t st, const void* G, int ldg, in
 
 template <class T>
 static int run_wgrad(wn_handle* h, cudaStream_t st, int cls, const WgradH& g) {
-  struct Label { wn_handle* h; Label(wn_handle* h_, const char* l) : h(h_) { h->cur_label = l; } ~Label() { h->cur_label = "misc"; } } lab(h, cls == CLS_DILATED ? "wgrad_dilated" : "wgrad_1x1");
+  LaunchLabel lab(h, cls == CLS_DILATED ? "wgrad_dilated" : "wgrad_1x1");
   int ktot = 0;
   for (int s = 0; s < g.nseg; ++s) ktot += g.seg[s].K;
   int nsplit = 1;
@@ -1208,7 +1241,7 @@ static int block_forward(wn_handle* h, cudaStream_t st, int l, const void* x_in,
           d.bias_r = P_(h, b.conv1.b_idx);
           int r;
           {
-            struct Label { wn_handle* h; Label(wn_handle* h_) : h(h_) { h->cur_label = "block_fwd"; } ~Label() { h->cur_label = "misc"; } } lab(h);
+            LaunchLabel lab(h, "block_fwd");
             LaunchScope ls(h, st, CLS_DILATED);
             r = c.tileN16 == 256 ? tc_block_fwd(h->tmaps, st, d) : -100;
           }
@@ -1362,23 +1395,7 @@ static int model_forward(wn_handle* h, cudaStream_t st, const float* x, int ldx,
       build_descs(descs);
       TcStackPlan* sp = nullptr;
       for (auto& q : h->stack_plans) if (q.B == B && q.T == Tn && q.cb == has_cb && q.drop == (h->drop_active && h->L > 1)) sp = &q;
-      int r = 0;
-      if (!sp) {
-        cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
-        cudaStreamIsCapturing(st, &cs);
-        if (cs == cudaStreamCaptureStatusNone) {
-          if (h->stack_plans.size() >= 4) {
-            CK(cudaDeviceSynchronize());
-            for (auto& g : h->graphs) if (g.exec) cudaGraphExecDestroy(g.exec);
-            h->graphs.clear();
-            for (auto& q : h->stack_plans) q.release();
-            h->stack_plans.clear();
-          }
-          h->stack_plans.push_back(TcStackPlan{});
-          r = tc_stack_build(h->tmaps, descs, &h->stack_plans.back());
-          if (r == 0) sp = &h->stack_plans.back(); else h->stack_plans.pop_back();
-        }
-      }
+      if (!sp) RET(new_plan(h, st, h->stack_plans, TcStackPlan{}, "stack forward", [&](TcStackPlan& p) { return tc_stack_build(h->tmaps, descs, &p); }, &sp));
       if (sp && h->drop_active) {
         // block 0's masked input from the input conv's output (every later block's comes out of the launch itself)
         LaunchScope ls(h, st, CLS_MISC);
@@ -1386,13 +1403,13 @@ static int model_forward(wn_handle* h, cudaStream_t st, const float* x, int ldx,
         dropout_apply<bf16><<<cdiv(n, 256), 256, 0, st>>>((const bf16*)h->h0, h->drop_mask, (bf16*)h->xdrop[0], n, 1.0f / (1.0f - c.dropout));
       }
       if (sp) {
-        struct Label { wn_handle* h; Label(wn_handle* h_) : h(h_) { h->cur_label = "stack_fwd"; } ~Label() { h->cur_label = "misc"; } } lab(h);
+        LaunchLabel lab(h, "stack_fwd");
         LaunchScope ls(h, st, CLS_DILATED);
-        r = tc_stack_launch(st, *sp, descs[0]);
+        const int r = tc_stack_launch(st, *sp, descs[0]);
         if (r == 0) { stacked = true; h->fused_fwd_launches = h->L; h->stack_fwd_layers = h->L; cur = h->xout[h->L - 1]; }
         else if (r == -100) h->launches--;
         else { set_err("stack forward launch failed (%d): %s", r, tc_last_error()); return WN_ERR_CUDA; }
-      } else if (r != 0 && r != -100) { set_err("stack forward plan failed (%d): %s", r, tc_last_error()); return WN_ERR_CUDA; }
+      }
     }
   }
   if (!stacked)
@@ -1501,16 +1518,46 @@ struct BwdSide {
   cudaEvent_t wait_dx;   // MAIN waits before writing dx_in   (side work of block l+1 read that buffer), may be null
 };
 
+// how block_backward runs one block of a backward pass (the default: alone, on one stream)
+struct BlockBwdMode {
+  void* dz = nullptr;                // gate-adjoint output (null: h->dz)
+  const BwdSide* side = nullptr;     // two-stream schedule: the block's events
+  // the weight gradients of conv1, conv_skip and the dilated stack are not launched here; their operands stay in per-block
+  // buffers and the problems are appended to h->wg_jobs for the grouped launch (gemm_tc_wgroup.cuh)
+  bool grouped = false;
+  // the gate adjoint and the dgrad of this block run inside the persistent stack-backward launch (gemm_tc_stack_bwd.cuh):
+  // only the weight-gradient problems are collected here
+  bool in_stack = false;
+  int side_group = -1, bucket = 0;   // grouped: side launch (-1: the final launch) and all-reduce bucket of the problems
+};
+
+// grouped weight-gradient problem of conv cv: dW = A^T G over its taps (tap k reads A shifted by -(K-1-k)*dil), the bias
+// gradient from the column sums of G, the L2 term when the model has one
+static TcWgJobDesc wg_job(wn_handle* h, const ConvP& cv, const void* A, int lda, const void* G, int ldg, int group, int bucket) {
+  TcWgJobDesc j{};
+  j.A = (const bf16*)A; j.lda = lda; j.cin = cv.cin; j.ntaps = cv.K;
+  for (int k = 0; k < cv.K; ++k) j.shift[k] = -(cv.K - 1 - k) * cv.dil;
+  j.G = (const bf16*)G; j.ldg = ldg; j.N = cv.cout;
+  j.dst = G_(h, cv.w_idx); j.w = h->cfg.l2_reg_factor > 0.f ? P_(h, cv.w_idx) : nullptr; j.bias = G_(h, cv.b_idx);
+  j.group = group; j.bucket = bucket;
+  return j;
+}
+// the same product as one per-block launch (run_wgrad)
+static WgradH wgrad_of(wn_handle* h, const ConvP& cv, const void* A, int lda, const void* G, int ldg, int B, int Tn, float l2coef) {
+  WgradH w{};
+  w.B = B; w.T = Tn; w.N = cv.cout; w.G = G; w.ldg = ldg; w.nseg = cv.K;
+  for (int k = 0; k < cv.K; ++k) w.seg[k] = SegH{A, lda, -(cv.K - 1 - k) * cv.dil, cv.cin};
+  w.dst = G_(h, cv.w_idx); w.w = P_(h, cv.w_idx); w.l2coef = l2coef; w.bias_dst = G_(h, cv.b_idx);
+  return w;
+}
+
 template <class T>
 static int block_backward(wn_handle* h, cudaStream_t st, int l, const void* x_in, const void* dxout, int ldxo, const void* dskip, int ldsk,
-                          void* dx_in, int ldxi, int B, int Tn, float l2coef, void* dzbuf = nullptr, const BwdSide* sd = nullptr,
-                          bool group = false, bool skip_chain = false) {
-  // skip_chain: the gate adjoint and the dgrad of this block run inside the persistent stack-backward launch
-  // (gemm_tc_stack_bwd.cuh): only the weight-gradient problems are collected here
-  // group: the weight gradients of conv1, conv_skip and the gated conv are not launched here; their operands stay in
-  // per-block buffers and the problems are appended to h->wg_jobs for the grouped launch (gemm_tc_wgroup.cuh)
+                          void* dx_in, int ldxi, int B, int Tn, float l2coef, const BlockBwdMode& m) {
   BlockP& b = h->blocks[l];
-  if (!dzbuf) dzbuf = h->dz;
+  void* const dzbuf = m.dz ? m.dz : h->dz;
+  const BwdSide* const sd = m.side;
+  const bool group = m.grouped, skip_chain = m.in_stack;
   const int depth = (int)b.stack.size();
   const size_t rows_cap = (size_t)h->maxB * h->maxT;
   const long long nR = (long long)B * Tn * h->R;
@@ -1544,13 +1591,8 @@ static int block_backward(wn_handle* h, cudaStream_t st, int l, const void* x_in
   if (side1) CK(cudaStreamWaitEvent(sd->side, sd->ev_in, 0));
   if (group) {
     if constexpr (sizeof(T) == 2) {
-      const bool l2 = h->cfg.l2_reg_factor > 0.f;
       if (d_o) {
-        TcWgJobDesc j{};
-        j.A = (const bf16*)g_l; j.lda = D; j.cin = D; j.ntaps = 1; j.shift[0] = 0;
-        j.G = (const bf16*)d_o; j.ldg = ld_o; j.N = R;
-        j.dst = G_(h, b.conv1.w_idx); j.w = l2 ? P_(h, b.conv1.w_idx) : nullptr; j.bias = G_(h, b.conv1.b_idx);
-        j.group = h->wg_cur_group; j.bucket = h->wg_cur_bucket;
+        TcWgJobDesc j = wg_job(h, b.conv1, g_l, D, d_o, ld_o, m.side_group, m.bucket);
         if (alias_split) j.bias_add_G = (const bf16*)dskip;
         h->wg_jobs.push_back(j);
         if (alias_split) {
@@ -1563,12 +1605,7 @@ static int block_backward(wn_handle* h, cudaStream_t st, int l, const void* x_in
       }
       if (b.has_skip) {
         if (dskip) {
-          TcWgJobDesc j{};
-          j.A = (const bf16*)g_l; j.lda = D; j.cin = D; j.ntaps = 1; j.shift[0] = 0;
-          j.G = (const bf16*)dskip; j.ldg = ldsk; j.N = S;
-          j.dst = G_(h, b.conv_skip.w_idx); j.w = l2 ? P_(h, b.conv_skip.w_idx) : nullptr; j.bias = G_(h, b.conv_skip.b_idx);
-          j.group = h->wg_cur_group; j.bucket = h->wg_cur_bucket;
-          h->wg_jobs.push_back(j);
+          h->wg_jobs.push_back(wg_job(h, b.conv_skip, g_l, D, dskip, ldsk, m.side_group, m.bucket));
         } else {
           unused_conv_grads(h, st, b.conv_skip.w_idx, b.conv_skip.b_idx, l2coef);
         }
@@ -1583,10 +1620,7 @@ static int block_backward(wn_handle* h, cudaStream_t st, int l, const void* x_in
     w.l2_a = TC_L2_FIRST;   // last use of g_l
     RET(run_wgrad<T>(h, s1, CLS_GEMM, w));
   } else if (d_o) {
-    WgradH w{};
-    w.B = B; w.T = Tn; w.N = R; w.G = d_o; w.ldg = ld_o; w.nseg = 1; w.seg[0] = SegH{g_l, D, 0, D};
-    w.dst = G_(h, b.conv1.w_idx); w.w = P_(h, b.conv1.w_idx); w.l2coef = l2coef;
-    w.bias_dst = G_(h, b.conv1.b_idx);
+    WgradH w = wgrad_of(h, b.conv1, g_l, D, d_o, ld_o, B, Tn, l2coef);
     w.side = side1;
     RET(run_wgrad<T>(h, s1, CLS_GEMM, w));
   } else {
@@ -1594,10 +1628,7 @@ static int block_backward(wn_handle* h, cudaStream_t st, int l, const void* x_in
   }
   if (b.has_skip && !cat && !group) {
     if (dskip) {
-      WgradH w{};
-      w.B = B; w.T = Tn; w.N = S; w.G = dskip; w.ldg = ldsk; w.nseg = 1; w.seg[0] = SegH{g_l, D, 0, D};
-      w.dst = G_(h, b.conv_skip.w_idx); w.w = P_(h, b.conv_skip.w_idx); w.l2coef = l2coef;
-      w.bias_dst = G_(h, b.conv_skip.b_idx);
+      WgradH w = wgrad_of(h, b.conv_skip, g_l, D, dskip, ldsk, B, Tn, l2coef);
       w.side = side1;
       RET(run_wgrad<T>(h, s1, CLS_GEMM, w));
     } else {
@@ -1643,22 +1674,13 @@ static int block_backward(wn_handle* h, cudaStream_t st, int l, const void* x_in
     // conditioning per-batch sums for the gated conv) are the column sums of the same G
     if (group) {
       if constexpr (sizeof(T) == 2) {
-        TcWgJobDesc jd{};
-        jd.A = (const bf16*)a_in; jd.lda = a_w; jd.cin = c.cin; jd.ntaps = c.K;
-        for (int k = 0; k < c.K; ++k) jd.shift[k] = -(c.K - 1 - k) * c.dil;
-        jd.G = (const bf16*)dcur; jd.ldg = dcw; jd.N = c.cout;
-        jd.dst = G_(h, c.w_idx); jd.w = h->cfg.l2_reg_factor > 0.f ? P_(h, c.w_idx) : nullptr; jd.bias = G_(h, c.b_idx);
+        TcWgJobDesc jd = wg_job(h, c, a_in, a_w, dcur, dcw, m.side_group, m.bucket);
         if (j == depth - 1 && b.has_cond) { jd.per_batch = h->dcb + (size_t)l * h->maxB * 2 * D; jd.ldpb = 2 * D; }
-        jd.group = h->wg_cur_group; jd.bucket = h->wg_cur_bucket;
         h->wg_jobs.push_back(jd);
       }
     } else {
-      WgradH w{};
-      w.bias_dst = G_(h, c.b_idx);
+      WgradH w = wgrad_of(h, c, a_in, a_w, dcur, dcw, B, Tn, l2coef);
       if (j == depth - 1 && b.has_cond && !h->cond_seq) { w.per_batch = h->dcb + (size_t)l * h->maxB * 2 * D; w.ldpb = 2 * D; }
-      w.B = B; w.T = Tn; w.N = c.cout; w.G = dcur; w.ldg = dcw; w.nseg = c.K;
-      for (int k = 0; k < c.K; ++k) w.seg[k] = SegH{a_in, a_w, -(c.K - 1 - k) * c.dil, c.cin};
-      w.dst = G_(h, c.w_idx); w.w = P_(h, c.w_idx); w.l2coef = l2coef;
       // the gated conv's wgrad reads dz and forward activations only: side stream
       const bool side2 = sd != nullptr && j == depth - 1;
       if (side2) CK(cudaStreamWaitEvent(sd->side, sd->ev_dz, 0));
@@ -1789,72 +1811,88 @@ static const BwdSide* side_setup(wn_handle* h, cudaStream_t st, int l, bool on, 
   return sd;
 }
 
+// ============================================================================ backward pass
+// The schedule of a backward pass, decided once per pass from the handle and the shape:
+//   fp32 tier                          per-block chain on one stream
+//   bf16, not grouped                  per-block chain, weight gradients on the side stream (use_side); with a separate skip,
+//                                      d x_out and d skip side by side in ping-pong buffers (cat)
+//   bf16, grouped (R, D, S multiples   per-block chain, every block's weight gradients in one grouped launch behind it; those of
+//   of 256)                            every n-th block in side launches beside the chain (side_pairs)
+//   bf16, grouped, stack backward (sb) the chain as one persistent launch, then the grouped launch, bucket by bucket (nb) when the
+//                                      step all-reduces its gradients
+struct BwdSchedule {
+  bool group = false;      // grouped weight gradients (gemm_tc_wgroup.cuh)
+  bool use_side = false;   // per-block weight gradients on the side stream
+  bool cat = false;        // [d x_out | d skip] ping-pong buffers
+  bool sb = false;         // stack backward (gemm_tc_stack_bwd.cuh)
+  int side_pairs = 0;      // CTA pairs the chain leaves to the side launches (0: none)
+  int nb = 1;              // all-reduce buckets of the grouped launch
+  TcWgGroupPlan* wplan = nullptr;   // grouped plan of this shape, once built
+  bool side_now = false;   // the side launches run in this pass
+  // side launch that takes the weight gradients of block l (-1: the final grouped launch)
+  int side_group(const wn_handle* h, int l) const {
+    return (side_pairs > 0 && (h->L - 1 - l) % h->wg_side_every == 0) ? (h->L - 1 - l) / h->wg_side_every : -1;
+  }
+  // two buckets: the first (last blocks, reduced beside the second bucket's kernels) takes ar_first_pct of the blocks — what stays
+  // exposed behind the pass is the second bucket's slice, so it is the smaller one; more buckets: equal groups
+  int bucket(const wn_handle* h, int l) const {
+    if (nb <= 1) return 0;
+    if (nb == 2) return (h->L - 1 - l) * 100 < h->L * h->ar_first_pct ? 0 : 1;
+    return ((h->L - 1 - l) * nb) / h->L;
+  }
+};
+
 template <class T>
-static int model_backward(wn_handle* h, cudaStream_t st, const float* x, int ldx, const float* cond_in, int B, int Tn, float l2coef) {
-  const wn_config& c = h->cfg;
+static BwdSchedule bwd_schedule(wn_handle* h, int B, int Tn) {
+  BwdSchedule s;
   // (bf16 tier only: the fp32 tier's wgrad / column-sum scratch buffers are not duplicated for a second stream)
-  const bool group = sizeof(T) == 2 && h->use_group_wgrad;
-  const bool use_side = sizeof(T) == 2 && h->prof_tag == 0 && h->side_stream != nullptr && !group;
-  const bool cat = sizeof(T) == 2 && h->dcatA != nullptr;
-  const int ldc = h->R + h->S;
-  const size_t rows_cap = (size_t)h->maxB * h->maxT;
-  auto dz_of = [&](int l) -> void* { return (T*)h->dz_all + (size_t)l * rows_cap * 2 * h->D; };
-  auto dx_of = [&](int l) -> void* { return (T*)h->dx_all + (size_t)l * rows_cap * h->R; };
-  h->wg_jobs.clear();
-  h->wg_last_tiles = 0; h->wg_last_side = 0;
+  if constexpr (sizeof(T) == 2) {
+    s.group = h->use_group_wgrad != 0;
+    s.use_side = h->prof_tag == 0 && h->side_stream != nullptr && !s.group;
+    s.cat = h->dcatA != nullptr;
+    // Backward chain as ONE persistent launch (gemm_tc_stack_bwd.cuh): D = R = 256, d z / d x_out
+    // of every block kept (grouped weight gradients), more 256-row tiles per layer than CTA pairs.  It takes every SM for the
+    // whole chain, so the weight gradients all run in the one grouped launch behind it (no side launches).
+    s.sb = s.group && !s.cat && h->use_stack_bwd && h->L >= 2 && h->D == h->R && h->D == 256 &&
+           h->K <= TC_MAX_TAPS && B * cdiv(Tn, 256) > tc_num_sms() / 2;
+    for (auto& b : h->blocks) {
+      if (!s.sb) break;
+      // multi-dilation blocks (plain conv layers of the launch): all convs 256 wide
+      s.sb = b.stack[0].cin % 64 == 0 && (!b.has_skip || h->S % 64 == 0) && b.stack.size() <= 16 &&
+             (b.stack.size() == 1 || (h->D == 256 && h->dp_keep.size() == (size_t)h->L));
+      for (size_t j = 0; s.sb && j + 1 < b.stack.size(); ++j) s.sb = b.stack[j].cout == h->D && b.stack[j].Wb16 != nullptr && b.stack[j].K == h->K;
+    }
+  }
   // Side launches: the persistent chain kernels need ceil(tiles / pairs) rounds; the same rounds fit on fewer CTA pairs
   // (256 tiles: 4 rounds on 74 or on 64 pairs), and the pairs left over run the weight gradients of every n-th block
   // beside the chain.  The plan (unit ranges per side group) exists from the second call on; the first call launches
   // every group at the end.
-  // Backward chain as ONE persistent launch (gemm_tc_stack_bwd.cuh): D = R = 256, d z / d x_out
-  // of every block kept (grouped weight gradients), more 256-row tiles per layer than CTA pairs.  It takes every SM for the
-  // whole chain, so the weight gradients all run in the one grouped launch behind it (no side launches).
-  bool sb_ok = false;
-  if constexpr (sizeof(T) == 2) {
-    sb_ok = group && !cat && h->use_stack_bwd && h->L >= 2 && h->D == h->R && h->D == 256 &&
-            h->K <= TC_MAX_TAPS && B * cdiv(Tn, 256) > tc_num_sms() / 2;
-    for (auto& b : h->blocks) {
-      if (!sb_ok) break;
-      // multi-dilation blocks (plain conv layers of the launch): all convs 256 wide
-      sb_ok = b.stack[0].cin % 64 == 0 && (!b.has_skip || h->S % 64 == 0) && b.stack.size() <= 16 &&
-              (b.stack.size() == 1 || (h->D == 256 && h->dp_keep.size() == (size_t)h->L));
-      for (size_t j = 0; sb_ok && j + 1 < b.stack.size(); ++j) sb_ok = b.stack[j].cout == h->D && b.stack[j].Wb16 != nullptr && b.stack[j].K == h->K;
-    }
-  }
-  h->stack_bwd_layers = 0;
-  int side_pairs = 0;
-  if (group && !sb_ok && h->side_stream != nullptr && h->wg_side_every > 0) {
+  if (s.group && !s.sb && h->side_stream != nullptr && h->wg_side_every > 0) {
     const int pairs = tc_num_sms() / 2, tiles = B * cdiv(Tn, 256);
     if (tiles > pairs) {
       const int rounds = cdiv(tiles, pairs);
-      side_pairs = pairs - cdiv(tiles, rounds);
+      s.side_pairs = pairs - cdiv(tiles, rounds);
     }
-    if (side_pairs < 6) side_pairs = 0;
+    if (s.side_pairs < 6) s.side_pairs = 0;
   }
-  auto side_group_of = [&](int l) -> int { return (side_pairs > 0 && (h->L - 1 - l) % h->wg_side_every == 0) ? (h->L - 1 - l) / h->wg_side_every : -1; };
   // bucketed all-reduce: only with the stack-backward launch (every SM busy until the chain ends, all filter gradients in the
   // final grouped launch) and a communicator that reduces inside this step
-  const int nb = (group && sb_ok && h->ar_now && h->prof_tag == 0 && h->comm_stream != nullptr) ? std::min(std::min(h->ar_buckets, h->L), 8) : 1;
-  // two buckets: the first (last blocks, reduced beside the second bucket's kernels) takes ar_first_pct of the blocks — what stays
-  // exposed behind the pass is the second bucket's slice, so it is the smaller one; more buckets: equal groups
-  auto bucket_of = [&](int l) -> int {
-    if (nb <= 1) return 0;
-    if (nb == 2) return (h->L - 1 - l) * 100 < h->L * h->ar_first_pct ? 0 : 1;
-    return ((h->L - 1 - l) * nb) / h->L;
-  };
-  auto block_off = [&](int l) -> long long {
-    if (l < h->L) return h->params[h->blocks[l].stack[0].w_idx].offset;
-    if (!h->head.empty()) return h->params[h->head[0].w_idx].offset;
-    if (!h->map_w.empty()) return h->params[h->map_w[0]].offset;
-    return h->n_scalars;
-  };
-  h->ar_early_lo = h->ar_early_hi = -1;
-  h->last_ar_buckets = 0;
-  TcWgGroupPlan* wplan = nullptr;
-  if (group) for (auto& wp : h->wg_plans) if (wp.B == B && wp.T == Tn && wp.drop == h->drop_active && wp.sb == sb_ok && wp.nb == nb) wplan = &wp.plan;
-  const bool side_now = wplan != nullptr && side_pairs > 0 && h->prof_tag == 0 && !wplan->side.empty();
-  g_tc_balance = side_now ? 1 : 0;
-  // ---- head
+  s.nb = (s.group && s.sb && h->ar_now && h->prof_tag == 0 && h->comm_stream != nullptr) ? std::min(std::min(h->ar_buckets, h->L), 8) : 1;
+  if (s.group) for (auto& wp : h->wg_plans) if (wp.B == B && wp.T == Tn && wp.drop == h->drop_active && wp.sb == s.sb && wp.nb == s.nb) s.wplan = &wp.plan;
+  s.side_now = s.wplan != nullptr && s.side_pairs > 0 && h->prof_tag == 0 && !s.wplan->side.empty();
+  return s;
+}
+
+// grouped weight gradients keep d z and d x_out of every block: block l's slab of dz_all / dx_all
+template <class T>
+static void* dz_slab(wn_handle* h, int l) { return (T*)h->dz_all + (size_t)l * h->maxB * h->maxT * 2 * h->D; }
+template <class T>
+static void* dx_slab(wn_handle* h, int l) { return (T*)h->dx_all + (size_t)l * h->maxB * h->maxT * h->R; }
+
+// ---- head, last conv first: its input gradient lands where the chain reads d x_out or d skip
+template <class T>
+static int head_backward(wn_handle* h, cudaStream_t st, const BwdSchedule& s, int B, int Tn, float l2coef) {
+  const wn_config& c = h->cfg;
   const void* dcur = h->dlogits;
   int dw = h->ldd;
   for (int i = (int)h->head.size() - 1; i >= 0; --i) {
@@ -1868,23 +1906,12 @@ static int model_backward(wn_handle* h, cudaStream_t st, const float* x, int ldx
     // (the head's d-activation buffers dlogits / dhA / dhB stay intact until the end of the pass when the head has <= 3 convs)
     bool head_grouped = false;
     if constexpr (sizeof(T) == 2) {
-      if (group && h->head.size() <= 3 && tc_wgrad_group_ok(hc.cin, hc.cout) && a_w == hc.cin) {
-        TcWgJobDesc j{};
-        j.A = (const bf16*)a_in; j.lda = a_w; j.cin = hc.cin; j.ntaps = 1; j.shift[0] = 0;
-        j.G = (const bf16*)dcur; j.ldg = dw; j.N = hc.cout;
-        j.dst = G_(h, hc.w_idx); j.w = c.l2_reg_factor > 0.f ? P_(h, hc.w_idx) : nullptr; j.bias = G_(h, hc.b_idx);
-        j.group = -1; j.bucket = nb - 1;      // (the head's gradients travel with the last bucket)
-        h->wg_jobs.push_back(j);
+      if (s.group && h->head.size() <= 3 && tc_wgrad_group_ok(hc.cin, hc.cout) && a_w == hc.cin) {
+        h->wg_jobs.push_back(wg_job(h, hc, a_in, a_w, dcur, dw, -1, s.nb - 1));      // (the head's gradients travel with the last bucket)
         head_grouped = true;
       }
     }
-    if (!head_grouped) {
-      WgradH w{};
-      w.bias_dst = G_(h, hc.b_idx);
-      w.B = B; w.T = Tn; w.N = hc.cout; w.G = dcur; w.ldg = dw; w.nseg = 1; w.seg[0] = SegH{a_in, a_w, 0, hc.cin};
-      w.dst = G_(h, hc.w_idx); w.w = P_(h, hc.w_idx); w.l2coef = l2coef;
-      RET(run_wgrad<T>(h, st, CLS_GEMM, w));
-    }
+    if (!head_grouped) RET(run_wgrad<T>(h, st, CLS_GEMM, wgrad_of(h, hc, a_in, a_w, dcur, dw, B, Tn, l2coef)));
     GemmH g;
     g.B = B; g.T = Tn; g.N = hc.cin; g.nseg = 1;
     g.seg[0] = SegH{dcur, dw, 0, (sizeof(T) == 2 && i + 1 == (int)h->head.size()) ? h->ldd : hc.cout};
@@ -1895,265 +1922,281 @@ static int model_backward(wn_handle* h, cudaStream_t st, const float* x, int ldx
     if (i > 0) {
       dst = (dcur == h->dhA) ? h->dhB : h->dhA;
       ep.out = (T*)dst; ep.ldo = hc.cin; ep.y = (const T*)h->hact[i - 1]; ep.ldy = hc.cin; ep.act = c.activation; ep.vec = vec_ok<T>(hc.cin);
-    } else if (cat) {
+    } else if (s.cat) {
+      const int ldc = h->R + h->S;
       dst = (T*)h->dcatA + h->R;
       ep.out = (T*)dst; ep.ldo = ldc; ep.y = nullptr; ep.act = ACT_LINEAR; ep.vec = vec_ok<T>(ldc);
     } else {
-      dst = c.use_skip ? h->dskip : (group ? dx_of(h->L - 1) : h->dxA);
+      dst = c.use_skip ? h->dskip : (s.group ? dx_slab<T>(h, h->L - 1) : h->dxA);
       ep.out = (T*)dst; ep.ldo = hc.cin; ep.y = nullptr; ep.act = ACT_LINEAR; ep.vec = vec_ok<T>(hc.cin);
     }
     RET((run_conv_gemm<T, EpiActBwd<T, T>>(h, st, CLS_GEMM, g, ep)));
     dcur = dst;
     dw = hc.cin;
   }
-  // ---- blocks
-  const void* dxout;
-  int ld_dx;
-  if (cat) {
-    // d skip is the same for every block (model.py:236): keep a copy beside each d x_out ping-pong buffer
-    CK(cudaMemcpy2DAsync((T*)h->dcatB + h->R, (size_t)ldc * sizeof(T), (const T*)h->dcatA + h->R, (size_t)ldc * sizeof(T), (size_t)h->S * sizeof(T),
-                         (size_t)B * Tn, cudaMemcpyDeviceToDevice, st));
-    const void* cur = nullptr;          // buffer holding d x_out of the block being processed
-    void* nxt = h->dcatB;
-    for (int l = h->L - 1; l >= 0; --l) {
-      const void* x_in = l > 0 ? h->xout[l - 1] : h->h0;
-      const void* dsk = cur ? (const void*)((const T*)cur + h->R) : (const void*)((const T*)h->dcatA + h->R);
-      BwdSide sd; const BwdSide* sdp = side_setup(h, st, l, use_side, &sd);
-      RET(block_backward<T>(h, st, l, x_in, cur, ldc, dsk, ldc, nxt, ldc, B, Tn, l2coef, (l & 1) ? h->dz2 : h->dz, sdp));
-      cur = nxt;
-      nxt = (nxt == h->dcatB) ? h->dcatA : h->dcatB;
-    }
-    dxout = cur; ld_dx = ldc;
-  } else {
-    const void* dskip = c.use_skip ? h->dskip : nullptr;
-    dxout = c.use_skip ? nullptr : (group ? dx_of(h->L - 1) : h->dxA);
-    bool stacked = false;
-    if constexpr (sizeof(T) == 2) {
-      if (sb_ok) {
-        // one desc per CONV in forward order: the plain convs of block l, then its gated conv
-        std::vector<TcStackBwdDesc> bdescs;
-        {
-          int conv_index = 0;
-          for (int l = 0; l < h->L; ++l) {
-            BlockP& b = h->blocks[l];
-            const int depth = (int)b.stack.size();
-            const bf16* blk_dxo = l == h->L - 1 ? (const bf16*)dxout : (const bf16*)dx_of(l);      // d x_out of this block (or null)
-            bf16* blk_dx = (bf16*)(l > 0 ? dx_of(l - 1) : h->dxA);                                   // gradient wrt the block input
-            const int next_first = conv_index + depth;      // desc that writes blk_dxo (first conv of block l + 1), if any
-            const bool dxo_in_launch = blk_dxo != nullptr && l < h->L - 1;
-            for (int j = 0; j < depth; ++j, ++conv_index) {
-              const ConvP& cv = b.stack[j];
-              TcStackBwdDesc d{};
-              const bool alias = h->alias_skip && dskip != nullptr;      // skip = conv1's output: d skip joins d x_out in front of Wr^T
-              d.B = B; d.T = Tn; d.nseg = cv.K; d.D = h->D; d.R = h->R; d.S = dskip ? (alias ? h->R : h->S) : 0;
-              for (int k = 0; k < cv.K; ++k) d.shift[k] = (cv.K - 1 - k) * cv.dil;
-              d.Wb = cv.Wb16; d.k_b = rup(cv.Kb16, 64);
-              d.drop_scale = h->drop_active ? 1.0f / (1.0f - c.dropout) : 0.f;
-              d.ein_layer = -1;
-              // what this conv's tile writes: the gradient wrt its input
-              d.dx = j == 0 ? blk_dx : (bf16*)h->dp_keep[l][j - 1];
-              if (j == 0) {
-                // first conv of the block: the block input is not activated; the residual gradient joins here
-                if (c.use_residual && blk_dxo) { d.out_mode = 1; d.ein = blk_dxo; d.ein_layer = dxo_in_launch ? next_first : -1; }
-                if (h->drop_active) d.mask = h->drop_mask + (size_t)l * rows_cap * h->R;
-              } else {
-                d.out_mode = 2; d.act = c.activation; d.ein = (const bf16*)h->acts[l][j - 1];
-              }
-              if (j < depth - 1) {
-                d.plain = 1; d.gin = (const bf16*)h->dp_keep[l][j];
-              } else {
-                d.dxo = blk_dxo;
-                d.dskip = ((b.has_skip || alias) && dskip) ? (const bf16*)dskip : nullptr; d.lds = h->Sp;
-                d.alias = alias ? 1 : 0;
-                d.z = (const bf16*)h->zbuf[l]; d.dz = (bf16*)dz_of(l);
-                const int rs = h->R + (b.has_skip ? h->S : 0), koff = (d.dxo || alias) ? 0 : h->R;
-                d.Wdg = b.Wdg16 + koff; d.k_dg = rup(rs, 64);
-                d.has_res = (c.use_residual && depth == 1) ? 1 : 0;
-              }
-              bdescs.push_back(d);
-            }
-          }
-        }
-        TcStackBwdPlan* sp = nullptr;
-        for (auto& q : h->stack_bwd_plans) if (q.B == B && q.T == Tn && q.drop == h->drop_active) sp = &q;
-        int r = 0;
-        if (!sp) {
-          cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
-          cudaStreamIsCapturing(st, &cs);
-          if (cs == cudaStreamCaptureStatusNone) {
-            if (h->stack_bwd_plans.size() >= 4) {
-              CK(cudaDeviceSynchronize());
-              for (auto& g : h->graphs) if (g.exec) cudaGraphExecDestroy(g.exec);
-              h->graphs.clear();
-              for (auto& q : h->stack_bwd_plans) q.release();
-              h->stack_bwd_plans.clear();
-            }
-            h->stack_bwd_plans.push_back(TcStackBwdPlan{});
-            r = tc_stack_bwd_build(h->tmaps, bdescs, &h->stack_bwd_plans.back());
-            if (r == 0) sp = &h->stack_bwd_plans.back(); else h->stack_bwd_plans.pop_back();
-          }
-        }
-        if (sp) {
-          struct Label { wn_handle* h; Label(wn_handle* h_) : h(h_) { h->cur_label = "stack_bwd"; } ~Label() { h->cur_label = "misc"; } } lab(h);
-          LaunchScope ls(h, st, CLS_DILATED);
-          r = tc_stack_bwd_launch(st, *sp, bdescs[0]);
-          if (r == 0) { stacked = true; h->stack_bwd_layers = h->L; }
-          else if (r == -100) h->launches--;
-          else { set_err("stack backward launch failed (%d): %s", r, tc_last_error()); return WN_ERR_CUDA; }
-        } else if (r != 0 && r != -100) { set_err("stack backward plan failed (%d): %s", r, tc_last_error()); return WN_ERR_CUDA; }
-      }
-    }
-    for (int l = h->L - 1; l >= 0; --l) {
-      const void* x_in = l > 0 ? h->xout[l - 1] : h->h0;
-      // grouped weight gradients: d x_out and d z of every block keep their own buffers until the grouped launch below
-      void* dx_in = group ? (l > 0 ? dx_of(l - 1) : h->dxA) : ((dxout == h->dxA) ? h->dxB : h->dxA);
-      BwdSide sd; const BwdSide* sdp = side_setup(h, st, l, use_side, &sd);
-      h->wg_cur_group = side_group_of(l);
-      h->wg_cur_bucket = bucket_of(l);
-      RET(block_backward<T>(h, st, l, x_in, dxout, h->R, dskip, h->Sp, dx_in, h->R, B, Tn, l2coef, group ? dz_of(l) : ((l & 1) ? h->dz2 : h->dz), sdp,
-                            group, stacked));
-      if constexpr (sizeof(T) == 2) {
-        if (side_now && h->wg_cur_group >= 0 && h->wg_cur_group < (int)wplan->side.size() && wplan->side[h->wg_cur_group].second > 0) {
-          // d z_l and d x_out_l are complete behind this block's kernels: its weight gradients start on the side stream
-          CK(cudaEventRecord(h->ev_blk_dz[l], st));
-          CK(cudaStreamWaitEvent(h->side_stream, h->ev_blk_dz[l], 0));
-          struct Label { wn_handle* h; Label(wn_handle* h_, const char* lb) : h(h_) { h->cur_label = lb; } ~Label() { h->cur_label = "misc"; } } lab(h, "wgrad_group");
-          LaunchScope ls(h, h->side_stream, CLS_DILATED);
-          int r = tc_wgrad_group_launch(h->side_stream, *wplan, wplan->side[h->wg_cur_group].first, wplan->side[h->wg_cur_group].second);
-          if (r != 0) { set_err("grouped wgrad side launch failed (%d): %s", r, tc_last_error()); return WN_ERR_CUDA; }
-          h->wg_last_side++;
-        }
-      }
-      dxout = dx_in;
-    }
-    h->wg_cur_group = -1; h->wg_cur_bucket = 0;
-    ld_dx = h->R;
+  return WN_OK;
+}
+
+// ---- per-block chain on [d x_out | d skip] ping-pong buffers (row width R + S); *dxout: d x_out of block 0
+template <class T>
+static int cat_chain(wn_handle* h, cudaStream_t st, const BwdSchedule& s, int B, int Tn, float l2coef, const void** dxout) {
+  const int ldc = h->R + h->S;
+  // d skip is the same for every block (model.py:236): keep a copy beside each d x_out ping-pong buffer
+  CK(cudaMemcpy2DAsync((T*)h->dcatB + h->R, (size_t)ldc * sizeof(T), (const T*)h->dcatA + h->R, (size_t)ldc * sizeof(T), (size_t)h->S * sizeof(T),
+                       (size_t)B * Tn, cudaMemcpyDeviceToDevice, st));
+  const void* cur = nullptr;          // buffer holding d x_out of the block being processed
+  void* nxt = h->dcatB;
+  for (int l = h->L - 1; l >= 0; --l) {
+    const void* x_in = l > 0 ? h->xout[l - 1] : h->h0;
+    const void* dsk = cur ? (const void*)((const T*)cur + h->R) : (const void*)((const T*)h->dcatA + h->R);
+    BwdSide sd;
+    BlockBwdMode m;
+    m.side = side_setup(h, st, l, s.use_side, &sd);
+    m.dz = (l & 1) ? h->dz2 : h->dz;
+    RET(block_backward<T>(h, st, l, x_in, cur, ldc, dsk, ldc, nxt, ldc, B, Tn, l2coef, m));
+    cur = nxt;
+    nxt = (nxt == h->dcatB) ? h->dcatA : h->dcatB;
   }
-  g_tc_balance = 0;
-  // ---- input conv (model.py:84-88): dW[k][c], db[c].  HBM-bound, small CTAs: with side launches it runs on the side stream
-  // beside the final grouped weight-gradient launch (its CTAs fit next to the tensor kernel's on the same SMs)
-  bool input_conv_done = false;
-  auto input_conv_bwd = [&](cudaStream_t s_) {
-    OuterLabel ol(h, "input_conv_bwd");
-    const bool wide = h->R % 2 == 0 && h->R / 2 <= 256 && ld_dx % 2 == 0;
-    const int chunks = cdiv(Tn, 64);
-    const int nparts = wide ? cdiv((long long)B * Tn, ICB_ROWS) : B * chunks;
-    {
-      LaunchScope ls(h, s_, CLS_MISC);
-      if (wide)
-        input_conv_bwd_stage1_wide<T><<<nparts, 256, 0, s_>>>(x, ldx, (const T*)dxout, ld_dx, h->colpart, B, Tn, h->R, h->K);
-      else
-        input_conv_bwd_stage1<T><<<dim3(cdiv(h->R, 64), chunks, B), 64, 0, s_>>>(x, ldx, (const T*)dxout, ld_dx, h->colpart, B, Tn, h->R, h->K, 64);
+  *dxout = cur;
+  return WN_OK;
+}
+
+// ---- gate adjoint and dgrads of every block as one persistent launch; *stacked: it ran (else the per-block chain runs them)
+static int stack_backward(wn_handle* h, cudaStream_t st, int B, int Tn, const void* dxout, const void* dskip, bool* stacked) {
+  const wn_config& c = h->cfg;
+  const size_t rows_cap = (size_t)h->maxB * h->maxT;
+  // one desc per CONV in forward order: the plain convs of block l, then its gated conv
+  std::vector<TcStackBwdDesc> bdescs;
+  int conv_index = 0;
+  for (int l = 0; l < h->L; ++l) {
+    BlockP& b = h->blocks[l];
+    const int depth = (int)b.stack.size();
+    const bf16* blk_dxo = l == h->L - 1 ? (const bf16*)dxout : (const bf16*)dx_slab<bf16>(h, l);      // d x_out of this block (or null)
+    bf16* blk_dx = (bf16*)(l > 0 ? dx_slab<bf16>(h, l - 1) : h->dxA);                                   // gradient wrt the block input
+    const int next_first = conv_index + depth;      // desc that writes blk_dxo (first conv of block l + 1), if any
+    const bool dxo_in_launch = blk_dxo != nullptr && l < h->L - 1;
+    for (int j = 0; j < depth; ++j, ++conv_index) {
+      const ConvP& cv = b.stack[j];
+      TcStackBwdDesc d{};
+      const bool alias = h->alias_skip && dskip != nullptr;      // skip = conv1's output: d skip joins d x_out in front of Wr^T
+      d.B = B; d.T = Tn; d.nseg = cv.K; d.D = h->D; d.R = h->R; d.S = dskip ? (alias ? h->R : h->S) : 0;
+      for (int k = 0; k < cv.K; ++k) d.shift[k] = (cv.K - 1 - k) * cv.dil;
+      d.Wb = cv.Wb16; d.k_b = rup(cv.Kb16, 64);
+      d.drop_scale = h->drop_active ? 1.0f / (1.0f - c.dropout) : 0.f;
+      d.ein_layer = -1;
+      // what this conv's tile writes: the gradient wrt its input
+      d.dx = j == 0 ? blk_dx : (bf16*)h->dp_keep[l][j - 1];
+      if (j == 0) {
+        // first conv of the block: the block input is not activated; the residual gradient joins here
+        if (c.use_residual && blk_dxo) { d.out_mode = 1; d.ein = blk_dxo; d.ein_layer = dxo_in_launch ? next_first : -1; }
+        if (h->drop_active) d.mask = h->drop_mask + (size_t)l * rows_cap * h->R;
+      } else {
+        d.out_mode = 2; d.act = c.activation; d.ein = (const bf16*)h->acts[l][j - 1];
+      }
+      if (j < depth - 1) {
+        d.plain = 1; d.gin = (const bf16*)h->dp_keep[l][j];
+      } else {
+        d.dxo = blk_dxo;
+        d.dskip = ((b.has_skip || alias) && dskip) ? (const bf16*)dskip : nullptr; d.lds = h->Sp;
+        d.alias = alias ? 1 : 0;
+        d.z = (const bf16*)h->zbuf[l]; d.dz = (bf16*)dz_slab<bf16>(h, l);
+        const int rs = h->R + (b.has_skip ? h->S : 0), koff = (d.dxo || alias) ? 0 : h->R;
+        d.Wdg = b.Wdg16 + koff; d.k_dg = rup(rs, 64);
+        d.has_res = (c.use_residual && depth == 1) ? 1 : 0;
+      }
+      bdescs.push_back(d);
     }
-    const long long kr = (long long)h->K * h->R;
-    {
-      LaunchScope ls(h, s_, CLS_MISC);
-      reduce_parts_tall<<<cdiv(kr, 32), 256, 0, s_>>>(h->colpart, nparts, (long long)(h->K + 1) * h->R, G_(h, h->input_conv.w_idx), kr,
-                                                   l2coef != 0.f ? P_(h, h->input_conv.w_idx) : nullptr, l2coef);
+  }
+  TcStackBwdPlan* sp = nullptr;
+  for (auto& q : h->stack_bwd_plans) if (q.B == B && q.T == Tn && q.drop == h->drop_active) sp = &q;
+  if (!sp) RET(new_plan(h, st, h->stack_bwd_plans, TcStackBwdPlan{}, "stack backward", [&](TcStackBwdPlan& p) { return tc_stack_bwd_build(h->tmaps, bdescs, &p); }, &sp));
+  if (!sp) return WN_OK;
+  LaunchLabel lab(h, "stack_bwd");
+  LaunchScope ls(h, st, CLS_DILATED);
+  const int r = tc_stack_bwd_launch(st, *sp, bdescs[0]);
+  if (r == 0) { *stacked = true; h->stack_bwd_layers = h->L; }
+  else if (r == -100) h->launches--;
+  else { set_err("stack backward launch failed (%d): %s", r, tc_last_error()); return WN_ERR_CUDA; }
+  return WN_OK;
+}
+
+// ---- per-block chain, behind the stack-backward launch when it ran (the blocks then only collect their weight-gradient
+// problems); with side launches, a side group's weight gradients start as soon as its block is done.  *dxout: d x_out of block 0
+template <class T>
+static int block_chain(wn_handle* h, cudaStream_t st, const BwdSchedule& s, int B, int Tn, float l2coef, const void** dxout_out) {
+  const wn_config& c = h->cfg;
+  const void* dskip = c.use_skip ? h->dskip : nullptr;
+  const void* dxout = c.use_skip ? nullptr : (s.group ? dx_slab<T>(h, h->L - 1) : h->dxA);
+  bool stacked = false;
+  if constexpr (sizeof(T) == 2) {
+    if (s.sb) RET(stack_backward(h, st, B, Tn, dxout, dskip, &stacked));
+  }
+  for (int l = h->L - 1; l >= 0; --l) {
+    const void* x_in = l > 0 ? h->xout[l - 1] : h->h0;
+    // grouped weight gradients: d x_out and d z of every block keep their own buffers until the grouped launch
+    void* dx_in = s.group ? (l > 0 ? dx_slab<T>(h, l - 1) : h->dxA) : ((dxout == h->dxA) ? h->dxB : h->dxA);
+    BwdSide sd;
+    BlockBwdMode m;
+    m.side = side_setup(h, st, l, s.use_side, &sd);
+    m.dz = s.group ? dz_slab<T>(h, l) : ((l & 1) ? h->dz2 : h->dz);
+    m.grouped = s.group; m.in_stack = stacked;
+    m.side_group = s.side_group(h, l); m.bucket = s.bucket(h, l);
+    RET(block_backward<T>(h, st, l, x_in, dxout, h->R, dskip, h->Sp, dx_in, h->R, B, Tn, l2coef, m));
+    if constexpr (sizeof(T) == 2) {
+      const int g = m.side_group;
+      if (s.side_now && g >= 0 && g < (int)s.wplan->side.size() && s.wplan->side[g].second > 0) {
+        // d z_l and d x_out_l are complete behind this block's kernels: its weight gradients start on the side stream
+        CK(cudaEventRecord(h->ev_blk_dz[l], st));
+        CK(cudaStreamWaitEvent(h->side_stream, h->ev_blk_dz[l], 0));
+        LaunchLabel lab(h, "wgrad_group");
+        LaunchScope ls(h, h->side_stream, CLS_DILATED);
+        int r = tc_wgrad_group_launch(h->side_stream, *s.wplan, s.wplan->side[g].first, s.wplan->side[g].second);
+        if (r != 0) { set_err("grouped wgrad side launch failed (%d): %s", r, tc_last_error()); return WN_ERR_CUDA; }
+        h->wg_last_side++;
+      }
     }
-    {
-      LaunchScope ls(h, s_, CLS_MISC);
-      reduce_parts_tall<<<cdiv(h->R, 32), 256, 0, s_>>>(h->colpart + kr, nparts, (long long)(h->K + 1) * h->R, G_(h, h->input_conv.b_idx), h->R, nullptr, 0.f);
+    dxout = dx_in;
+  }
+  *dxout_out = dxout;
+  return WN_OK;
+}
+
+// ---- input conv (model.py:84-88): dW[k][c], db[c].  HBM-bound, small CTAs
+template <class T>
+static void input_conv_backward(wn_handle* h, cudaStream_t s_, const float* x, int ldx, const void* dxout, int ld_dx, int B, int Tn, float l2coef) {
+  OuterLabel ol(h, "input_conv_bwd");
+  const bool wide = h->R % 2 == 0 && h->R / 2 <= 256 && ld_dx % 2 == 0;
+  const int chunks = cdiv(Tn, 64);
+  const int nparts = wide ? cdiv((long long)B * Tn, ICB_ROWS) : B * chunks;
+  {
+    LaunchScope ls(h, s_, CLS_MISC);
+    if (wide)
+      input_conv_bwd_stage1_wide<T><<<nparts, 256, 0, s_>>>(x, ldx, (const T*)dxout, ld_dx, h->colpart, B, Tn, h->R, h->K);
+    else
+      input_conv_bwd_stage1<T><<<dim3(cdiv(h->R, 64), chunks, B), 64, 0, s_>>>(x, ldx, (const T*)dxout, ld_dx, h->colpart, B, Tn, h->R, h->K, 64);
+  }
+  const long long kr = (long long)h->K * h->R;
+  {
+    LaunchScope ls(h, s_, CLS_MISC);
+    reduce_parts_tall<<<cdiv(kr, 32), 256, 0, s_>>>(h->colpart, nparts, (long long)(h->K + 1) * h->R, G_(h, h->input_conv.w_idx), kr,
+                                                 l2coef != 0.f ? P_(h, h->input_conv.w_idx) : nullptr, l2coef);
+  }
+  {
+    LaunchScope ls(h, s_, CLS_MISC);
+    reduce_parts_tall<<<cdiv(h->R, 32), 256, 0, s_>>>(h->colpart + kr, nparts, (long long)(h->K + 1) * h->R, G_(h, h->input_conv.b_idx), h->R, nullptr, 0.f);
+  }
+}
+
+// ---- every block's conv1 / conv_skip / gated-conv weight gradients in ONE launch (+ one finish), or bucket by bucket with the
+// early all-reduce; *cond_done: the bucket launches also wrote the conditioning filter gradients
+static int grouped_wgrad(wn_handle* h, cudaStream_t st, const BwdSchedule& s, int B, int Tn, float l2coef, bool* cond_done) {
+  const TcWgGroupPlan* plan = s.wplan;
+  if (!plan) {
+    wn_handle::WgPlan* wp = nullptr;
+    RET(new_plan(h, st, h->wg_plans, wn_handle::WgPlan{B, Tn, h->drop_active, s.sb, s.nb, TcWgGroupPlan{}}, "grouped wgrad", [&](wn_handle::WgPlan& p) {
+      return tc_wgrad_group_build(h->tmaps, h->wg_jobs, B, Tn, h->wg_force_split, h->wg_pair_tiles != 0, s.side_pairs, &p.plan);
+    }, &wp));
+    if (!wp) { set_err("grouped wgrad: no plan for (%d, %d) while capturing", B, Tn); return WN_ERR_STATE; }
+    plan = &wp->plan;
+  }
+  LaunchLabel lab(h, "wgrad_group");
+  h->wg_last_tiles = plan->ntiles; h->wg_last_partials = plan->npartial;
+  if (s.nb > 1 && (int)plan->buckets.size() == s.nb && !s.side_now) {
+    // ---- bucket by bucket: launch, finish, (conditioning filter gradients of the bucket's blocks,) all-reduce on comm_stream
+    auto block_off = [&](int l) -> long long {
+      if (l < h->L) return h->params[h->blocks[l].stack[0].w_idx].offset;
+      if (!h->head.empty()) return h->params[h->head[0].w_idx].offset;
+      if (!h->map_w.empty()) return h->params[h->map_w[0]].offset;
+      return h->n_scalars;
+    };
+    for (int k = 0; k < s.nb; ++k) {
+      const TcWgGroupPlan::Bucket& bk = plan->buckets[k];
+      {
+        LaunchScope ls(h, st, CLS_DILATED);
+        int r = tc_wgrad_group_launch(st, *plan, bk.unit0, bk.nunits);
+        if (r != 0) { set_err("grouped wgrad launch failed (%d): %s", r, tc_last_error()); return WN_ERR_CUDA; }
+      }
+      {
+        OuterLabel ol(h, "wgrad_group_finish");
+        LaunchScope ls(h, st, CLS_DILATED);
+        int r = tc_wgrad_group_finish_launch(st, *plan, l2coef, k);
+        if (r != 0) { set_err("grouped wgrad finish failed (%d): %s", r, tc_last_error()); return WN_ERR_CUDA; }
+      }
+      // blocks of this bucket: l_hi .. l_lo (descending walk: bucket 0 holds the last blocks)
+      int l_lo = h->L, l_hi = -1;
+      for (int l = 0; l < h->L; ++l) if (s.bucket(h, l) == k) { if (l < l_lo) l_lo = l; if (l > l_hi) l_hi = l; }
+      if (h->cfg.conditioning && l_hi >= l_lo) {
+        OuterLabel ol(h, "cond_bwd");
+        LaunchScope ls(h, st, CLS_MISC);
+        const int n = 2 * h->D;
+        cond_wgrad_all<<<dim3(cdiv((h->Cc + 1) * n, 128), l_hi - l_lo + 1), 128, 0, st>>>(h->last_cond, h->Cc, h->dcb, (long long)h->maxB * n, h->d_params,
+                                                                                     h->d_grads, h->d_cond_offsets, B, n, l2coef, l_lo);
+      }
+      if (k + 1 < s.nb && l_hi >= l_lo) {
+        // every gradient of blocks l_lo .. l_hi is final: reduce that slice of the flat buffer beside the next bucket's kernels
+        const long long lo = block_off(l_lo), hi = block_off(l_hi + 1);
+        CK(cudaEventRecord(h->ev_bucket[k], st));
+        CK(cudaStreamWaitEvent(h->comm_stream, h->ev_bucket[k], 0));
+        h->launches++;
+        const int r = g_nccl.AllReduce(h->d_grads + lo, h->d_grads + lo, (size_t)(hi - lo), WN_NCCL_FLOAT32, WN_NCCL_SUM, h->comm, h->comm_stream);
+        if (r != 0) { set_err("ncclAllReduce (bucket %d) failed (%d): %s", k, r, nccl_errstr(r)); return WN_ERR_CUDA; }
+        h->last_ar_buckets++;
+        if (h->ar_early_lo < 0 || lo < h->ar_early_lo) h->ar_early_lo = lo;
+        if (hi > h->ar_early_hi) h->ar_early_hi = hi;
+      }
     }
-  };
-  // (the stack-backward path has no side launches, but the same trick applies: d h0 is final behind the chain launch, and the
-  // three small launches run beside the grouped weight-gradient launch instead of behind it)
-  const bool icb_side = !side_now && h->stack_bwd_layers > 0 && h->side_stream != nullptr && h->prof_tag == 0 && group && !h->wg_jobs.empty();
-  if (side_now || icb_side) {
+    *cond_done = h->cfg.conditioning != 0;
+    return WN_OK;
+  }
+  {
+    LaunchScope ls(h, st, CLS_DILATED);
+    // without side launches (first call of a shape, profiling passes, WN_TC_GROUP_SIDE_EVERY=0) the side groups' units, which
+    // follow the final group's in the table, run in the same launch
+    int r = tc_wgrad_group_launch(st, *plan, 0, s.side_now ? plan->final_units : plan->nunits);
+    if (r != 0) { set_err("grouped wgrad launch failed (%d): %s", r, tc_last_error()); return WN_ERR_CUDA; }
+  }
+  if (s.side_now) {
+    // the side launches of this pass must be complete before the finish reads their partial tiles
+    CK(cudaEventRecord(h->ev_wg_side, h->side_stream));
+    CK(cudaStreamWaitEvent(st, h->ev_wg_side, 0));
+  }
+  OuterLabel ol(h, "wgrad_group_finish");
+  LaunchScope ls(h, st, CLS_DILATED);
+  int r = tc_wgrad_group_finish_launch(st, *plan, l2coef);
+  if (r != 0) { set_err("grouped wgrad finish failed (%d): %s", r, tc_last_error()); return WN_ERR_CUDA; }
+  return WN_OK;
+}
+
+template <class T>
+static int model_backward(wn_handle* h, cudaStream_t st, const float* x, int ldx, const float* cond_in, int B, int Tn, float l2coef) {
+  const BwdSchedule s = bwd_schedule<T>(h, B, Tn);
+  h->wg_jobs.clear();
+  h->wg_last_tiles = 0; h->wg_last_side = 0;
+  h->stack_bwd_layers = 0;
+  h->ar_early_lo = h->ar_early_hi = -1;
+  h->last_ar_buckets = 0;
+  const void* dxout;
+  {
+    // with side launches, the persistent kernels of the head and the chain leave CTA pairs free for them
+    TcBalanceScope balance(s.side_now);
+    RET(head_backward<T>(h, st, s, B, Tn, l2coef));
+    if (s.cat) RET(cat_chain<T>(h, st, s, B, Tn, l2coef, &dxout));
+    else RET(block_chain<T>(h, st, s, B, Tn, l2coef, &dxout));
+  }
+  const int ld_dx = s.cat ? h->R + h->S : h->R;
+  // The input conv's gradients run on the side stream beside the final grouped weight-gradient launch (their CTAs fit next to
+  // the tensor kernel's on the same SMs) with side launches, and behind the stack-backward launch: d h0 is final there too.
+  const bool grouped = s.group && !h->wg_jobs.empty();
+  const bool icb_side = !s.side_now && h->stack_bwd_layers > 0 && h->side_stream != nullptr && h->prof_tag == 0 && grouped;
+  if (s.side_now || icb_side) {
     CK(cudaEventRecord(h->ev_blk_in[0], st));
     CK(cudaStreamWaitEvent(h->side_stream, h->ev_blk_in[0], 0));
-    input_conv_bwd(h->side_stream);
-    input_conv_done = true;
-    if (!(group && !h->wg_jobs.empty())) { CK(cudaEventRecord(h->ev_wg_side, h->side_stream)); CK(cudaStreamWaitEvent(st, h->ev_wg_side, 0)); }
+    input_conv_backward<T>(h, h->side_stream, x, ldx, dxout, ld_dx, B, Tn, l2coef);
+    if (!grouped) { CK(cudaEventRecord(h->ev_wg_side, h->side_stream)); CK(cudaStreamWaitEvent(st, h->ev_wg_side, 0)); }
   }
+  bool cond_wgrad_done = false;
   if constexpr (sizeof(T) == 2) {
-    if (group && !h->wg_jobs.empty()) {
-      // ---- every block's conv1 / conv_skip / gated-conv weight gradients in ONE launch (+ one finish)
-      TcWgGroupPlan* plan = wplan;
-      if (!plan) {
-        cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
-        cudaStreamIsCapturing(st, &cs);
-        if (cs != cudaStreamCaptureStatusNone) { set_err("grouped wgrad: no plan for (%d, %d) while capturing", B, Tn); return WN_ERR_STATE; }
-        if (h->wg_plans.size() >= 4) {
-          // captured step graphs hold pointers into the plans' tables: they go with them
-          CK(cudaDeviceSynchronize());
-          for (auto& g : h->graphs) if (g.exec) cudaGraphExecDestroy(g.exec);
-          h->graphs.clear();
-          for (auto& wp : h->wg_plans) wp.plan.release();
-          h->wg_plans.clear();
-        }
-        h->wg_plans.push_back(wn_handle::WgPlan{B, Tn, h->drop_active, sb_ok, nb, TcWgGroupPlan{}});
-        plan = &h->wg_plans.back().plan;
-        int r = tc_wgrad_group_build(h->tmaps, h->wg_jobs, B, Tn, h->wg_force_split, h->wg_pair_tiles != 0, side_pairs, plan);
-        if (r != 0) { h->wg_plans.pop_back(); set_err("grouped wgrad plan failed (%d): %s", r, tc_last_error()); return WN_ERR_CUDA; }
-      }
-      bool cond_wgrad_done = false;
-      if (nb > 1 && (int)plan->buckets.size() == nb && !side_now) {
-        // ---- bucket by bucket: launch, finish, (conditioning filter gradients of the bucket's blocks,) all-reduce on comm_stream
-        struct Label { wn_handle* h; Label(wn_handle* h_, const char* l) : h(h_) { h->cur_label = l; } ~Label() { h->cur_label = "misc"; } } lab(h, "wgrad_group");
-        h->wg_last_tiles = plan->ntiles; h->wg_last_partials = plan->npartial;
-        for (int k = 0; k < nb; ++k) {
-          const TcWgGroupPlan::Bucket& bk = plan->buckets[k];
-          {
-            LaunchScope ls(h, st, CLS_DILATED);
-            int r = tc_wgrad_group_launch(st, *plan, bk.unit0, bk.nunits);
-            if (r != 0) { set_err("grouped wgrad launch failed (%d): %s", r, tc_last_error()); return WN_ERR_CUDA; }
-          }
-          {
-            OuterLabel ol(h, "wgrad_group_finish");
-            LaunchScope ls(h, st, CLS_DILATED);
-            int r = tc_wgrad_group_finish_launch(st, *plan, l2coef, k);
-            if (r != 0) { set_err("grouped wgrad finish failed (%d): %s", r, tc_last_error()); return WN_ERR_CUDA; }
-          }
-          // blocks of this bucket: l_hi .. l_lo (descending walk: bucket 0 holds the last blocks)
-          int l_lo = h->L, l_hi = -1;
-          for (int l = 0; l < h->L; ++l) if (bucket_of(l) == k) { if (l < l_lo) l_lo = l; if (l > l_hi) l_hi = l; }
-          if (c.conditioning && l_hi >= l_lo) {
-            OuterLabel ol(h, "cond_bwd");
-            LaunchScope ls(h, st, CLS_MISC);
-            const int n = 2 * h->D;
-            cond_wgrad_all<<<dim3(cdiv((h->Cc + 1) * n, 128), l_hi - l_lo + 1), 128, 0, st>>>(h->last_cond, h->Cc, h->dcb, (long long)h->maxB * n, h->d_params,
-                                                                                         h->d_grads, h->d_cond_offsets, B, n, l2coef, l_lo);
-          }
-          if (k + 1 < nb && l_hi >= l_lo) {
-            // every gradient of blocks l_lo .. l_hi is final: reduce that slice of the flat buffer beside the next bucket's kernels
-            const long long lo = block_off(l_lo), hi = block_off(l_hi + 1);
-            CK(cudaEventRecord(h->ev_bucket[k], st));
-            CK(cudaStreamWaitEvent(h->comm_stream, h->ev_bucket[k], 0));
-            h->launches++;
-            const int r = g_nccl.AllReduce(h->d_grads + lo, h->d_grads + lo, (size_t)(hi - lo), WN_NCCL_FLOAT32, WN_NCCL_SUM, h->comm, h->comm_stream);
-            if (r != 0) { set_err("ncclAllReduce (bucket %d) failed (%d): %s", k, r, nccl_errstr(r)); return WN_ERR_CUDA; }
-            h->last_ar_buckets++;
-            if (h->ar_early_lo < 0 || lo < h->ar_early_lo) h->ar_early_lo = lo;
-            if (hi > h->ar_early_hi) h->ar_early_hi = hi;
-          }
-        }
-        cond_wgrad_done = c.conditioning != 0;
-      } else
-      {
-        struct Label { wn_handle* h; Label(wn_handle* h_, const char* l) : h(h_) { h->cur_label = l; } ~Label() { h->cur_label = "misc"; } } lab(h, "wgrad_group");
-        {
-          LaunchScope ls(h, st, CLS_DILATED);
-          h->wg_last_tiles = plan->ntiles; h->wg_last_partials = plan->npartial;
-          // without side launches (first call of a shape, profiling passes, WN_TC_GROUP_SIDE_EVERY=0) the side groups' units, which
-          // follow the final group's in the table, run in the same launch
-          int r = tc_wgrad_group_launch(st, *plan, 0, side_now ? plan->final_units : plan->nunits);
-          if (r != 0) { set_err("grouped wgrad launch failed (%d): %s", r, tc_last_error()); return WN_ERR_CUDA; }
-        }
-        if (side_now) {
-          // the side launches of this pass must be complete before the finish reads their partial tiles
-          CK(cudaEventRecord(h->ev_wg_side, h->side_stream));
-          CK(cudaStreamWaitEvent(st, h->ev_wg_side, 0));
-        }
-        {
-          OuterLabel ol(h, "wgrad_group_finish");
-          LaunchScope ls(h, st, CLS_DILATED);
-          int r = tc_wgrad_group_finish_launch(st, *plan, l2coef);
-          if (r != 0) { set_err("grouped wgrad finish failed (%d): %s", r, tc_last_error()); return WN_ERR_CUDA; }
-        }
-      }
-      h->cond_wgrad_done = cond_wgrad_done;
-    }
+    if (grouped) RET(grouped_wgrad(h, st, s, B, Tn, l2coef, &cond_wgrad_done));
   }
   if (icb_side) {
     // join: the input conv's gradients are part of what the all-reduce behind this pass (and the caller) reads
@@ -2161,18 +2204,10 @@ static int model_backward(wn_handle* h, cudaStream_t st, const float* x, int ldx
     CK(cudaStreamWaitEvent(st, h->ev_wg_side, 0));
   }
   // join: every side-stream wgrad (and its finish kernel) is complete before anything below reads the gradients
-  if (use_side) CK(cudaStreamWaitEvent(st, h->ev_blk_done[0], 0));
-  if (!input_conv_done) input_conv_bwd(st);
-  if (c.conditioning) { OuterLabel ol(h, "cond_bwd"); RET(cond_backward(h, st, cond_in, h->last_cond, B, 0, h->L, true, h->dcond, l2coef, h->cond_wgrad_done)); }
-  h->cond_wgrad_done = false;
+  if (s.use_side) CK(cudaStreamWaitEvent(st, h->ev_blk_done[0], 0));
+  if (!s.side_now && !icb_side) input_conv_backward<T>(h, st, x, ldx, dxout, ld_dx, B, Tn, l2coef);
+  if (h->cfg.conditioning) { OuterLabel ol(h, "cond_bwd"); RET(cond_backward(h, st, cond_in, h->last_cond, B, 0, h->L, true, h->dcond, l2coef, cond_wgrad_done)); }
   return WN_OK;
-}
-
-// captured step graphs bake in the launch sequence: anything that changes it (communicator, fused all-reduce) drops them
-static void drop_graphs_fwd(wn_handle* h) {
-  cudaDeviceSynchronize();
-  for (auto& g : h->graphs) if (g.exec) cudaGraphExecDestroy(g.exec);
-  h->graphs.clear();
 }
 
 // ============================================================================ public entry points
@@ -2514,10 +2549,6 @@ extern "C" int wn_adam_restore(wn_handle* h, const float* m_dev, const float* v_
   return WN_OK;
 }
 
-static void drop_graphs(wn_handle* h) {
-  for (auto& g : h->graphs) if (g.exec) cudaGraphExecDestroy(g.exec);
-  h->graphs.clear();
-}
 extern "C" int wn_set_dropout_masks(wn_handle* h, const uint8_t* keep_host, int B, int T) {
   RET(check_bt(h, B, T));
   if (h->cfg.dropout <= 0.f || !h->drop_mask) { set_err("model was built with dropout == 0"); return WN_ERR_STATE; }
@@ -2667,7 +2698,8 @@ extern "C" int wn_comm_init(wn_handle* h, const uint8_t* id128, int nranks, int 
   const int r = g_nccl.CommInitRank(&c, nranks, id, rank);
   if (r != 0) { set_err("ncclCommInitRank failed (%d): %s", r, nccl_errstr(r)); return WN_ERR_CUDA; }
   h->comm = c; h->comm_owned = true; h->comm_nranks = nranks; h->comm_rank = rank;
-  drop_graphs_fwd(h);
+  cudaDeviceSynchronize();
+  drop_graphs(h);
   return WN_OK;
 }
 extern "C" int wn_comm_attach(wn_handle* h, void* nccl_comm, int nranks, int rank) {
@@ -2676,12 +2708,13 @@ extern "C" int wn_comm_attach(wn_handle* h, void* nccl_comm, int nranks, int ran
   if (nccl_comm && nccl_load(err, sizeof(err)) != 0) { set_err("%s", err); return WN_ERR_CUDA; }
   if (h->comm && h->comm_owned) g_nccl.CommDestroy(h->comm);
   h->comm = (wn_ncclComm_t)nccl_comm; h->comm_owned = false; h->comm_nranks = nccl_comm ? nranks : 1; h->comm_rank = rank;
-  drop_graphs_fwd(h);
+  cudaDeviceSynchronize();
+  drop_graphs(h);
   return WN_OK;
 }
 extern "C" int wn_comm_fuse_allreduce(wn_handle* h, int on) {
   if (!h) { set_err("null handle"); return WN_ERR_VALUE; }
-  if ((on != 0) != (h->ar_in_step != 0)) { h->ar_in_step = on ? 1 : 0; drop_graphs_fwd(h); }
+  if ((on != 0) != (h->ar_in_step != 0)) { h->ar_in_step = on ? 1 : 0; cudaDeviceSynchronize(); drop_graphs(h); }
   return WN_OK;
 }
 extern "C" int wn_allreduce_grads(wn_handle* h, void* stream) {
@@ -2737,7 +2770,7 @@ static int step_common(wn_handle* h, const float* frames_dev, const float* cond_
     for (auto& g : h->graphs)
       if (g.frames == frames_dev && g.cond == cond_dev && g.B == B && g.T == T && g.nrep == n_replicas && g.loss == loss_dev && g.train == train) { sg = &g; break; }
     if (!sg) {
-      if (h->graphs.size() >= 8) { for (auto& g : h->graphs) if (g.exec) cudaGraphExecDestroy(g.exec); h->graphs.clear(); }
+      if (h->graphs.size() >= 8) drop_graphs(h);
       h->graphs.push_back({frames_dev, cond_dev, B, T, n_replicas, loss_dev, train, 0, 0, nullptr});
       sg = &h->graphs.back();
     }
@@ -2921,7 +2954,7 @@ static int layer_bwd_entry(wn_handle* h, int l, const float* dxo, const float* d
     dsk_t = h->dskip;
   }
   const void* xin = l == 0 ? h->layer_in : h->xout[l - 1];
-  RET(block_backward<T>(h, st, l, xin, dxo_t, h->R, dsk_t, h->Sp, dx ? h->dxB : nullptr, h->R, B, Tn, 0.f));
+  RET(block_backward<T>(h, st, l, xin, dxo_t, h->R, dsk_t, h->Sp, dx ? h->dxB : nullptr, h->R, B, Tn, 0.f, BlockBwdMode{}));
   if (dx) {
     LaunchScope ls(h, st, CLS_MISC);
     convert_kernel<T, float><<<cdiv(nR, 256), 256, 0, st>>>((const T*)h->dxB, dx, nR);
