@@ -167,6 +167,15 @@ int wn_forward(wn_handle* h, const float* x_dev, const float* cond_dev, int B, i
 /* the same with Keras' `training` argument (model.py:213, layers.py:178,195-196): training != 0 applies the block dropout
  * (fresh Philox masks, or the masks injected with wn_set_dropout_masks) exactly as the forward half of wn_train_step does. */
 int wn_forward_ex(wn_handle* h, const float* x_dev, const float* cond_dev, int B, int T, int training, float* out_dev, void* stream);
+/* Adjoint of the last wn_forward_ex on this handle (tf.GradientTape over WaveNet.call, model.py:213-239):
+ * dpred (B,T,Cout) fp32, 16-byte aligned = d loss / d (the tensor wn_forward_ex returned: softmax probabilities, or the 3M
+ * mixture parameters).  Every parameter gradient lands in wn_grads_dev(), overwritten: no L2 term (model.py:331-334 belongs
+ * to train_step, not to call), no loss scaling, no all-reduce.  dcond_dev (B,cond_in) fp32 or NULL receives
+ * d loss / d cond (through the mapping MLP).  x and cond passed to that forward must still be valid.  The dropout masks of
+ * a training forward are reused.  Calling it twice after one forward gives the same gradients.
+ * WN_ERR_STATE: no wn_forward_ex since the handle's activations, weights or dropout masks last changed (a train/test
+ * step, wn_generate, a wn_layer_* forward, wn_set_param / wn_params_changed / wn_adam_step, wn_set_dropout_masks). */
+int wn_backward(wn_handle* h, const float* dpred_dev, float* dcond_dev, void* stream);
 
 /* ---- WaveNet.loss_fn(target, pred) (model.py:505-551) on MATERIALISED predictions ------------------------------------
  * pred (B,T,Cout) fp32 = a WaveNet.call output (softmax probabilities, or [weights | means | log-scales] mixture
@@ -249,7 +258,7 @@ int wn_debug_bench(int which, int reps, const void* a_bf16_dev, int lda, const v
                    int nseg, const int* shifts, int K, int N, void* out_dev, int ldo, float* ms_out);
 
 /* ---- introspection for benchmarks --------------------------------------------------------- */
-/* number of kernel launches issued by the last wn_train_step / wn_forward on this handle */
+/* number of kernel launches issued by the last wn_train_step / wn_forward / wn_backward on this handle */
 int64_t wn_last_launch_count(const wn_handle* h);
 /* accumulate CUDA-event time of one kernel class over subsequent steps: tag 0 = off,
  * 1 = dilated-conv GEMMs (fwd+dgrad+wgrad), 2 = all GEMMs, 3 = loss/head reductions */
@@ -277,7 +286,7 @@ int wn_profile_begin(wn_handle* h, int tag);
 int wn_profile_end(wn_handle* h, double* ms, int64_t* launches);
 /* per-launch record of the last wn_profile_end: returns the number of timed launches; fills duration (ms) and a
  * short label of launch i: the phase ("input_conv_fwd", "cond_fwd", "skip_sum", "head_fwd", "loss", "loss_finalize",
- * "head_bwd", "wgrad_group_finish", "input_conv_bwd", "cond_bwd") or, inside the block loop, the kernel ("stack_fwd",
+ * "head_bwd", "wgrad_group_finish", "input_conv_bwd", "cond_bwd", "pred_vjp" (wn_backward's adjoint of the predictions)) or, inside the block loop, the kernel ("stack_fwd",
  * "block_fwd", "gate", "bias_act_res", "gate_bwd", "dgrad", "wgrad_dilated", "wgrad_1x1", "wgrad_group", "misc") */
 int wn_profile_get(wn_handle* h, int i, double* ms, char* label, int label_len);
 const char* wn_build_info(void);

@@ -847,6 +847,98 @@ __global__ void __launch_bounds__(256) softmax_ce_reg_kernel(const float* __rest
   }
 }
 
+// ------------------------------------------------------------------ adjoint of the probabilities WaveNet.call returns (model.py:238)
+// dlogits[r][c] = p_c (dp_c - sum_j p_j dp_j) for a caller's dp = d loss / d p.  One warp per row; p is recomputed from the logits
+// with softmax_ce_kernel's arithmetic, so it is bit-for-bit the p that wn_forward returned.  Columns [C, ldd) are zeroed: the head's
+// dgrad contracts over ldd columns on the bf16 tier.
+template <class TD>
+__global__ void __launch_bounds__(256) softmax_vjp_kernel(const float* __restrict__ logits, int C, const float* __restrict__ dp, long long rows,
+                                                          TD* __restrict__ dlogits, int ldd) {
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const long long row = (long long)blockIdx.x * 8 + warp;
+  if (row >= rows) return;
+  const float* lp = logits + row * C;
+  const float* gp = dp + row * C;
+  float m = -INFINITY;
+  for (int c = lane * 4; c < C; c += 128) {
+    const float4 v = *reinterpret_cast<const float4*>(lp + c);
+    m = fmaxf(m, fmaxf(fmaxf(v.x, v.y), fmaxf(v.z, v.w)));
+  }
+  m = warp_max(m);
+  float s = 0.f;
+  for (int c = lane * 4; c < C; c += 128) {
+    const float4 v = *reinterpret_cast<const float4*>(lp + c);
+    s += expf(v.x - m) + expf(v.y - m) + expf(v.z - m) + expf(v.w - m);
+  }
+  s = warp_sum(s);
+  const float inv = 1.0f / s;
+  float dot = 0.f;
+  for (int c = lane * 4; c < C; c += 128) {
+    const float4 v = *reinterpret_cast<const float4*>(lp + c);
+    const float4 g = *reinterpret_cast<const float4*>(gp + c);
+    dot += expf(v.x - m) * inv * g.x + expf(v.y - m) * inv * g.y + expf(v.z - m) * inv * g.z + expf(v.w - m) * inv * g.w;
+  }
+  dot = warp_sum(dot);
+  for (int c = lane * 4; c < C; c += 128) {
+    const float4 v = *reinterpret_cast<const float4*>(lp + c);
+    const float4 g = *reinterpret_cast<const float4*>(gp + c);
+    const float p[4] = {expf(v.x - m) * inv, expf(v.y - m) * inv, expf(v.z - m) * inv, expf(v.w - m) * inv};
+    const float gv[4] = {g.x, g.y, g.z, g.w};
+#pragma unroll
+    for (int i = 0; i < 4; ++i) dlogits[row * ldd + c + i] = from_f<TD>(p[i] * (gv[i] - dot));
+  }
+  for (int c = C + lane; c < ldd; c += 32) dlogits[row * ldd + c] = from_f<TD>(0.f);
+}
+
+// register-resident variant for C = 128 * NV4 classes (C = 256 for 8-bit audio): logits and dp are read once; p has the arithmetic
+// order of softmax_ce_reg_kernel (bit-identical to softmax_vjp_kernel)
+template <class TD, int NV4>
+__global__ void __launch_bounds__(256) softmax_vjp_reg_kernel(const float* __restrict__ logits, const float* __restrict__ dp, long long rows,
+                                                              TD* __restrict__ dlogits, int ldd) {
+  constexpr int C = 128 * NV4;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const long long row = (long long)blockIdx.x * 8 + warp;
+  if (row >= rows) return;
+  float4 v[NV4], g[NV4];
+#pragma unroll
+  for (int i = 0; i < NV4; ++i) {
+    v[i] = *reinterpret_cast<const float4*>(logits + row * C + lane * 4 + i * 128);
+    g[i] = *reinterpret_cast<const float4*>(dp + row * C + lane * 4 + i * 128);
+  }
+  float m = -INFINITY;
+#pragma unroll
+  for (int i = 0; i < NV4; ++i) m = fmaxf(m, fmaxf(fmaxf(v[i].x, v[i].y), fmaxf(v[i].z, v[i].w)));
+  m = warp_max(m);
+  float s = 0.f;
+#pragma unroll
+  for (int i = 0; i < NV4; ++i) {
+    v[i].x = expf(v[i].x - m); v[i].y = expf(v[i].y - m); v[i].z = expf(v[i].z - m); v[i].w = expf(v[i].w - m);
+    s += v[i].x + v[i].y + v[i].z + v[i].w;
+  }
+  s = warp_sum(s);
+  const float inv = 1.0f / s;
+  float dot = 0.f;
+#pragma unroll
+  for (int i = 0; i < NV4; ++i) {
+    v[i].x *= inv; v[i].y *= inv; v[i].z *= inv; v[i].w *= inv;
+    dot += v[i].x * g[i].x + v[i].y * g[i].y + v[i].z * g[i].z + v[i].w * g[i].w;
+  }
+  dot = warp_sum(dot);
+#pragma unroll
+  for (int i = 0; i < NV4; ++i) {
+    const int c = lane * 4 + i * 128;
+    const float d[4] = {v[i].x * (g[i].x - dot), v[i].y * (g[i].y - dot), v[i].z * (g[i].z - dot), v[i].w * (g[i].w - dot)};
+    if constexpr (sizeof(TD) == 2) {
+      uint2 q;
+      q.x = pack_bf16x2(d[0], d[1]); q.y = pack_bf16x2(d[2], d[3]);
+      *reinterpret_cast<uint2*>(dlogits + row * ldd + c) = q;
+    } else {
+      *reinterpret_cast<float4*>(dlogits + row * ldd + c) = make_float4(d[0], d[1], d[2], d[3]);
+    }
+  }
+  for (int c = C + lane; c < ldd; c += 32) dlogits[row * ldd + c] = from_f<TD>(0.f);
+}
+
 // ------------------------------------------------------------------ WaveNet.loss_fn on materialised probabilities (model.py:516)
 // tf.keras.losses.sparse_categorical_crossentropy(target, probs), Keras 3 semantics [TF-internal, restated]: the probabilities
 // are clipped to [1e-7, 1 - 1e-7], their logarithm is taken as logits of sparse_softmax_cross_entropy_with_logits:

@@ -189,7 +189,9 @@ struct wn_handle {
   cudaStream_t own_stream = nullptr;
   // state
   int lastB = 0, lastT = 0;
+  // the last wn_forward_ex, which wn_backward differentiates: valid until the activations, the weights or the dropout masks change
   bool fwd_valid = false;
+  struct FwdRecord { int B = 0, T = 0; bool training = false; const float* x = nullptr; int ldx = 0; const float* cond = nullptr; } fwd;
   bool layer_fwd_valid[WN_MAX_DILATIONS] = {};
   bool layer_drop[WN_MAX_DILATIONS] = {};     // wn_layer_forward_ex ran block l with dropout active (its adjoint must too)
   // conditioning sequences of the layer API (wn_layer_forward_seq); buffers exist on layer handles with conditioning only
@@ -2339,6 +2341,7 @@ extern "C" int wn_generate(wn_handle* h, const float* prime_dev, int n_prime, co
   if (!prime_dev || n_prime < 1 || B < 1 || B > 64 || B > h->maxB || length < 1 || (!out_dev && !pred_dev)) { set_err("bad generate arguments (1 <= batch <= min(64, max_batch))"); return WN_ERR_VALUE; }
   if ((size_t)GEN_ROWS * h->K * (h->R > h->D ? h->R : h->D) * 4 > 160 * 1024) { set_err("generation: K * channels too large for the step kernel"); return WN_ERR_UNSUPPORTED; }
   CK(cudaSetDevice(h->cfg.device));
+  h->fwd_valid = false;       // (the conditioning MLP's activations and the conditioning biases are overwritten)
   cudaStream_t user = (cudaStream_t)stream, st = h->own_stream;
   const int cap = n_prime + length + 1;
   RET(gen_alloc(h, B, cap));
@@ -2555,6 +2558,7 @@ extern "C" int wn_set_dropout_masks(wn_handle* h, const uint8_t* keep_host, int 
   CK(cudaSetDevice(h->cfg.device));
   CK(cudaDeviceSynchronize());
   drop_graphs(h);
+  h->fwd_valid = false;
   if (!keep_host) { h->drop_injected = false; return WN_OK; }
   const size_t n = (size_t)B * T * h->R, slab = (size_t)h->maxB * h->maxT * h->R;
   for (int l = 0; l < h->L; ++l) CK(cudaMemcpy(h->drop_mask + l * slab, keep_host + l * n, n, cudaMemcpyHostToDevice));
@@ -2614,13 +2618,72 @@ extern "C" int wn_forward_ex(wn_handle* h, const float* x_dev, const float* cond
   if (training && h->cfg.dropout >= 1.f) { set_err("dropout must be < 1 for training"); return WN_ERR_VALUE; }
   CK(cudaSetDevice(h->cfg.device));
   h->launches = 0;
+  h->fwd_valid = false;
   cudaStream_t st = (cudaStream_t)stream;
   int r = h->cfg.precision == WN_BF16 ? forward_entry<bf16>(h, x_dev, cond_dev, B, T, training, out_dev, st)
                                       : forward_entry<float>(h, x_dev, cond_dev, B, T, training, out_dev, st);
+  h->drop_active = false;
   RET(r);
   CK(cudaGetLastError());
-  h->fwd_valid = false;
+  // (lastB / lastT stay those of the last train/test step: wn_sample_last_step reads them)
+  h->fwd = wn_handle::FwdRecord{B, T, training != 0, x_dev, T, cond_dev};
+  h->fwd_valid = true;
+  return WN_OK;
+}
+
+// d loss / d cond_in of the model: without a mapping MLP that is h->dcond; with one, cond_backward leaves the gradient of the first
+// mapping layer's pre-activation in the buffer its ping-pong ends on (d0 = dcond, then d1 = cond_dact, d2 = cond_dact2, alternating)
+static int cond_input_grad(wn_handle* h, cudaStream_t st, int B, float* dcond) {
+  const int n = (int)h->map_w.size();
+  if (n == 0) {
+    CK(cudaMemcpyAsync(dcond, h->dcond, (size_t)B * h->cfg.cond_in * 4, cudaMemcpyDeviceToDevice, st));
+    return WN_OK;
+  }
+  const float* dpre = n == 1 ? h->dcond : (n - 1) % 2 == 1 ? h->cond_dact : h->cond_dact2;
+  const int K = h->cfg.cond_in, N = h->map_width[0];
+  LaunchScope ls(h, st, CLS_MISC);
+  dense_small_dgrad<<<cdiv(B * K, 4), 128, 0, st>>>(dpre, N, P_(h, h->map_w[0]), dcond, K, B, K, N, 0);
+  return WN_OK;
+}
+
+template <class T>
+static int backward_entry(wn_handle* h, const float* dpred, float* dcond, cudaStream_t st) {
+  const int B = h->fwd.B, Tn = h->fwd.T;
+  const long long rows = (long long)B * Tn;
+  {
+    // dlogits = the adjoint of what wn_forward_ex returned: the softmax's VJP, or dpred itself for the raw mixture parameters
+    OuterLabel ol(h, "pred_vjp");
+    LaunchScope ls(h, st, CLS_LOSS);
+    if (h->cfg.sampling_function == WN_CATEGORICAL) {
+      if (h->Cout == 256 && h->ldl == 256 && h->ldd % 4 == 0)
+        softmax_vjp_reg_kernel<T, 2><<<cdiv(rows, 8), 256, 0, st>>>(h->logits, dpred, rows, (T*)h->dlogits, h->ldd);
+      else
+        softmax_vjp_kernel<T><<<cdiv(rows, 8), 256, 0, st>>>(h->logits, h->Cout, dpred, rows, (T*)h->dlogits, h->ldd);
+    } else {
+      convert_pad_kernel<float, T><<<cdiv(rows * h->ldd, 256), 256, 0, st>>>(dpred, h->Cout, (T*)h->dlogits, h->ldd, rows);
+    }
+  }
+  RET(model_backward<T>(h, st, h->fwd.x, h->fwd.ldx, h->fwd.cond, B, Tn, 0.f));
+  if (dcond) RET(cond_input_grad(h, st, B, dcond));
+  return WN_OK;
+}
+
+extern "C" int wn_backward(wn_handle* h, const float* dpred_dev, float* dcond_dev, void* stream) {
+  if (!h) { set_err("null handle"); return WN_ERR_VALUE; }
+  if (!dpred_dev || ((uintptr_t)dpred_dev & 15) != 0) { set_err("dpred must be a 16-byte aligned device buffer"); return WN_ERR_VALUE; }
+  if (dcond_dev && !h->cfg.conditioning) { set_err("the model has no conditioning input"); return WN_ERR_VALUE; }
+  if (!h->fwd_valid) { set_err("wn_backward needs a wn_forward_ex since the handle's activations or weights last changed"); return WN_ERR_STATE; }
+  CK(cudaSetDevice(h->cfg.device));
+  h->launches = 0;
+  cudaStream_t st = (cudaStream_t)stream;
+  // the stack-backward plans are keyed on drop_active, and the forward's keep-masks are still in drop_mask
+  h->drop_active = h->fwd.training && h->cfg.dropout > 0.f;
+  h->ar_now = false;
+  h->lastB = h->fwd.B; h->lastT = h->fwd.T;     // wn_debug_tensor reads the pass just differentiated
+  int r = h->cfg.precision == WN_BF16 ? backward_entry<bf16>(h, dpred_dev, dcond_dev, st) : backward_entry<float>(h, dpred_dev, dcond_dev, st);
   h->drop_active = false;
+  RET(r);
+  CK(cudaGetLastError());
   return WN_OK;
 }
 extern "C" int wn_forward(wn_handle* h, const float* x_dev, const float* cond_dev, int B, int T, float* out_dev, void* stream) {
@@ -2757,6 +2820,7 @@ static int step_common(wn_handle* h, const float* frames_dev, const float* cond_
   if (n_replicas < 1 || !frames_dev || !loss_dev) { set_err("bad step arguments"); return WN_ERR_VALUE; }
   if (train && h->cfg.dropout >= 1.f) { set_err("dropout must be < 1 for training"); return WN_ERR_VALUE; }
   CK(cudaSetDevice(h->cfg.device));
+  h->fwd_valid = false;
   cudaStream_t st = (cudaStream_t)stream;
   auto run = [&](cudaStream_t s) -> int {
     h->launches = 0;
@@ -2822,6 +2886,7 @@ extern "C" int wn_train_step_host(wn_handle* h, const float* frames_host, const 
   RET(check_bt(h, B, T));
   if (!frames_host || !loss_host) { set_err("bad step arguments"); return WN_ERR_VALUE; }
   CK(cudaSetDevice(h->cfg.device));
+  h->fwd_valid = false;
   cudaStream_t st = h->own_stream;
   const size_t fb = (size_t)B * (T + 1) * 4;
   memcpy(h->pin_frames, frames_host, fb);
@@ -2903,6 +2968,7 @@ static int layer_forward_call(wn_handle* h, int block, const float* x_dev, const
                               float* x_out_dev, float* skip_dev, void* stream) {
   CK(cudaSetDevice(h->cfg.device));
   h->launches = 0;
+  h->fwd_valid = false;
   cudaStream_t st = (cudaStream_t)stream;
   int r = h->cfg.precision == WN_BF16 ? layer_fwd_entry<bf16>(h, block, x_dev, cond_dev, seq, B, T, training, x_out_dev, skip_dev, st)
                                       : layer_fwd_entry<float>(h, block, x_dev, cond_dev, seq, B, T, training, x_out_dev, skip_dev, st);

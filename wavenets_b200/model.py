@@ -133,6 +133,7 @@ class WaveNet:
     self._sample_seed, self._sample_calls = 0x42, 0
     self._pin_logs, self._pin_events, self._pending_slot = None, None, 0
     self._last_frames, self._last_rows = None, 0
+    self._last_call = None       # (x, cond, output shape) of the last call: backward() reads them again
     self.n_replicas = 1          # MirroredStrategy replica count (train.py:203); set by parallel.attach()
     self.replica_rank = 0        # this process's replica index: folded into the dropout key (independent masks per replica)
     self._process_group = None   # torch.distributed group (gloo tests / fallback when NCCL cannot be loaded)
@@ -327,11 +328,38 @@ class WaveNet:
     B, T = x2.shape
     cout = 3 * self.num_mixtures if self.num_mixtures is not None else 2 ** self.bits
     out = torch.empty((B, T, cout), dtype=torch.float32, device=dev)
+    self._last_call = None
     # training=True: Keras runs the blocks' Dropout layers (layers.py:195-196) — fresh masks per call
     _lib.check(h.lib.wn_forward_ex(h.h, h.ptr(x2), h.ptr(cond), B, T, 1 if training else 0, h.ptr(out), h.stream_ptr()))
+    self._last_call = (x2, cond, (B, T, cout))
     return out
 
   __call__ = call
+
+  def backward(self, dpred):
+    """Gradients of the last `call` for a loss the caller computes on its output (tf.GradientTape over model(inputs),
+    then tape.gradient(loss, model.trainable_variables)).  `dpred` (B, T, C) = d loss / d pred, pred being what `call`
+    returned (probabilities or mixture parameters).  The gradients land in `get_grads()` / `handle.flat_grads` as after
+    `train_step`: clipped per replica when the optimizer has clipnorm, then summed over the replicas, ready for
+    `optimizer.apply_gradients(model)`; no L2 term (model.py:331-334 belongs to train_step, not to call).  Returns
+    d loss / d cond ((B, cond_in) tensor), or None without conditioning.  Anything that changes the weights, the
+    activations or the dropout masks (train_step, generate, set_weights, optimizer.apply_gradients, ...) between the
+    call and this one makes it raise."""
+    last = self._last_call
+    if last is None:
+      raise RuntimeError('backward needs a preceding call on this model')
+    x2, cond, shape = last
+    h = self.handle
+    dpred = as_dev(dpred, h.device)
+    if tuple(dpred.shape) != shape:
+      raise ValueError(f'dpred must have the shape {shape} of the last call output, got {tuple(dpred.shape)}')
+    if dpred.data_ptr() % 16:
+      dpred = dpred.clone()
+    dcond = torch.empty((shape[0], int(cond.shape[-1])), dtype=torch.float32, device=h.device) if cond is not None else None
+    _lib.check(h.lib.wn_backward(h.h, h.ptr(dpred), h.ptr(dcond), h.stream_ptr()))
+    # the library reduces inside wn_train_step only (wn_comm_fuse_allreduce): here the all-reduce always follows
+    self._reduce_grads(allreduce_done=False)
+    return dcond
 
   # ------------------------------------------------------------------ targets (model.py:151-155)
   def prepare_target(self, x):
@@ -383,17 +411,23 @@ class WaveNet:
         _lib.check(h.lib.wn_comm_fuse_allreduce(h.h, 1 if fuse else 0))
         self._ar_fused = fuse
     _lib.check(fn(h.h, h.ptr(frames), h.ptr(cond), B, T, self.n_replicas, h.ptr(h._loss), h.stream_ptr()))
-    clip = train and self.optimizer is not None and getattr(self.optimizer, 'clipnorm', None)
-    if clip:
-      self.optimizer.clip(self)      # Keras: each replica clips its own gradients, then they are summed
-    if train and self.n_replicas > 1:
-      # MirroredStrategy's gradient all-reduce (SUM: the loss is already divided by the global batch, model.py:328)
+    if train:
+      # (fused: wn_train_step enqueued the all-reduce behind the backward pass, inside the step graph)
+      self._reduce_grads(allreduce_done=self._ar_fused)
+    return h._loss[:2]
+
+  def _reduce_grads(self, allreduce_done: bool):
+    """What follows the gradients of one replica: per-replica clipnorm (Keras clips on every replica before the sum), then
+    MirroredStrategy's gradient all-reduce (SUM: the loss is already divided by the global batch, model.py:328)."""
+    h = self.handle
+    if self.optimizer is not None and getattr(self.optimizer, 'clipnorm', None):
+      self.optimizer.clip(self)
+    if self.n_replicas > 1:
       if self._comm is not None:
-        if not self._ar_fused:       # (fused: wn_train_step enqueued it behind the backward pass, inside the step graph)
+        if not allreduce_done:
           _lib.check(h.lib.wn_allreduce_grads(h.h, h.stream_ptr()))
       elif self._process_group is not None:
         torch.distributed.all_reduce(h.flat_grads, op=torch.distributed.ReduceOp.SUM, group=self._process_group)
-    return h._loss[:2]
 
   def train_step(self, data):
     """Forward + loss + backward; gradients land in `get_grads()` / `handle.flat_grads`.
