@@ -156,6 +156,40 @@ def test_saturated_categorical_loss_three_way():
     assert abs(num - g[pname][idx]) <= 1e-4 * max(1.0, abs(num)) + 5e-3 * abs(num), (pname, num, g[pname][idx])
 
 
+@pytest.mark.parametrize('bits', [1, 16])
+@pytest.mark.parametrize('clipped', [False, True])
+def test_categorical_loss_and_dlogits_at_extreme_class_counts(bits, clipped):
+  """loss_and_dlogits at 2 and 65,536 classes (the GPU class-count tests rest on it there) against torch autograd of the torch
+  restatement, with the Keras 3 clip inactive, or active on part of the targets and on many entries per row."""
+  import torch
+  C = 2 ** bits
+  cfg = oracle_config(dict(channels=8, blocks=1, final_layers_channels=[], dilation_bound=2, bits=bits), 0)
+  rng = np.random.default_rng(bits)
+  B, T = 2, 12
+  y = rng.uniform(-1, 1, (B, T, 1))
+  idx = wo.discretize(y[..., 0], bits)
+  logits = rng.standard_normal((B, T, C)) * (30.0 if clipped else 0.3)
+  if clipped:       # every other row: the target at the row's maximum, so that some targets stay un-clipped
+    rows = np.arange(T) % 2 == 0
+    top = logits.max(-1)
+    np.put_along_axis(logits, idx[..., None], np.where(rows, top, np.take_along_axis(logits, idx[..., None], -1)[..., 0])[..., None], -1)
+  loss, d = wo.loss_and_dlogits(cfg, logits, y, 0.5)
+  lt = torch.tensor(logits, requires_grad=True)
+  loss_t = tr.loss_per_sample(cfg, lt, torch.tensor(y))
+  (loss_t.sum() * 0.5).backward()
+  pr = np.exp(logits - logits.max(-1, keepdims=True))
+  pr /= pr.sum(-1, keepdims=True)
+  p_y = np.take_along_axis(pr, idx[..., None], -1)[..., 0]
+  out = (pr < 1e-7) | (pr > 1 - 1e-7)
+  if clipped:
+    in_y = (p_y >= 1e-7) & (p_y <= 1 - 1e-7)
+    assert out.sum(-1).max() >= C // 2 and in_y.any() and not in_y.all()    # clipped and un-clipped targets both present
+  else:
+    assert not out.any()
+  assert rel_err(loss, loss_t.detach().numpy()) < 1e-12
+  assert rel_err(d, lt.grad.numpy()) < 1e-10
+
+
 def test_replica_scaling():
   # compute_average_loss divides by B*replicas: two replicas' grads SUM to the 1-replica grads
   kw = SMALL_MODELS['categorical_multidil']

@@ -674,6 +674,15 @@ __device__ __forceinline__ float wn_ce_clip_grad(const WnCeClip& cc, float p, bo
   return p * ((in ? cc.S_inv : 0.0f) - (is_target ? cc.y_coef : 0.0f) - cc.dot);
 }
 
+// Row access of the generic softmax kernels below.  C = 2^bits is a multiple of 4 except at C = 2 (1-bit audio), where a float4
+// would take the next row's two values (and be 8-byte aligned on odd rows).  There the row is read element by element into a float4
+// whose missing lanes hold `pad`: -inf for logits (p = 0, nothing added to the max, the sum or dot) and 0 for dp; the loops skip
+// those lanes for the clip sums and the stores.  For C >= 4 this is the plain float4 load.
+__device__ __forceinline__ float4 wn_row_ld4(const float* __restrict__ p, int c, int C, float pad) {
+  if (C >= 4) return *reinterpret_cast<const float4*>(p + c);
+  return make_float4(p[c], c + 1 < C ? p[c + 1] : pad, c + 2 < C ? p[c + 2] : pad, pad);
+}
+
 // ------------------------------------------------------------------ softmax-256 cross entropy (model.py:114-118,516)
 // One warp per row.  logits fp32 [rows][C]; the target index is quantised on the fly from
 // frames[b][t+1] (model.py:319-320).  Writes per-block loss partials, dlogits (= scale *
@@ -690,13 +699,13 @@ __global__ void __launch_bounds__(256) softmax_ce_kernel(const float* __restrict
     const float* lp = logits + row * C;
     float m = -INFINITY;
     for (int c = lane * 4; c < C; c += 128) {
-      const float4 v = *reinterpret_cast<const float4*>(lp + c);
+      const float4 v = wn_row_ld4(lp, c, C, -INFINITY);
       m = fmaxf(m, fmaxf(fmaxf(v.x, v.y), fmaxf(v.z, v.w)));
     }
     m = warp_max(m);
     float s = 0.f;
     for (int c = lane * 4; c < C; c += 128) {
-      const float4 v = *reinterpret_cast<const float4*>(lp + c);
+      const float4 v = wn_row_ld4(lp, c, C, -INFINITY);
       s += expf(v.x - m) + expf(v.y - m) + expf(v.z - m) + expf(v.w - m);
     }
     s = warp_sum(s);
@@ -706,10 +715,11 @@ __global__ void __launch_bounds__(256) softmax_ce_kernel(const float* __restrict
     float delta = 0.f, pm = 0.f;
     bool any_out = false;
     for (int c = lane * 4; c < C; c += 128) {
-      const float4 v = *reinterpret_cast<const float4*>(lp + c);
+      const float4 v = wn_row_ld4(lp, c, C, -INFINITY);
       const float p[4] = {expf(v.x - m) * inv, expf(v.y - m) * inv, expf(v.z - m) * inv, expf(v.w - m) * inv};
 #pragma unroll
       for (int i = 0; i < 4; ++i) {
+        if (c + i >= C) break;
         const bool in = p[i] >= WN_CE_EPS && p[i] <= 1.0f - WN_CE_EPS;
         any_out |= !in;
         delta += fminf(fmaxf(p[i], WN_CE_EPS), 1.0f - WN_CE_EPS) - p[i];
@@ -731,13 +741,16 @@ __global__ void __launch_bounds__(256) softmax_ce_kernel(const float* __restrict
       wn_ce_clip(cc, delta, pm, 0.5f, 0.f);
     }
     for (int c = lane * 4; c < C; c += 128) {
-      const float4 v = *reinterpret_cast<const float4*>(lp + c);
+      const float4 v = wn_row_ld4(lp, c, C, -INFINITY);
       float p[4] = {expf(v.x - m) * inv, expf(v.y - m) * inv, expf(v.z - m) * inv, expf(v.w - m) * inv};
-      if (probs) *reinterpret_cast<float4*>(probs + row * C + c) = make_float4(p[0], p[1], p[2], p[3]);
+      if (probs) {
+        if (C >= 4) *reinterpret_cast<float4*>(probs + row * C + c) = make_float4(p[0], p[1], p[2], p[3]);
+        else for (int i = 0; i < 4 && c + i < C; ++i) probs[row * C + c + i] = p[i];
+      }
       if (dlogits) {
 #pragma unroll
         for (int i = 0; i < 4; ++i)
-          dlogits[row * ldd + c + i] = from_f<TD>((clipped ? wn_ce_clip_grad(cc, p[i], c + i == idx) : p[i] - (c + i == idx ? 1.0f : 0.0f)) * scale);
+          if (c + i < C) dlogits[row * ldd + c + i] = from_f<TD>((clipped ? wn_ce_clip_grad(cc, p[i], c + i == idx) : p[i] - (c + i == idx ? 1.0f : 0.0f)) * scale);
       }
     }
   }
@@ -861,31 +874,31 @@ __global__ void __launch_bounds__(256) softmax_vjp_kernel(const float* __restric
   const float* gp = dp + row * C;
   float m = -INFINITY;
   for (int c = lane * 4; c < C; c += 128) {
-    const float4 v = *reinterpret_cast<const float4*>(lp + c);
+    const float4 v = wn_row_ld4(lp, c, C, -INFINITY);
     m = fmaxf(m, fmaxf(fmaxf(v.x, v.y), fmaxf(v.z, v.w)));
   }
   m = warp_max(m);
   float s = 0.f;
   for (int c = lane * 4; c < C; c += 128) {
-    const float4 v = *reinterpret_cast<const float4*>(lp + c);
+    const float4 v = wn_row_ld4(lp, c, C, -INFINITY);
     s += expf(v.x - m) + expf(v.y - m) + expf(v.z - m) + expf(v.w - m);
   }
   s = warp_sum(s);
   const float inv = 1.0f / s;
   float dot = 0.f;
   for (int c = lane * 4; c < C; c += 128) {
-    const float4 v = *reinterpret_cast<const float4*>(lp + c);
-    const float4 g = *reinterpret_cast<const float4*>(gp + c);
+    const float4 v = wn_row_ld4(lp, c, C, -INFINITY);
+    const float4 g = wn_row_ld4(gp, c, C, 0.f);
     dot += expf(v.x - m) * inv * g.x + expf(v.y - m) * inv * g.y + expf(v.z - m) * inv * g.z + expf(v.w - m) * inv * g.w;
   }
   dot = warp_sum(dot);
   for (int c = lane * 4; c < C; c += 128) {
-    const float4 v = *reinterpret_cast<const float4*>(lp + c);
-    const float4 g = *reinterpret_cast<const float4*>(gp + c);
+    const float4 v = wn_row_ld4(lp, c, C, -INFINITY);
+    const float4 g = wn_row_ld4(gp, c, C, 0.f);
     const float p[4] = {expf(v.x - m) * inv, expf(v.y - m) * inv, expf(v.z - m) * inv, expf(v.w - m) * inv};
     const float gv[4] = {g.x, g.y, g.z, g.w};
 #pragma unroll
-    for (int i = 0; i < 4; ++i) dlogits[row * ldd + c + i] = from_f<TD>(p[i] * (gv[i] - dot));
+    for (int i = 0; i < 4; ++i) if (c + i < C) dlogits[row * ldd + c + i] = from_f<TD>(p[i] * (gv[i] - dot));
   }
   for (int c = C + lane; c < ldd; c += 32) dlogits[row * ldd + c] = from_f<TD>(0.f);
 }
