@@ -343,6 +343,26 @@ static int new_plan(wn_handle* h, cudaStream_t st, std::vector<Plan>& plans, con
   return WN_ERR_CUDA;
 }
 
+// the kept plan whose key matches (at most one does), else a new one
+template <class Plan, class Match, class Build>
+static int plan_for(wn_handle* h, cudaStream_t st, std::vector<Plan>& plans, Match match, const char* what, Build build, Plan** out) {
+  for (auto& q : plans) if (match(q)) { *out = &q; return WN_OK; }
+  return new_plan(h, st, plans, Plan{}, what, build, out);
+}
+// the persistent launches return -100 for a shape they do not take: nothing ran, so the launch is not counted.  *ran: it ran
+template <class Launch>
+static int launch_persistent(wn_handle* h, cudaStream_t st, const char* label, const char* what, Launch launch, bool* ran) {
+  LaunchLabel lab(h, label);
+  LaunchScope ls(h, st, CLS_DILATED);
+  const int r = launch();
+  *ran = r == 0;
+  if (r == -100) h->launches--;
+  else if (r != 0) { set_err("%s launch failed (%d): %s", what, r, tc_last_error()); return WN_ERR_CUDA; }
+  return WN_OK;
+}
+// a persistent stack launch is free of deadlock only while a layer has more 256-row tiles than the GPU has CTA pairs (DESIGN.md §5)
+static bool more_tiles_than_pairs(int B, int Tn) { return B * cdiv(Tn, 256) > tc_num_sms() / 2; }
+
 // ============================================================================ build
 static int add_param(wn_handle* h, const std::string& name, std::initializer_list<int> shape) {
   ParamInfo p;
@@ -1170,26 +1190,25 @@ static bool mapping_args(wn_handle* h, const float* cond_in, int B, float l2coef
   a->d0 = h->dcond; a->d1 = h->cond_dact; a->d2 = h->cond_dact2;
   return true;
 }
-static int cond_forward(wn_handle* h, cudaStream_t st, const float* cond_in, int B, bool run_mapping, const float** cond_out) {
-  const float* cur = cond_in;
-  int width = h->cfg.cond_in;
+// the mapping MLP's output (cond_in itself without mapping layers)
+static const float* cond_forward(wn_handle* h, cudaStream_t st, const float* cond_in, int B) {
   MapArgs ma;
-  if (run_mapping && mapping_args(h, cond_in, B, 0.f, &ma)) {
+  if (mapping_args(h, cond_in, B, 0.f, &ma)) {
     LaunchScope ls(h, st, CLS_MISC);
     mapping_fwd_fused<<<1, 256, 0, st>>>(ma);
-    cur = h->cond_act[ma.n_layers - 1];
-  } else if (run_mapping) {
-    for (size_t i = 0; i < h->map_w.size(); ++i) {
-      LaunchScope ls(h, st, CLS_MISC);
-      const int n = h->map_width[i];
-      dense_small_fwd<<<cdiv(B * n, 128), 128, 0, st>>>(cur, width, P_(h, h->map_w[i]), P_(h, h->map_b[i]), h->cond_act[i], n, B, width, n,
-                                                      h->cfg.mapping_activation);
-      cur = h->cond_act[i];
-      width = n;
-    }
+    return h->cond_act[ma.n_layers - 1];
   }
-  *cond_out = cur;
-  return WN_OK;
+  const float* cur = cond_in;
+  int width = h->cfg.cond_in;
+  for (size_t i = 0; i < h->map_w.size(); ++i) {
+    LaunchScope ls(h, st, CLS_MISC);
+    const int n = h->map_width[i];
+    dense_small_fwd<<<cdiv(B * n, 128), 128, 0, st>>>(cur, width, P_(h, h->map_w[i]), P_(h, h->map_b[i]), h->cond_act[i], n, B, width, n,
+                                                    h->cfg.mapping_activation);
+    cur = h->cond_act[i];
+    width = n;
+  }
+  return cur;
 }
 static void cond_bias_block(wn_handle* h, cudaStream_t st, int l, const float* cond, int B) {
   const BlockP& b = h->blocks[l];
@@ -1198,6 +1217,46 @@ static void cond_bias_block(wn_handle* h, cudaStream_t st, int l, const float* c
   dense_small_fwd<<<cdiv(B * n, 128), 128, 0, st>>>(cond, h->Cc, P_(h, b.cw_idx), P_(h, b.cb_idx), h->cb + (size_t)l * h->maxB * n, n, B, h->Cc, n,
                                                   ACT_LINEAR);
 }
+// ---- conditioning of the whole model: the mapping MLP, then cb of every block; h->last_cond: the mapped conditioning (null without)
+static void model_cond_forward(wn_handle* h, cudaStream_t st, const float* cond_in, int B) {
+  h->last_cond = nullptr;
+  if (!h->cfg.conditioning) return;
+  OuterLabel ol(h, "cond_fwd");
+  h->last_cond = cond_forward(h, st, cond_in, B);
+  LaunchScope ls(h, st, CLS_MISC);
+  const int n = 2 * h->D;
+  cond_bias_all<<<dim3(cdiv(B * n, 128), h->L), 128, 0, st>>>(h->last_cond, h->Cc, h->d_params, h->d_cond_offsets, h->cb, (long long)h->maxB * n, B, n);
+}
+
+// the conv part of a fused-kernel desc (gemm_tc_block.cuh, gemm_tc_stack.cuh): conv cv over A (row width lda), writing xout
+static TcBlockDesc conv_desc(wn_handle* h, const ConvP& cv, const void* A, int lda, void* xout, int B, int Tn) {
+  TcBlockDesc d{};
+  d.B = B; d.T = Tn; d.nseg = cv.K; d.Cin = cv.cin; d.D = h->D; d.R = h->R; d.has_res = 1;
+  for (int k = 0; k < cv.K; ++k) d.shift[k] = -(cv.K - 1 - k) * cv.dil;
+  d.A = (const bf16*)A; d.lda = lda; d.xout = (bf16*)xout;
+  d.W1 = cv.Wf16; d.k1 = cv.Kf16; d.bias_g = P_(h, cv.b_idx);
+  return d;
+}
+// block l's gated conv over A + gate + conv1 + residual x_in as one fused-kernel desc
+static TcBlockDesc block_desc(wn_handle* h, int l, const void* A, int lda, const void* x_in, bool has_cb, int B, int Tn) {
+  const BlockP& b = h->blocks[l];
+  TcBlockDesc d = conv_desc(h, b.stack.back(), A, lda, h->xout[l], B, Tn);
+  d.X = (const bf16*)x_in; d.ldx = h->R; d.W2 = b.Wres16;
+  d.z = (bf16*)h->zbuf[l]; d.g = (bf16*)h->G_all + (size_t)l * h->maxB * h->maxT * h->D;
+  d.cbias = has_cb ? h->cb + (size_t)l * h->maxB * 2 * h->D : nullptr;
+  d.bias_r = P_(h, b.conv1.b_idx);
+  return d;
+}
+
+// training-mode dropout on block l's conv branch only: xdrop[l]; the residual still reads x_in (layers.py:192-196)
+template <class T>
+static const void* dropout_conv_input(wn_handle* h, cudaStream_t st, int l, const void* x_in, int B, int Tn) {
+  LaunchScope ls(h, st, CLS_MISC);
+  const long long n = (long long)B * Tn * h->R;
+  dropout_apply<T><<<cdiv(n, 256), 256, 0, st>>>((const T*)x_in, h->drop_mask + (size_t)l * h->maxB * h->maxT * h->R, (T*)h->xdrop[l], n,
+                                                1.0f / (1.0f - h->cfg.dropout));
+  return h->xdrop[l];
+}
 
 // WaveNetLayer.call for block l (layers.py:178-224); x_in (B,T,R) in T
 template <class T>
@@ -1205,16 +1264,8 @@ static int block_forward(wn_handle* h, cudaStream_t st, int l, const void* x_in,
   BlockP& b = h->blocks[l];
   const int depth = (int)b.stack.size();
   const size_t rows_cap = (size_t)h->maxB * h->maxT;
-  const void* cur = x_in;
+  const void* cur = h->drop_active ? dropout_conv_input<T>(h, st, l, x_in, B, Tn) : x_in;
   int curw = h->R;
-  if (h->drop_active) {
-    // training-mode dropout on the conv branch only; the residual below still reads x_in (layers.py:192-196)
-    LaunchScope ls(h, st, CLS_MISC);
-    const long long n = (long long)B * Tn * h->R;
-    dropout_apply<T><<<cdiv(n, 256), 256, 0, st>>>((const T*)x_in, h->drop_mask + (size_t)l * rows_cap * h->R, (T*)h->xdrop[l], n,
-                                                  1.0f / (1.0f - h->cfg.dropout));
-    cur = h->xdrop[l];
-  }
   for (int j = 0; j < depth; ++j) {
     const ConvP& c = b.stack[j];
     GemmH g;
@@ -1233,23 +1284,10 @@ static int block_forward(wn_handle* h, cudaStream_t st, int l, const void* x_in,
       if constexpr (sizeof(T) == 2) {
         // bf16 tier: gated conv + gate + conv1 (+ residual) as ONE kernel when the shapes allow (gemm_tc_block.cuh)
         if (b.Wres16 && h->cfg.use_residual && c.K <= TC_MAX_TAPS && !h->cond_seq) {
-          TcBlockDesc d{};
-          d.B = B; d.T = Tn; d.nseg = c.K; d.Cin = c.cin; d.D = h->D; d.R = h->R; d.has_res = 1;
-          for (int k = 0; k < c.K; ++k) d.shift[k] = -(c.K - 1 - k) * c.dil;
-          d.A = (const bf16*)cur; d.lda = curw; d.X = (const bf16*)x_in; d.ldx = h->R;
-          d.W1 = c.Wf16; d.k1 = c.Kf16; d.W2 = b.Wres16;
-          d.z = (bf16*)h->zbuf[l]; d.g = (bf16*)h->G_all + (size_t)l * rows_cap * h->D; d.xout = (bf16*)h->xout[l];
-          d.bias_g = P_(h, c.b_idx); d.cbias = has_cb ? h->cb + (size_t)l * h->maxB * 2 * h->D : nullptr;
-          d.bias_r = P_(h, b.conv1.b_idx);
-          int r;
-          {
-            LaunchLabel lab(h, "block_fwd");
-            LaunchScope ls(h, st, CLS_DILATED);
-            r = c.tileN16 == 256 ? tc_block_fwd(h->tmaps, st, d) : -100;
-          }
-          if (r == 0) { h->fused_fwd_launches++; return WN_OK; }
-          if (r != -100) { set_err("fused block forward launch failed (%d): %s", r, tc_last_error()); return WN_ERR_CUDA; }
-          h->launches--;      // not launched: fall through to the separate kernels
+          const TcBlockDesc d = block_desc(h, l, cur, curw, x_in, has_cb, B, Tn);
+          bool ran;
+          RET(launch_persistent(h, st, "block_fwd", "fused block forward", [&] { return c.tileN16 == 256 ? tc_block_fwd(h->tmaps, st, d) : -100; }, &ran));
+          if (ran) { h->fused_fwd_launches++; return WN_OK; }      // else: the separate kernels below
         }
       }
       typename EpiGate<T, sizeof(T) == 2>::Params ep{};
@@ -1310,116 +1348,79 @@ static int skip_gemm(wn_handle* h, cudaStream_t st, int l0, int nl, TO* out, int
   return run_conv_gemm<T, EpiBiasActRes<T, TO, sizeof(T) == 2>>(h, st, CLS_GEMM, g, ep);
 }
 
-// WaveNet.call up to the logits (model.py:213-239).  x (B,T) fp32 with row stride ldx.
+// ---- input conv (model.py:84-88) into h0.  HBM-bound, small CTAs
 template <class T>
-static int model_forward(wn_handle* h, cudaStream_t st, const float* x, int ldx, const float* cond_in, int B, int Tn) {
+static void input_conv_forward(wn_handle* h, cudaStream_t st, const float* x, int ldx, int B, int Tn) {
+  OuterLabel ol(h, "input_conv_fwd");
+  LaunchScope ls(h, st, CLS_MISC);
+  const long long total = (long long)B * Tn * h->R;
+  if (h->R % 8 == 0 && h->R / 8 <= 256)
+    input_conv_fwd_rows<T><<<cdiv((long long)B * Tn, ICF_ROWS), 256, 0, st>>>(x, ldx, P_(h, h->input_conv.w_idx), P_(h, h->input_conv.b_idx), (T*)h->h0, B, Tn, h->R, h->K);
+  else if (h->R % 8 == 0)
+    input_conv_fwd_vec8<T><<<cdiv(total / 8, 256), 256, 0, st>>>(x, ldx, P_(h, h->input_conv.w_idx), P_(h, h->input_conv.b_idx), (T*)h->h0, B, Tn, h->R, h->K);
+  else
+    input_conv_fwd<T><<<cdiv(total, 256), 256, 0, st>>>(x, ldx, P_(h, h->input_conv.w_idx), P_(h, h->input_conv.b_idx), (T*)h->h0, B, Tn, h->R, h->K);
+}
+
+// The whole residual stack runs as ONE persistent launch (gemm_tc_stack.cuh) when every block takes the fused forward and a
+// layer has more 256-row tiles than the GPU has CTA pairs.  Multi-dilation blocks (layers.py:64-88): every conv in front of the
+// gated conv is a PLAIN layer of the same launch (its output is kept for the backward pass, as before).
+static bool stack_forward_ok(wn_handle* h, int B, int Tn) {
+  bool ok = h->use_stack_fwd && h->cfg.use_residual && h->L >= 2 && h->D == h->R && (h->D == 256 || h->D == 128) && more_tiles_than_pairs(B, Tn);
+  for (auto& b : h->blocks) {
+    if (!ok) break;
+    const ConvP& cv = b.stack.back();
+    ok = b.Wres16 != nullptr && cv.tileN16 == 256 && cv.K <= TC_MAX_TAPS && cv.cin % 64 == 0;
+    for (size_t j = 0; ok && j + 1 < b.stack.size(); ++j) {
+      const ConvP& pc = b.stack[j];
+      // plain layers run as one 256-wide tile per m tile: D = 256 only; all convs share K and the input width
+      ok = h->D == 256 && pc.cout == h->D && pc.cin == cv.cin && pc.K == cv.K && pc.Wf16 != nullptr && pc.N16 == 256 && b.stack.size() <= 16;
+    }
+  }
+  return ok;
+}
+
+// ---- every block's convs, gate, conv1 and residual as one persistent launch; *stacked: it ran (else the per-block loop runs them)
+static int stack_forward(wn_handle* h, cudaStream_t st, int B, int Tn, bool* stacked) {
   const wn_config& c = h->cfg;
-  h->fused_fwd_launches = 0;
-  const float* cond = nullptr;
-  if (c.conditioning) {
-    OuterLabel ol(h, "cond_fwd");
-    RET(cond_forward(h, st, cond_in, B, true, &cond));
-    {
-      LaunchScope ls(h, st, CLS_MISC);
-      const int n = 2 * h->D;
-      cond_bias_all<<<dim3(cdiv(B * n, 128), h->L), 128, 0, st>>>(cond, h->Cc, h->d_params, h->d_cond_offsets, h->cb, (long long)h->maxB * n, B, n);
-    }
-  }
-  h->last_cond = cond;
-  {
-    OuterLabel ol(h, "input_conv_fwd");
-    LaunchScope ls(h, st, CLS_MISC);
-    const long long total = (long long)B * Tn * h->R;
-    if (h->R % 8 == 0 && h->R / 8 <= 256)
-      input_conv_fwd_rows<T><<<cdiv((long long)B * Tn, ICF_ROWS), 256, 0, st>>>(x, ldx, P_(h, h->input_conv.w_idx), P_(h, h->input_conv.b_idx), (T*)h->h0, B, Tn, h->R, h->K);
-    else if (h->R % 8 == 0)
-      input_conv_fwd_vec8<T><<<cdiv(total / 8, 256), 256, 0, st>>>(x, ldx, P_(h, h->input_conv.w_idx), P_(h, h->input_conv.b_idx), (T*)h->h0, B, Tn, h->R, h->K);
-    else
-      input_conv_fwd<T><<<cdiv(total, 256), 256, 0, st>>>(x, ldx, P_(h, h->input_conv.w_idx), P_(h, h->input_conv.b_idx), (T*)h->h0, B, Tn, h->R, h->K);
-  }
-  const void* cur = h->h0;
-  bool stacked = false;
-  h->stack_fwd_layers = 0;
-  if constexpr (sizeof(T) == 2) {
-    // the whole residual stack as ONE persistent launch (gemm_tc_stack.cuh) when every block takes the fused forward
-    // and a layer has more 256-row tiles than the GPU has CTA pairs.  Multi-dilation blocks (layers.py:64-88): every conv in
-    // front of the gated conv is a PLAIN layer of the same launch (its output is kept for the backward pass, as before).
-    bool ok = h->use_stack_fwd && c.use_residual && h->L >= 2 && h->D == h->R &&
-              (h->D == 256 || h->D == 128) && B * cdiv(Tn, 256) > tc_num_sms() / 2;
-    for (auto& b : h->blocks) {
-      if (!ok) break;
-      const ConvP& cv = b.stack.back();
-      ok = b.Wres16 != nullptr && cv.tileN16 == 256 && cv.K <= TC_MAX_TAPS && cv.cin % 64 == 0;
-      for (size_t j = 0; ok && j + 1 < b.stack.size(); ++j) {
-        const ConvP& pc = b.stack[j];
-        // plain layers run as one 256-wide tile per m tile: D = 256 only; all convs share K and the input width
-        ok = h->D == 256 && pc.cout == h->D && pc.cin == cv.cin && pc.K == cv.K && pc.Wf16 != nullptr && pc.N16 == 256 && b.stack.size() <= 16;
-      }
-    }
-    if (ok) {
-      const size_t rows_cap = (size_t)h->maxB * h->maxT;
-      const bool has_cb = c.conditioning != 0;
-      // one desc per CONV: the plain convs of block l, then its gated conv + tail
-      auto build_descs = [&](std::vector<TcBlockDesc>& descs) {
-        descs.clear();
-        for (int l = 0; l < h->L; ++l) {
-          BlockP& b = h->blocks[l];
-          const void* x_in = l > 0 ? h->xout[l - 1] : h->h0;
-          // training-mode dropout without leaving the launch: the conv branch of block l reads xdrop[l] = keep_l * x / (1 - rate),
-          // written by the OUT epilogue of block l-1 next to x_out (block 0: by dropout_apply on h0 below); the residual reads x
-          const void* cur = h->drop_active ? (const void*)h->xdrop[l] : x_in;
-          const int depth = (int)b.stack.size();
-          for (int j = 0; j < depth; ++j) {
-            const ConvP& cv = b.stack[j];
-            TcBlockDesc d{};
-            d.B = B; d.T = Tn; d.nseg = cv.K; d.Cin = cv.cin; d.D = h->D; d.R = h->R; d.has_res = 1;
-            for (int k = 0; k < cv.K; ++k) d.shift[k] = -(cv.K - 1 - k) * cv.dil;
-            d.A = (const bf16*)cur; d.lda = j == 0 ? h->R : h->D;
-            d.W1 = cv.Wf16; d.k1 = cv.Kf16;
-            d.bias_g = P_(h, cv.b_idx);
-            if (h->drop_active) d.drop_scale = 1.0f / (1.0f - c.dropout);
-            if (j < depth - 1) {
-              d.plain = 1; d.act = c.activation;
-              d.xout = (bf16*)h->acts[l][j];
-              cur = h->acts[l][j];
-            } else {
-              d.X = (const bf16*)x_in; d.ldx = h->R; d.W2 = b.Wres16;
-              d.z = (bf16*)h->zbuf[l]; d.g = (bf16*)h->G_all + (size_t)l * rows_cap * h->D; d.xout = (bf16*)h->xout[l];
-              d.cbias = has_cb ? h->cb + (size_t)l * h->maxB * 2 * h->D : nullptr;
-              d.bias_r = P_(h, b.conv1.b_idx);
-              if (h->drop_active && l + 1 < h->L) { d.mask_next = h->drop_mask + (size_t)(l + 1) * rows_cap * h->R; d.xdrop_next = (bf16*)h->xdrop[l + 1]; }
-            }
-            descs.push_back(d);
-          }
-        }
-      };
-      std::vector<TcBlockDesc> descs;
-      build_descs(descs);
-      TcStackPlan* sp = nullptr;
-      for (auto& q : h->stack_plans) if (q.B == B && q.T == Tn && q.cb == has_cb && q.drop == (h->drop_active && h->L > 1)) sp = &q;
-      if (!sp) RET(new_plan(h, st, h->stack_plans, TcStackPlan{}, "stack forward", [&](TcStackPlan& p) { return tc_stack_build(h->tmaps, descs, &p); }, &sp));
-      if (sp && h->drop_active) {
-        // block 0's masked input from the input conv's output (every later block's comes out of the launch itself)
-        LaunchScope ls(h, st, CLS_MISC);
-        const long long n = (long long)B * Tn * h->R;
-        dropout_apply<bf16><<<cdiv(n, 256), 256, 0, st>>>((const bf16*)h->h0, h->drop_mask, (bf16*)h->xdrop[0], n, 1.0f / (1.0f - c.dropout));
-      }
-      if (sp) {
-        LaunchLabel lab(h, "stack_fwd");
-        LaunchScope ls(h, st, CLS_DILATED);
-        const int r = tc_stack_launch(st, *sp, descs[0]);
-        if (r == 0) { stacked = true; h->fused_fwd_launches = h->L; h->stack_fwd_layers = h->L; cur = h->xout[h->L - 1]; }
-        else if (r == -100) h->launches--;
-        else { set_err("stack forward launch failed (%d): %s", r, tc_last_error()); return WN_ERR_CUDA; }
-      }
-    }
-  }
-  if (!stacked)
+  const bool has_cb = c.conditioning != 0;
+  // one desc per CONV: the plain convs of block l, then its gated conv + tail
+  std::vector<TcBlockDesc> descs;
   for (int l = 0; l < h->L; ++l) {
-    RET(block_forward<T>(h, st, l, cur, c.conditioning != 0, B, Tn));
-    cur = h->xout[l];
+    const BlockP& b = h->blocks[l];
+    const void* x_in = l > 0 ? h->xout[l - 1] : h->h0;
+    // training-mode dropout without leaving the launch: the conv branch of block l reads xdrop[l] = keep_l * x / (1 - rate),
+    // written by the OUT epilogue of block l-1 next to x_out (block 0: by dropout_conv_input on h0 below); the residual reads x
+    const void* cur = h->drop_active ? (const void*)h->xdrop[l] : x_in;
+    int lda = h->R;
+    for (size_t j = 0; j + 1 < b.stack.size(); ++j) {
+      TcBlockDesc d = conv_desc(h, b.stack[j], cur, lda, h->acts[l][j], B, Tn);
+      d.plain = 1; d.act = c.activation;
+      descs.push_back(d);
+      cur = h->acts[l][j];
+      lda = h->D;
+    }
+    TcBlockDesc d = block_desc(h, l, cur, lda, x_in, has_cb, B, Tn);
+    if (h->drop_active && l + 1 < h->L) { d.mask_next = h->drop_mask + (size_t)(l + 1) * h->maxB * h->maxT * h->R; d.xdrop_next = (bf16*)h->xdrop[l + 1]; }
+    descs.push_back(d);
   }
-  const void* head_in = cur;
+  if (h->drop_active) for (TcBlockDesc& d : descs) d.drop_scale = 1.0f / (1.0f - c.dropout);
+  TcStackPlan* sp = nullptr;
+  RET(plan_for(h, st, h->stack_plans, [&](const TcStackPlan& q) { return q.B == B && q.T == Tn && q.cb == has_cb && q.drop == (h->drop_active && h->L > 1); },
+               "stack forward", [&](TcStackPlan& p) { return tc_stack_build(h->tmaps, descs, &p); }, &sp));
+  if (!sp) return WN_OK;
+  // block 0's masked input from the input conv's output (every later block's comes out of the launch itself)
+  if (h->drop_active) dropout_conv_input<bf16>(h, st, 0, h->h0, B, Tn);
+  RET(launch_persistent(h, st, "stack_fwd", "stack forward", [&] { return tc_stack_launch(st, *sp, descs[0]); }, stacked));
+  if (*stacked) { h->fused_fwd_launches = h->L; h->stack_fwd_layers = h->L; }
+  return WN_OK;
+}
+
+// ---- skip sum and head convs on the last block's output, into the logits
+template <class T>
+static int head_forward(wn_handle* h, cudaStream_t st, int B, int Tn) {
+  const wn_config& c = h->cfg;
+  const void* head_in = h->xout[h->L - 1];
   int head_w = h->R;
   if (c.use_skip) {
     OuterLabel ol(h, "skip_sum");
@@ -1430,12 +1431,11 @@ static int model_forward(wn_handle* h, cudaStream_t st, const float* x, int ldx,
   OuterLabel ol_head(h, "head_fwd");
   for (size_t i = 0; i < h->head.size(); ++i) {
     const ConvP& hc = h->head[i];
-    const bool last = i + 1 == h->head.size();
     GemmH g;
     g.B = B; g.T = Tn; g.N = hc.cout; g.nseg = 1;
     g.seg[0] = SegH{head_in, head_w, 0, hc.cin};
     fill_w(g, hc, false);
-    if (!last) {
+    if (i + 1 < h->head.size()) {
       typename EpiBiasActRes<T, T, sizeof(T) == 2>::Params ep{};
       ep.out = (T*)h->hact[i]; ep.ldo = hc.cout; ep.bias = P_(h, hc.b_idx); ep.act = c.activation; ep.N = hc.cout; ep.vec = vec_ok<T>(hc.cout);
       RET((run_conv_gemm<T, EpiBiasActRes<T, T, sizeof(T) == 2>>(h, st, CLS_GEMM, g, ep)));
@@ -1448,6 +1448,20 @@ static int model_forward(wn_handle* h, cudaStream_t st, const float* x, int ldx,
     }
   }
   return WN_OK;
+}
+
+// WaveNet.call up to the logits (model.py:213-239).  x (B,T) fp32 with row stride ldx.
+template <class T>
+static int model_forward(wn_handle* h, cudaStream_t st, const float* x, int ldx, const float* cond_in, int B, int Tn) {
+  h->fused_fwd_launches = 0; h->stack_fwd_layers = 0;
+  model_cond_forward(h, st, cond_in, B);
+  input_conv_forward<T>(h, st, x, ldx, B, Tn);
+  bool stacked = false;
+  if constexpr (sizeof(T) == 2) {
+    if (stack_forward_ok(h, B, Tn)) RET(stack_forward(h, st, B, Tn, &stacked));
+  }
+  for (int l = 0; !stacked && l < h->L; ++l) RET(block_forward<T>(h, st, l, l > 0 ? h->xout[l - 1] : h->h0, h->cfg.conditioning != 0, B, Tn));
+  return head_forward<T>(h, st, B, Tn);
 }
 
 // loss (model.py:505-551) on the logits; optionally dlogits and probabilities
@@ -1856,7 +1870,7 @@ static BwdSchedule bwd_schedule(wn_handle* h, int B, int Tn) {
     // of every block kept (grouped weight gradients), more 256-row tiles per layer than CTA pairs.  It takes every SM for the
     // whole chain, so the weight gradients all run in the one grouped launch behind it (no side launches).
     s.sb = s.group && !s.cat && h->use_stack_bwd && h->L >= 2 && h->D == h->R && h->D == 256 &&
-           h->K <= TC_MAX_TAPS && B * cdiv(Tn, 256) > tc_num_sms() / 2;
+           h->K <= TC_MAX_TAPS && more_tiles_than_pairs(B, Tn);
     for (auto& b : h->blocks) {
       if (!s.sb) break;
       // multi-dilation blocks (plain conv layers of the launch): all convs 256 wide
@@ -1869,12 +1883,9 @@ static BwdSchedule bwd_schedule(wn_handle* h, int B, int Tn) {
   // (256 tiles: 4 rounds on 74 or on 64 pairs), and the pairs left over run the weight gradients of every n-th block
   // beside the chain.  The plan (unit ranges per side group) exists from the second call on; the first call launches
   // every group at the end.
-  if (s.group && !s.sb && h->side_stream != nullptr && h->wg_side_every > 0) {
-    const int pairs = tc_num_sms() / 2, tiles = B * cdiv(Tn, 256);
-    if (tiles > pairs) {
-      const int rounds = cdiv(tiles, pairs);
-      s.side_pairs = pairs - cdiv(tiles, rounds);
-    }
+  if (s.group && !s.sb && h->side_stream != nullptr && h->wg_side_every > 0 && more_tiles_than_pairs(B, Tn)) {
+    const int pairs = tc_num_sms() / 2, tiles = B * cdiv(Tn, 256), rounds = cdiv(tiles, pairs);
+    s.side_pairs = pairs - cdiv(tiles, rounds);
     if (s.side_pairs < 6) s.side_pairs = 0;
   }
   // bucketed all-reduce: only with the stack-backward launch (every SM busy until the chain ends, all filter gradients in the
@@ -2010,15 +2021,11 @@ static int stack_backward(wn_handle* h, cudaStream_t st, int B, int Tn, const vo
     }
   }
   TcStackBwdPlan* sp = nullptr;
-  for (auto& q : h->stack_bwd_plans) if (q.B == B && q.T == Tn && q.drop == h->drop_active) sp = &q;
-  if (!sp) RET(new_plan(h, st, h->stack_bwd_plans, TcStackBwdPlan{}, "stack backward", [&](TcStackBwdPlan& p) { return tc_stack_bwd_build(h->tmaps, bdescs, &p); }, &sp));
+  RET(plan_for(h, st, h->stack_bwd_plans, [&](const TcStackBwdPlan& q) { return q.B == B && q.T == Tn && q.drop == h->drop_active; },
+               "stack backward", [&](TcStackBwdPlan& p) { return tc_stack_bwd_build(h->tmaps, bdescs, &p); }, &sp));
   if (!sp) return WN_OK;
-  LaunchLabel lab(h, "stack_bwd");
-  LaunchScope ls(h, st, CLS_DILATED);
-  const int r = tc_stack_bwd_launch(st, *sp, bdescs[0]);
-  if (r == 0) { *stacked = true; h->stack_bwd_layers = h->L; }
-  else if (r == -100) h->launches--;
-  else { set_err("stack backward launch failed (%d): %s", r, tc_last_error()); return WN_ERR_CUDA; }
+  RET(launch_persistent(h, st, "stack_bwd", "stack backward", [&] { return tc_stack_bwd_launch(st, *sp, bdescs[0]); }, stacked));
+  if (*stacked) h->stack_bwd_layers = h->L;
   return WN_OK;
 }
 
@@ -2348,7 +2355,6 @@ extern "C" int wn_generate(wn_handle* h, const float* prime_dev, int n_prime, co
   wn_handle::Gen& G = h->gen;
   CK(cudaEventRecord(h->ev_in, user)); CK(cudaStreamWaitEvent(st, h->ev_in, 0));
   // state: zero histories are the causal padding (nothing before the prime is ever needed at the last position, model.py:122)
-  for (size_t i = 0; i < G.allocs.size(); ++i) { /* buffers are re-zeroed lazily below */ }
   CK(cudaMemsetAsync(G.audio, 0, (size_t)G.B * G.cap * 4, st));
   for (auto& hl : G.hist) for (float* p : hl) if (p) CK(cudaMemsetAsync(p, 0, (size_t)G.B * G.cap * 4 * ((p == hl[0]) ? h->R : h->D), st));
   CK(cudaMemsetAsync(G.t_dev, 0, 4, st));
@@ -2356,8 +2362,7 @@ extern "C" int wn_generate(wn_handle* h, const float* prime_dev, int n_prime, co
   if (teacher_dev) CK(cudaMemcpy2DAsync(G.audio + n_prime, (size_t)G.cap * 4, teacher_dev, (size_t)length * 4, (size_t)length * 4, B, cudaMemcpyDeviceToDevice, st));
   bool has_cb = false;
   if (h->cfg.conditioning) {
-    const float* cond = nullptr;
-    RET(cond_forward(h, st, cond_dev, B, true, &cond));
+    const float* cond = cond_forward(h, st, cond_dev, B);
     const int n = 2 * h->D;
     cond_bias_all<<<dim3(cdiv(B * n, 128), h->L), 128, 0, st>>>(cond, h->Cc, h->d_params, h->d_cond_offsets, h->cb, (long long)h->maxB * n, B, n);
     has_cb = true;
@@ -2916,17 +2921,12 @@ static int layer_fwd_entry(wn_handle* h, int l, const float* x, const float* con
   h->layer_drop[l] = h->drop_active;
   draw_dropout_masks(h, st, B, Tn, l);
   const long long nR = (long long)B * Tn * h->R;
-  const void* xin;
-  // keep a private copy of the block input (needed by the backward pass)
-  void* slot = l == 0 ? h->layer_in : h->xout[l - 1];
-  if (l > 0 && h->L > 1) {
-    // blocks of a bare stack are chained by the caller; input of block l lives in xout[l-1]
-  }
+  // keep a private copy of the block input (needed by the backward pass); block l > 0 keeps it where the model does, in xout[l-1]
+  void* xin = l == 0 ? h->layer_in : h->xout[l - 1];
   {
     LaunchScope ls(h, st, CLS_MISC);
-    convert_kernel<float, T><<<cdiv(nR, 256), 256, 0, st>>>(x, (T*)slot, nR);
+    convert_kernel<float, T><<<cdiv(nR, 256), 256, 0, st>>>(x, (T*)xin, nR);
   }
-  xin = slot;
   bool has_cb = false;
   h->layer_cseq[l] = nullptr;
   if (seq) {
