@@ -153,7 +153,11 @@ int wn_adam_restore(wn_handle* h, const float* m_dev, const float* v_dev, int64_
 /* ---- dropout (layers.py:109-112,195-196; Keras Dropout on the block input of the conv branch) --------
  * Training passes draw keep-masks with a counter-based Philox-4x32-10 keyed by (seed, step): TF's RNG
  * stream cannot be reproduced, so parity runs inject the masks instead.
- * keep_host: [blocks][B*T*channels] bytes (1 = keep), NULL returns to Philox masks. */
+ * keep_host: [blocks][B*T*channels] bytes (1 = keep), NULL returns to Philox masks.
+ * The masks belong to the (B, T) they were packed for: a training pass at any other shape (wn_train_step,
+ * wn_train_step_host, wn_forward_ex with training != 0, wn_layer_forward_ex / _seq with training != 0) fails with
+ * WN_ERR_STATE until masks of its shape are injected or NULL is passed.  Passes without dropout (inference, test steps)
+ * run at any shape that fits the workspace. */
 int wn_set_dropout_masks(wn_handle* h, const uint8_t* keep_host, int B, int T);
 int wn_set_dropout_seed(wn_handle* h, uint64_t seed);
 

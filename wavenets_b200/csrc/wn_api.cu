@@ -174,6 +174,7 @@ struct wn_handle {
   unsigned long long* d_drop_ctr = nullptr;
   unsigned long long drop_seed = 0x243F6A8885A308D3ull;
   bool drop_injected = false;   // masks were supplied by wn_set_dropout_masks: do not redraw
+  int drop_B = 0, drop_T = 0;   // ... packed for this (B, T), row b*T + t of every slab
   bool drop_active = false;     // the pass being enqueued is a training pass with dropout > 0
   // optimizer state (wn_adam_*): allocated on first use
   float* opt_m = nullptr; float* opt_v = nullptr;
@@ -2568,7 +2569,15 @@ extern "C" int wn_set_dropout_masks(wn_handle* h, const uint8_t* keep_host, int 
   const size_t n = (size_t)B * T * h->R, slab = (size_t)h->maxB * h->maxT * h->R;
   for (int l = 0; l < h->L; ++l) CK(cudaMemcpy(h->drop_mask + l * slab, keep_host + l * n, n, cudaMemcpyHostToDevice));
   h->drop_injected = true;
+  h->drop_B = B; h->drop_T = T;
   return WN_OK;
+}
+// a training pass reads the keep-mask of (b, t) at row b*T + t of its own T: injected masks belong to the shape they were packed for
+static int check_injected_mask_shape(wn_handle* h, int B, int T, bool training) {
+  if (!training || h->cfg.dropout <= 0.f || !h->drop_injected || (B == h->drop_B && T == h->drop_T)) return WN_OK;
+  set_err("dropout masks were injected for (batch, time) = (%d, %d); a training pass at (%d, %d) needs masks of its own shape "
+          "(or none: wn_set_dropout_masks(NULL) returns to Philox masks)", h->drop_B, h->drop_T, B, T);
+  return WN_ERR_STATE;
 }
 extern "C" int wn_set_dropout_seed(wn_handle* h, uint64_t seed) {
   if (!h) { set_err("null handle"); return WN_ERR_VALUE; }
@@ -2621,6 +2630,7 @@ extern "C" int wn_forward_ex(wn_handle* h, const float* x_dev, const float* cond
   if (!h->cfg.has_head || !h->cfg.has_input_conv) { set_err("wn_forward needs a full model handle"); return WN_ERR_STATE; }
   if (h->cfg.conditioning && !cond_dev) { set_err("Conditioning must be provided."); return WN_ERR_VALUE; }
   if (training && h->cfg.dropout >= 1.f) { set_err("dropout must be < 1 for training"); return WN_ERR_VALUE; }
+  RET(check_injected_mask_shape(h, B, T, training != 0));
   CK(cudaSetDevice(h->cfg.device));
   h->launches = 0;
   h->fwd_valid = false;
@@ -2824,6 +2834,7 @@ static int step_common(wn_handle* h, const float* frames_dev, const float* cond_
   if (h->cfg.conditioning && !cond_dev) { set_err("Conditioning must be provided."); return WN_ERR_VALUE; }
   if (n_replicas < 1 || !frames_dev || !loss_dev) { set_err("bad step arguments"); return WN_ERR_VALUE; }
   if (train && h->cfg.dropout >= 1.f) { set_err("dropout must be < 1 for training"); return WN_ERR_VALUE; }
+  RET(check_injected_mask_shape(h, B, T, train));
   CK(cudaSetDevice(h->cfg.device));
   h->fwd_valid = false;
   cudaStream_t st = (cudaStream_t)stream;
@@ -2985,6 +2996,7 @@ extern "C" int wn_layer_forward_ex(wn_handle* h, int block, const float* x_dev, 
   RET(check_bt(h, B, T));
   if (block < 0 || block >= h->L || !x_dev || !x_out_dev) { set_err("bad layer arguments"); return WN_ERR_VALUE; }
   if (training && h->cfg.dropout >= 1.f) { set_err("dropout must be < 1 for training"); return WN_ERR_VALUE; }
+  RET(check_injected_mask_shape(h, B, T, training != 0));
   return layer_forward_call(h, block, x_dev, cond_dev, false, B, T, training, x_out_dev, skip_dev, stream);
 }
 extern "C" int wn_layer_forward_seq(wn_handle* h, int block, const float* x_dev, const float* cond_dev, int B, int T, int training,
@@ -2995,6 +3007,7 @@ extern "C" int wn_layer_forward_seq(wn_handle* h, int block, const float* x_dev,
   if (!h->blocks[block].has_cond) { set_err("block %d was built without conditioning", block); return WN_ERR_VALUE; }
   if (h->Ccs == 0) { set_err("conditioning sequences are built for layer handles (has_head = 0) only"); return WN_ERR_UNSUPPORTED; }
   if (training && h->cfg.dropout >= 1.f) { set_err("dropout must be < 1 for training"); return WN_ERR_VALUE; }
+  RET(check_injected_mask_shape(h, B, T, training != 0));
   return layer_forward_call(h, block, x_dev, cond_dev, true, B, T, training, x_out_dev, skip_dev, stream);
 }
 extern "C" int wn_layer_forward(wn_handle* h, int block, const float* x_dev, const float* cond_dev, int B, int T, float* x_out_dev, float* skip_dev,
