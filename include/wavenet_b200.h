@@ -180,6 +180,15 @@ int wn_forward_ex(wn_handle* h, const float* x_dev, const float* cond_dev, int B
  * WN_ERR_STATE: no wn_forward_ex since the handle's activations, weights or dropout masks last changed (a train/test
  * step, wn_generate, a wn_layer_* forward, wn_set_param / wn_params_changed / wn_adam_step, wn_set_dropout_masks). */
 int wn_backward(wn_handle* h, const float* dpred_dev, float* dcond_dev, void* stream);
+/* wn_backward plus the input gradient, and the choice to skip the parameter gradients (tape.gradient(loss, x) of a frozen
+ * model: distillation through a teacher's input, priors and perceptual losses on audio, saliency).  wn_backward is
+ * wn_backward_ex(h, dpred, dcond, NULL, 1, stream).
+ * dx_dev (B,T) fp32 or NULL receives d loss / d x for the x (B,T) passed to the last wn_forward_ex (row stride T).
+ * param_grads == 0: no parameter gradient is computed and wn_grads_dev() is left untouched, bit for bit; dx and dcond are
+ * the same as with param_grads != 0 (dx bit for bit; dcond up to the fp32 summation order of the conditioning sums).
+ * WN_ERR_VALUE: param_grads == 0 with dx_dev and dcond_dev both NULL (nothing to compute).  The state rules are
+ * wn_backward's; either mode may follow the other after one wn_forward_ex. */
+int wn_backward_ex(wn_handle* h, const float* dpred_dev, float* dcond_dev, float* dx_dev, int param_grads, void* stream);
 
 /* ---- WaveNet.loss_fn(target, pred) (model.py:505-551) on MATERIALISED predictions ------------------------------------
  * pred (B,T,Cout) fp32 = a WaveNet.call output (softmax probabilities, or [weights | means | log-scales] mixture
@@ -290,7 +299,8 @@ int wn_profile_begin(wn_handle* h, int tag);
 int wn_profile_end(wn_handle* h, double* ms, int64_t* launches);
 /* per-launch record of the last wn_profile_end: returns the number of timed launches; fills duration (ms) and a
  * short label of launch i: the phase ("input_conv_fwd", "cond_fwd", "skip_sum", "head_fwd", "loss", "loss_finalize",
- * "head_bwd", "wgrad_group_finish", "input_conv_bwd", "cond_bwd", "pred_vjp" (wn_backward's adjoint of the predictions)) or, inside the block loop, the kernel ("stack_fwd",
+ * "head_bwd", "wgrad_group_finish", "input_conv_bwd", "cond_bwd", "pred_vjp" (wn_backward's adjoint of the predictions),
+ * "input_dgrad" (wn_backward_ex's d loss / d x)) or, inside the block loop, the kernel ("stack_fwd",
  * "block_fwd", "gate", "bias_act_res", "gate_bwd", "dgrad", "wgrad_dilated", "wgrad_1x1", "wgrad_group", "misc") */
 int wn_profile_get(wn_handle* h, int i, double* ms, char* label, int label_len);
 const char* wn_build_info(void);

@@ -194,6 +194,125 @@ __global__ void __launch_bounds__(256) input_conv_bwd_stage1_wide(const float* _
   }
 }
 
+// input conv dgrad, the adjoint of input_conv_fwd onto the 1-channel signal:
+//   dx[b,s] = sum_k [s+(K-1-k) < T] * q_k(b, s+(K-1-k)),   q_k(b,t) = sum_c dh[b,t,c] * W[k,0,c]
+// One CTA = ICD_ROWS positions of one sequence.  Every dh row the CTA needs (its own rows plus the K-1 halo rows after them,
+// cut at the sequence end so the next batch row is never read) is read once, by one warp: each lane holds V channels per
+// 16-byte load (V = 1: the scalar path for widths and strides that are not multiples of 16 bytes) and K partial dot products,
+// then a butterfly shuffle sums the lanes.  Fixed summation order everywhere: bit-reproducible.  dx (B,T) fp32, row stride T.
+#define ICD_ROWS 64
+#define ICD_MAXK 4
+#define ICD_RPW ((ICD_ROWS + ICD_MAXK - 1 + 7) / 8)     // q rows per warp (8 warps)
+template <class T, int V>
+__global__ void __launch_bounds__(256) input_conv_dgrad(const T* __restrict__ dh, int lddh, const float* __restrict__ W, float* __restrict__ dx,
+                                                        int Tn, int R, int K) {
+  __shared__ float q[ICD_MAXK][ICD_ROWS + ICD_MAXK - 1];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int b = blockIdx.y, t0 = blockIdx.x * ICD_ROWS;
+  const int nq = min(ICD_ROWS + K - 1, Tn - t0);
+  const T* base = dh + ((long long)b * Tn + t0) * lddh;
+  float acc[ICD_RPW][ICD_MAXK];
+#pragma unroll
+  for (int i = 0; i < ICD_RPW; ++i)
+#pragma unroll
+    for (int k = 0; k < ICD_MAXK; ++k) acc[i][k] = 0.f;
+  for (int c = lane * V; c < R; c += 32 * V) {
+    float w[ICD_MAXK][V];
+#pragma unroll
+    for (int k = 0; k < ICD_MAXK; ++k)
+#pragma unroll
+      for (int j = 0; j < V; ++j) w[k][j] = k < K ? W[k * R + c + j] : 0.f;
+    // every row's load first (rows past nq read as zero): one memory latency per chunk, not one per row
+    using Vec = std::conditional_t<V == 8, uint4, std::conditional_t<V == 4, float4, T>>;
+    Vec raw[ICD_RPW];
+#pragma unroll
+    for (int i = 0; i < ICD_RPW; ++i) {
+      const int r = warp + 8 * i;
+      if (r < nq) raw[i] = *reinterpret_cast<const Vec*>(base + (long long)r * lddh + c);
+      else raw[i] = Vec{};
+    }
+#pragma unroll
+    for (int i = 0; i < ICD_RPW; ++i) {
+      float d[V];
+      if constexpr (V == 8) {
+        const uint32_t a[4] = {raw[i].x, raw[i].y, raw[i].z, raw[i].w};
+#pragma unroll
+        for (int j = 0; j < 4; ++j) { d[2 * j] = __uint_as_float(a[j] << 16); d[2 * j + 1] = __uint_as_float(a[j] & 0xffff0000u); }
+      } else if constexpr (V == 4) {
+        d[0] = raw[i].x; d[1] = raw[i].y; d[2] = raw[i].z; d[3] = raw[i].w;
+      } else {
+        d[0] = to_f(raw[i]);
+      }
+#pragma unroll
+      for (int k = 0; k < ICD_MAXK; ++k)
+#pragma unroll
+        for (int j = 0; j < V; ++j) acc[i][k] = fmaf(d[j], w[k][j], acc[i][k]);
+    }
+  }
+#pragma unroll
+  for (int i = 0; i < ICD_RPW; ++i)
+#pragma unroll
+    for (int k = 0; k < ICD_MAXK; ++k) {
+      const int r = warp + 8 * i;
+      if (k >= K || r >= nq) continue;      // (warp-uniform)
+      float v = acc[i][k];
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+      if (lane == 0) q[k][r] = v;
+    }
+  __syncthreads();
+  const int sl = threadIdx.x;
+  if (sl < ICD_ROWS && t0 + sl < Tn) {
+    float s = 0.f;
+    for (int k = 0; k < K; ++k) {
+      const int r = sl + K - 1 - k;     // (r < nq <=> t0 + r < T: a tap past the sequence end contributes zero)
+      if (r < nq) s += q[k][r];
+    }
+    dx[(long long)b * Tn + t0 + sl] = s;
+  }
+}
+
+// per-batch column sums of several (B,T,N) slabs in one launch: out[l*out_slab + b*ldpb + n] = sum_t G[l*slab + (b*T+t)*ldg + n].
+// One CTA = 64 columns (a column pair per lane) of one (slab, batch row): 8 row lanes walk T in 4 independent chains and meet in
+// shared memory in a fixed order (bit-reproducible).  N and ldg even.
+template <class T>
+__global__ void __launch_bounds__(256) colsum_per_batch_slabs(const T* __restrict__ G, long long slab, int ldg, int Tn, int N, float* __restrict__ out,
+                                                              long long out_slab, int ldpb) {
+  __shared__ float sh[8][64];
+  const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
+  const int n = blockIdx.x * 64 + 2 * tx;
+  const int b = blockIdx.y, l = blockIdx.z;
+  float s[4][2] = {};
+  if (n < N) {
+    const T* p = G + l * slab + ((long long)b * Tn + ty) * ldg + n;
+    int t = ty;
+    for (; t + 24 < Tn; t += 32, p += 32LL * ldg) {
+#pragma unroll
+      for (int u = 0; u < 4; ++u) {
+        float2 v;
+        if constexpr (sizeof(T) == 2) {
+          const uint32_t w = *reinterpret_cast<const uint32_t*>(p + 8LL * u * ldg);
+          v = make_float2(__uint_as_float(w << 16), __uint_as_float(w & 0xffff0000u));
+        } else {
+          v = *reinterpret_cast<const float2*>(p + 8LL * u * ldg);
+        }
+        s[u][0] += v.x; s[u][1] += v.y;
+      }
+    }
+    for (; t < Tn; t += 8, p += 8LL * ldg) { s[0][0] += to_f(p[0]); s[0][1] += to_f(p[1]); }
+  }
+  sh[ty][2 * tx] = (s[0][0] + s[1][0]) + (s[2][0] + s[3][0]);
+  sh[ty][2 * tx + 1] = (s[0][1] + s[1][1]) + (s[2][1] + s[3][1]);
+  __syncthreads();
+  if (ty < 2) {
+    const int c = 2 * tx + ty;
+    float r = 0.f;
+#pragma unroll
+    for (int k = 0; k < 8; ++k) r += sh[k][c];
+    if (blockIdx.x * 64 + c < N) out[l * out_slab + (long long)b * ldpb + blockIdx.x * 64 + c] = r;
+  }
+}
+
 // ------------------------------------------------------------------ generic deterministic reductions
 // out[j] = scale * sum_{i<n_parts} partial[i*stride + j]  (+ addend[j]*add_coef), j < n
 __global__ void reduce_parts(const float* __restrict__ partial, int n_parts, long long stride, float* __restrict__ out, long long n,

@@ -1545,6 +1545,9 @@ struct BlockBwdMode {
   // the gate adjoint and the dgrad of this block run inside the persistent stack-backward launch (gemm_tc_stack_bwd.cuh):
   // only the weight-gradient problems are collected here
   bool in_stack = false;
+  // false: no weight gradient of the block is launched, collected or written; a conditioned block's per-batch sums of d z
+  // (which its gated conv's weight gradient would produce) are column sums of their own
+  bool param_grads = true;
   int side_group = -1, bucket = 0;   // grouped: side launch (-1: the final launch) and all-reduce bucket of the problems
 };
 
@@ -1606,7 +1609,9 @@ static int block_backward(wn_handle* h, cudaStream_t st, int l, const void* x_in
   const bool side1 = sd != nullptr && d_o != h->dotmp;
   cudaStream_t s1 = side1 ? sd->side : st;
   if (side1) CK(cudaStreamWaitEvent(sd->side, sd->ev_in, 0));
-  if (group) {
+  if (!m.param_grads) {
+    // (input gradients only: conv1 / conv_skip contribute their dgrads below, through Wdg)
+  } else if (group) {
     if constexpr (sizeof(T) == 2) {
       if (d_o) {
         TcWgJobDesc j = wg_job(h, b.conv1, g_l, D, d_o, ld_o, m.side_group, m.bucket);
@@ -1643,7 +1648,7 @@ static int block_backward(wn_handle* h, cudaStream_t st, int l, const void* x_in
   } else {
     unused_conv_grads(h, st, b.conv1.w_idx, b.conv1.b_idx, l2coef);
   }
-  if (b.has_skip && !cat && !group) {
+  if (m.param_grads && b.has_skip && !cat && !group) {
     if (dskip) {
       WgradH w = wgrad_of(h, b.conv_skip, g_l, D, dskip, ldsk, B, Tn, l2coef);
       w.side = side1;
@@ -1689,7 +1694,10 @@ static int block_backward(wn_handle* h, cudaStream_t st, int l, const void* x_in
     const int a_w = j == 0 ? R : D;
     // weight grad: rows (k, cin) <- taps of a_in shifted by -(K-1-k)*d ; the bias grad (and the
     // conditioning per-batch sums for the gated conv) are the column sums of the same G
-    if (group) {
+    if (!m.param_grads) {
+      // (grouped: d z of every block is kept, and model_backward sums them all in one launch behind the chain)
+      if (!group && j == depth - 1 && b.has_cond) run_colsum<T>(h, st, dcur, dcw, B, Tn, c.cout, h->dcb + (size_t)l * h->maxB * 2 * D, 2 * D, nullptr);
+    } else if (group) {
       if constexpr (sizeof(T) == 2) {
         TcWgJobDesc jd = wg_job(h, c, a_in, a_w, dcur, dcw, m.side_group, m.bucket);
         if (j == depth - 1 && b.has_cond) { jd.per_batch = h->dcb + (size_t)l * h->maxB * 2 * D; jd.ldpb = 2 * D; }
@@ -1751,11 +1759,12 @@ static int block_backward(wn_handle* h, cudaStream_t st, int l, const void* x_in
 }
 
 // conditioning adjoint: dWc_l, dbc_l from dcb; dcond = sum_l dcb_l Wc_l^T; then the mapping MLP
+// (param_grads == false, whole model only: the dgrads alone, the mapping MLP's result in the buffers of its per-layer chain)
 static int cond_backward(wn_handle* h, cudaStream_t st, const float* cond_in, const float* cond, int B, int l0, int nl, bool run_mapping, float* dcond_out,
-                         float l2coef, bool skip_wgrad = false) {
+                         float l2coef, bool skip_wgrad = false, bool param_grads = true) {
   const int n = 2 * h->D;
   if (l0 == 0 && nl == h->L) {
-    if (!skip_wgrad) {
+    if (!skip_wgrad && param_grads) {
       LaunchScope ls(h, st, CLS_MISC);
       cond_wgrad_all<<<dim3(cdiv((h->Cc + 1) * n, 128), h->L), 128, 0, st>>>(cond, h->Cc, h->dcb, (long long)h->maxB * n, h->d_params, h->d_grads,
                                                                           h->d_cond_offsets, B, n, l2coef, 0);
@@ -1784,7 +1793,7 @@ static int cond_backward(wn_handle* h, cudaStream_t st, const float* cond_in, co
   }
   if (!run_mapping) return WN_OK;
   MapArgs ma;
-  if (dcond_out == h->dcond && mapping_args(h, cond_in, B, l2coef, &ma)) {
+  if (param_grads && dcond_out == h->dcond && mapping_args(h, cond_in, B, l2coef, &ma)) {
     LaunchScope ls(h, st, CLS_MISC);
     mapping_bwd_fused<<<1, 256, 0, st>>>(ma);
     return WN_OK;
@@ -1798,11 +1807,11 @@ static int cond_backward(wn_handle* h, cudaStream_t st, const float* cond_in, co
       LaunchScope ls(h, st, CLS_MISC);
       dense_small_actgrad<<<cdiv(B * nn, 128), 128, 0, st>>>(dcur, h->cond_act[i], B * nn, h->cfg.mapping_activation);
     }
-    {
+    if (param_grads) {
       LaunchScope ls(h, st, CLS_MISC);
       dense_small_wgrad<<<cdiv((kin + 1) * nn, 128), 128, 0, st>>>(inp, kin, dcur, nn, G_(h, h->map_w[i]), G_(h, h->map_b[i]), B, kin, nn);
     }
-    if (l2coef != 0.f) {
+    if (param_grads && l2coef != 0.f) {
       LaunchScope ls(h, st, CLS_MISC);
       const long long cnt = h->params[h->map_w[i]].count;
       reduce_parts<<<cdiv(cnt, 256), 256, 0, st>>>(G_(h, h->map_w[i]), 1, 0, G_(h, h->map_w[i]), cnt, P_(h, h->map_w[i]), l2coef);
@@ -1837,7 +1846,10 @@ static const BwdSide* side_setup(wn_handle* h, cudaStream_t st, int l, bool on, 
 //   of 256)                            every n-th block in side launches beside the chain (side_pairs)
 //   bf16, grouped, stack backward (sb) the chain as one persistent launch, then the grouped launch, bucket by bucket (nb) when the
 //                                      step all-reduces its gradients
+// Without parameter gradients (wn_backward_ex with param_grads == 0) the same chain runs on the same buffers, alone: no weight-
+// gradient launch of any kind, no side stream, no side launches (the persistent chain kernels keep their full grids).
 struct BwdSchedule {
+  bool param_grads = true; // the parameter gradients are computed (false: input gradients only)
   bool group = false;      // grouped weight gradients (gemm_tc_wgroup.cuh)
   bool use_side = false;   // per-block weight gradients on the side stream
   bool cat = false;        // [d x_out | d skip] ping-pong buffers
@@ -1860,12 +1872,13 @@ struct BwdSchedule {
 };
 
 template <class T>
-static BwdSchedule bwd_schedule(wn_handle* h, int B, int Tn) {
+static BwdSchedule bwd_schedule(wn_handle* h, int B, int Tn, bool param_grads) {
   BwdSchedule s;
+  s.param_grads = param_grads;
   // (bf16 tier only: the fp32 tier's wgrad / column-sum scratch buffers are not duplicated for a second stream)
   if constexpr (sizeof(T) == 2) {
     s.group = h->use_group_wgrad != 0;
-    s.use_side = h->prof_tag == 0 && h->side_stream != nullptr && !s.group;
+    s.use_side = param_grads && h->prof_tag == 0 && h->side_stream != nullptr && !s.group;
     s.cat = h->dcatA != nullptr;
     // Backward chain as ONE persistent launch (gemm_tc_stack_bwd.cuh): D = R = 256, d z / d x_out
     // of every block kept (grouped weight gradients), more 256-row tiles per layer than CTA pairs.  It takes every SM for the
@@ -1884,14 +1897,14 @@ static BwdSchedule bwd_schedule(wn_handle* h, int B, int Tn) {
   // (256 tiles: 4 rounds on 74 or on 64 pairs), and the pairs left over run the weight gradients of every n-th block
   // beside the chain.  The plan (unit ranges per side group) exists from the second call on; the first call launches
   // every group at the end.
-  if (s.group && !s.sb && h->side_stream != nullptr && h->wg_side_every > 0 && more_tiles_than_pairs(B, Tn)) {
+  if (param_grads && s.group && !s.sb && h->side_stream != nullptr && h->wg_side_every > 0 && more_tiles_than_pairs(B, Tn)) {
     const int pairs = tc_num_sms() / 2, tiles = B * cdiv(Tn, 256), rounds = cdiv(tiles, pairs);
     s.side_pairs = pairs - cdiv(tiles, rounds);
     if (s.side_pairs < 6) s.side_pairs = 0;
   }
   // bucketed all-reduce: only with the stack-backward launch (every SM busy until the chain ends, all filter gradients in the
   // final grouped launch) and a communicator that reduces inside this step
-  s.nb = (s.group && s.sb && h->ar_now && h->prof_tag == 0 && h->comm_stream != nullptr) ? std::min(std::min(h->ar_buckets, h->L), 8) : 1;
+  s.nb = (param_grads && s.group && s.sb && h->ar_now && h->prof_tag == 0 && h->comm_stream != nullptr) ? std::min(std::min(h->ar_buckets, h->L), 8) : 1;
   if (s.group) for (auto& wp : h->wg_plans) if (wp.B == B && wp.T == Tn && wp.drop == h->drop_active && wp.sb == s.sb && wp.nb == s.nb) s.wplan = &wp.plan;
   s.side_now = s.wplan != nullptr && s.side_pairs > 0 && h->prof_tag == 0 && !s.wplan->side.empty();
   return s;
@@ -1920,12 +1933,12 @@ static int head_backward(wn_handle* h, cudaStream_t st, const BwdSchedule& s, in
     // (the head's d-activation buffers dlogits / dhA / dhB stay intact until the end of the pass when the head has <= 3 convs)
     bool head_grouped = false;
     if constexpr (sizeof(T) == 2) {
-      if (s.group && h->head.size() <= 3 && tc_wgrad_group_ok(hc.cin, hc.cout) && a_w == hc.cin) {
+      if (s.param_grads && s.group && h->head.size() <= 3 && tc_wgrad_group_ok(hc.cin, hc.cout) && a_w == hc.cin) {
         h->wg_jobs.push_back(wg_job(h, hc, a_in, a_w, dcur, dw, -1, s.nb - 1));      // (the head's gradients travel with the last bucket)
         head_grouped = true;
       }
     }
-    if (!head_grouped) RET(run_wgrad<T>(h, st, CLS_GEMM, wgrad_of(h, hc, a_in, a_w, dcur, dw, B, Tn, l2coef)));
+    if (s.param_grads && !head_grouped) RET(run_wgrad<T>(h, st, CLS_GEMM, wgrad_of(h, hc, a_in, a_w, dcur, dw, B, Tn, l2coef)));
     GemmH g;
     g.B = B; g.T = Tn; g.N = hc.cin; g.nseg = 1;
     g.seg[0] = SegH{dcur, dw, 0, (sizeof(T) == 2 && i + 1 == (int)h->head.size()) ? h->ldd : hc.cout};
@@ -1967,6 +1980,7 @@ static int cat_chain(wn_handle* h, cudaStream_t st, const BwdSchedule& s, int B,
     BlockBwdMode m;
     m.side = side_setup(h, st, l, s.use_side, &sd);
     m.dz = (l & 1) ? h->dz2 : h->dz;
+    m.param_grads = s.param_grads;
     RET(block_backward<T>(h, st, l, x_in, cur, ldc, dsk, ldc, nxt, ldc, B, Tn, l2coef, m));
     cur = nxt;
     nxt = (nxt == h->dcatB) ? h->dcatA : h->dcatB;
@@ -2049,7 +2063,7 @@ static int block_chain(wn_handle* h, cudaStream_t st, const BwdSchedule& s, int 
     BlockBwdMode m;
     m.side = side_setup(h, st, l, s.use_side, &sd);
     m.dz = s.group ? dz_slab<T>(h, l) : ((l & 1) ? h->dz2 : h->dz);
-    m.grouped = s.group; m.in_stack = stacked;
+    m.grouped = s.group; m.in_stack = stacked; m.param_grads = s.param_grads;
     m.side_group = s.side_group(h, l); m.bucket = s.bucket(h, l);
     RET(block_backward<T>(h, st, l, x_in, dxout, h->R, dskip, h->Sp, dx_in, h->R, B, Tn, l2coef, m));
     if constexpr (sizeof(T) == 2) {
@@ -2095,6 +2109,20 @@ static void input_conv_backward(wn_handle* h, cudaStream_t s_, const float* x, i
     LaunchScope ls(h, s_, CLS_MISC);
     reduce_parts_tall<<<cdiv(h->R, 32), 256, 0, s_>>>(h->colpart + kr, nparts, (long long)(h->K + 1) * h->R, G_(h, h->input_conv.b_idx), h->R, nullptr, 0.f);
   }
+}
+
+// ---- input conv dgrad: dx (B,T) fp32 = d loss / d x from the final d h0 (row stride ld_dx: R, or R + S in the cat layout)
+template <class T>
+static void input_conv_dgrad_run(wn_handle* h, cudaStream_t st, const void* dh0, int ld_dx, float* dx, int B, int Tn) {
+  OuterLabel ol(h, "input_dgrad");
+  LaunchScope ls(h, st, CLS_MISC);
+  constexpr int V = 16 / sizeof(T);
+  const bool vec = (h->R * sizeof(T)) % 16 == 0 && (ld_dx * sizeof(T)) % 16 == 0 && ((uintptr_t)dh0 & 15) == 0;
+  const dim3 grid(cdiv(Tn, ICD_ROWS), B);
+  if (vec)
+    input_conv_dgrad<T, V><<<grid, 256, 0, st>>>((const T*)dh0, ld_dx, P_(h, h->input_conv.w_idx), dx, Tn, h->R, h->K);
+  else
+    input_conv_dgrad<T, 1><<<grid, 256, 0, st>>>((const T*)dh0, ld_dx, P_(h, h->input_conv.w_idx), dx, Tn, h->R, h->K);
 }
 
 // ---- every block's conv1 / conv_skip / gated-conv weight gradients in ONE launch (+ one finish), or bucket by bucket with the
@@ -2177,9 +2205,11 @@ static int grouped_wgrad(wn_handle* h, cudaStream_t st, const BwdSchedule& s, in
   return WN_OK;
 }
 
+// dx (or null): d loss / d x of the input signal.  param_grads == false: no parameter gradient is computed or written
 template <class T>
-static int model_backward(wn_handle* h, cudaStream_t st, const float* x, int ldx, const float* cond_in, int B, int Tn, float l2coef) {
-  const BwdSchedule s = bwd_schedule<T>(h, B, Tn);
+static int model_backward(wn_handle* h, cudaStream_t st, const float* x, int ldx, const float* cond_in, int B, int Tn, float l2coef,
+                          float* dx = nullptr, bool param_grads = true) {
+  const BwdSchedule s = bwd_schedule<T>(h, B, Tn, param_grads);
   h->wg_jobs.clear();
   h->wg_last_tiles = 0; h->wg_last_side = 0;
   h->stack_bwd_layers = 0;
@@ -2194,6 +2224,20 @@ static int model_backward(wn_handle* h, cudaStream_t st, const float* x, int ldx
     else RET(block_chain<T>(h, st, s, B, Tn, l2coef, &dxout));
   }
   const int ld_dx = s.cat ? h->R + h->S : h->R;
+  if (dx) input_conv_dgrad_run<T>(h, st, dxout, ld_dx, dx, B, Tn);
+  if (!s.param_grads) {
+    if (!h->cfg.conditioning) return WN_OK;
+    OuterLabel ol(h, "cond_bwd");
+    if (s.group) {
+      // the per-batch sums of every block's kept d z (the per-block chain took them block by block)
+      const int n = 2 * h->D;
+      LaunchScope ls(h, st, CLS_MISC);
+      colsum_per_batch_slabs<T><<<dim3(cdiv(n, 64), B, h->L), 256, 0, st>>>((const T*)h->dz_all, (long long)h->maxB * h->maxT * n, n, Tn, n, h->dcb,
+                                                                          (long long)h->maxB * n, n);
+    }
+    // d cond from the per-batch sums, through the mapping MLP's dgrads
+    return cond_backward(h, st, cond_in, h->last_cond, B, 0, h->L, true, h->dcond, 0.f, false, false);
+  }
   // The input conv's gradients run on the side stream beside the final grouped weight-gradient launch (their CTAs fit next to
   // the tensor kernel's on the same SMs) with side launches, and behind the stack-backward launch: d h0 is final there too.
   const bool grouped = s.group && !h->wg_jobs.empty();
@@ -2662,7 +2706,7 @@ static int cond_input_grad(wn_handle* h, cudaStream_t st, int B, float* dcond) {
 }
 
 template <class T>
-static int backward_entry(wn_handle* h, const float* dpred, float* dcond, cudaStream_t st) {
+static int backward_entry(wn_handle* h, const float* dpred, float* dcond, float* dx, bool param_grads, cudaStream_t st) {
   const int B = h->fwd.B, Tn = h->fwd.T;
   const long long rows = (long long)B * Tn;
   {
@@ -2678,15 +2722,16 @@ static int backward_entry(wn_handle* h, const float* dpred, float* dcond, cudaSt
       convert_pad_kernel<float, T><<<cdiv(rows * h->ldd, 256), 256, 0, st>>>(dpred, h->Cout, (T*)h->dlogits, h->ldd, rows);
     }
   }
-  RET(model_backward<T>(h, st, h->fwd.x, h->fwd.ldx, h->fwd.cond, B, Tn, 0.f));
+  RET(model_backward<T>(h, st, h->fwd.x, h->fwd.ldx, h->fwd.cond, B, Tn, 0.f, dx, param_grads));
   if (dcond) RET(cond_input_grad(h, st, B, dcond));
   return WN_OK;
 }
 
-extern "C" int wn_backward(wn_handle* h, const float* dpred_dev, float* dcond_dev, void* stream) {
+extern "C" int wn_backward_ex(wn_handle* h, const float* dpred_dev, float* dcond_dev, float* dx_dev, int param_grads, void* stream) {
   if (!h) { set_err("null handle"); return WN_ERR_VALUE; }
   if (!dpred_dev || ((uintptr_t)dpred_dev & 15) != 0) { set_err("dpred must be a 16-byte aligned device buffer"); return WN_ERR_VALUE; }
   if (dcond_dev && !h->cfg.conditioning) { set_err("the model has no conditioning input"); return WN_ERR_VALUE; }
+  if (!param_grads && !dx_dev && !dcond_dev) { set_err("wn_backward_ex without parameter gradients needs dx or dcond: nothing to compute"); return WN_ERR_VALUE; }
   if (!h->fwd_valid) { set_err("wn_backward needs a wn_forward_ex since the handle's activations or weights last changed"); return WN_ERR_STATE; }
   CK(cudaSetDevice(h->cfg.device));
   h->launches = 0;
@@ -2695,11 +2740,15 @@ extern "C" int wn_backward(wn_handle* h, const float* dpred_dev, float* dcond_de
   h->drop_active = h->fwd.training && h->cfg.dropout > 0.f;
   h->ar_now = false;
   h->lastB = h->fwd.B; h->lastT = h->fwd.T;     // wn_debug_tensor reads the pass just differentiated
-  int r = h->cfg.precision == WN_BF16 ? backward_entry<bf16>(h, dpred_dev, dcond_dev, st) : backward_entry<float>(h, dpred_dev, dcond_dev, st);
+  int r = h->cfg.precision == WN_BF16 ? backward_entry<bf16>(h, dpred_dev, dcond_dev, dx_dev, param_grads != 0, st)
+                                      : backward_entry<float>(h, dpred_dev, dcond_dev, dx_dev, param_grads != 0, st);
   h->drop_active = false;
   RET(r);
   CK(cudaGetLastError());
   return WN_OK;
+}
+extern "C" int wn_backward(wn_handle* h, const float* dpred_dev, float* dcond_dev, void* stream) {
+  return wn_backward_ex(h, dpred_dev, dcond_dev, nullptr, 1, stream);
 }
 extern "C" int wn_forward(wn_handle* h, const float* x_dev, const float* cond_dev, int B, int T, float* out_dev, void* stream) {
   return wn_forward_ex(h, x_dev, cond_dev, B, T, 0, out_dev, stream);

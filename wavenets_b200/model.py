@@ -331,12 +331,12 @@ class WaveNet:
     self._last_call = None
     # training=True: Keras runs the blocks' Dropout layers (layers.py:195-196) — fresh masks per call
     _lib.check(h.lib.wn_forward_ex(h.h, h.ptr(x2), h.ptr(cond), B, T, 1 if training else 0, h.ptr(out), h.stream_ptr()))
-    self._last_call = (x2, cond, (B, T, cout))
+    self._last_call = (x2, cond, (B, T, cout), tuple(x.shape))
     return out
 
   __call__ = call
 
-  def backward(self, dpred):
+  def backward(self, dpred, input_grad=False, param_grads=True):
     """Gradients of the last `call` for a loss the caller computes on its output (tf.GradientTape over model(inputs),
     then tape.gradient(loss, model.trainable_variables)).  `dpred` (B, T, C) = d loss / d pred, pred being what `call`
     returned (probabilities or mixture parameters).  The gradients land in `get_grads()` / `handle.flat_grads` as after
@@ -344,11 +344,18 @@ class WaveNet:
     `optimizer.apply_gradients(model)`; no L2 term (model.py:331-334 belongs to train_step, not to call).  Returns
     d loss / d cond ((B, cond_in) tensor), or None without conditioning.  Anything that changes the weights, the
     activations or the dropout masks (train_step, generate, set_weights, optimizer.apply_gradients, ...) between the
-    call and this one makes it raise."""
+    call and this one makes it raise.
+
+    input_grad=True also gives d loss / d x (tape.gradient(loss, x)) and returns (dx, dcond): dx has the shape of the
+    waveform passed to `call`, (B, T, 1) or (B, T), and is this replica's own (never reduced).  param_grads=False computes
+    no parameter gradient at all (a frozen model used as a differentiable function of its input): `get_grads()` keeps what
+    it held, and no clipnorm or all-reduce runs.  It needs something to compute: input_grad=True or conditioning."""
     last = self._last_call
     if last is None:
       raise RuntimeError('backward needs a preceding call on this model')
-    x2, cond, shape = last
+    x2, cond, shape, x_shape = last
+    if not param_grads and not input_grad and cond is None:
+      raise ValueError('backward(param_grads=False) needs input_grad=True or a conditioned model: nothing to compute')
     h = self.handle
     dpred = as_dev(dpred, h.device)
     if tuple(dpred.shape) != shape:
@@ -356,9 +363,13 @@ class WaveNet:
     if dpred.data_ptr() % 16:
       dpred = dpred.clone()
     dcond = torch.empty((shape[0], int(cond.shape[-1])), dtype=torch.float32, device=h.device) if cond is not None else None
-    _lib.check(h.lib.wn_backward(h.h, h.ptr(dpred), h.ptr(dcond), h.stream_ptr()))
-    # the library reduces inside wn_train_step only (wn_comm_fuse_allreduce): here the all-reduce always follows
-    self._reduce_grads(allreduce_done=False)
+    dx = torch.empty(shape[:2], dtype=torch.float32, device=h.device) if input_grad else None
+    _lib.check(h.lib.wn_backward_ex(h.h, h.ptr(dpred), h.ptr(dcond), h.ptr(dx), 1 if param_grads else 0, h.stream_ptr()))
+    if param_grads:
+      # the library reduces inside wn_train_step only (wn_comm_fuse_allreduce): here the all-reduce always follows
+      self._reduce_grads(allreduce_done=False)
+    if input_grad:
+      return dx.reshape(x_shape), dcond
     return dcond
 
   # ------------------------------------------------------------------ targets (model.py:151-155)
